@@ -20,10 +20,13 @@ One JSON line is printed by rank 0.  Besides the headline keys of the contract i
 Under torchrun each rank drives one GPU; chains are sharded by global chain id with no data-path
 collective; the only collective is the final gather of the per-chain averages (NCCL), inside the e2e region.
 `--workload X` runs a single workload as the headline instead (development).
+`--dump-outputs DIR` writes what the headline's last timed step left for a caller (rank 0's chains) as DIR/<name>.npy,
+so that two builds can be compared output for output on identical, seeded inputs.
 """
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -34,6 +37,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(ROOT, "polymer-stats_b200"))
+sys.dont_write_bytecode = True   # the tree may be read-only; the benchmark writes nothing into it
 
 METRIC = "monomer MC updates/sec (whole box), interacting n=512 dielectric chains"
 UNIT = "updates/s"
@@ -299,8 +303,37 @@ def shard_of(W, rank, world, chains_override=None):
     return cases[lo:hi], rep, lo * rep, (hi - lo) * rep, len(cases) * rep
 
 
-def measure(cx: Ctx, name: str, steps: int, warmup: int, want_e2e=True, chains_override=None, S_override=None):
-    """One workload on this rank's GPU: device-timed resident `value`, e2e through the public API, roofline."""
+DUMP_BYTES = 63_000_000   # array data of one dump; with the .npy headers it stays below 64 MB
+
+
+def dump_outputs(ens, clustering: bool, out_dir: str):
+    """Write what a caller of the timed path receives after its last step, as float64 .npy files: the chain states
+    (phi, theta), the per-chain averages, acceptance rates, normalisers and step diagnostics, and for the clustering
+    driver its extra averages and cluster statistics.  When all of it exceeds DUMP_BYTES, the same fixed, seeded sample
+    of chains is taken from every array; chain_index.npy names the chains written."""
+    import numpy as np
+    phi, theta = ens.get_state_all()
+    avg, ar, nrm = ens.averages()
+    arrays = {"phi": phi, "theta": theta, "averages": avg, "acc_rate": ar, "normalizer": nrm,
+              "diagnostics": ens.diagnostics()}
+    if clustering:
+        arrays.update(extra_averages=ens.extra_averages(), cluster_stats=ens.cluster_stats())
+    per_chain = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    keep = min(ens.nchains, DUMP_BYTES // per_chain)
+    idx = np.arange(ens.nchains)
+    if keep < ens.nchains:
+        idx = np.sort(np.random.default_rng(SEED).choice(ens.nchains, keep, replace=False))
+    arrays["chain_index"] = idx
+    os.makedirs(out_dir, exist_ok=True)
+    for nm, a in arrays.items():
+        a = a if nm == "chain_index" else a[idx]
+        np.save(os.path.join(out_dir, nm + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
+def measure(cx: Ctx, name: str, steps: int, warmup: int, want_e2e=True, chains_override=None, S_override=None,
+            dump_dir=None):
+    """One workload on this rank's GPU: device-timed resident `value`, e2e through the public API, roofline;
+    with dump_dir, the outputs of the last timed step are written there (dump_outputs)."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -346,6 +379,8 @@ def measure(cx: Ctx, name: str, steps: int, warmup: int, want_e2e=True, chains_o
     cx.barrier()
     t_w1 = time.perf_counter()
     launches = ens.launch_count() - launches0
+    if dump_dir and cx.rank == 0:
+        dump_outputs(ens, clustering, dump_dir)
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=cx.dev)
     if cx.world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -530,7 +565,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline only: skip workloads / strong / multi_abi")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's outputs after its last timed step to DIR/<name>.npy (float64, < 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -577,9 +616,10 @@ def main():
     cx.derived_tf = 148 * 64 * 2 * 1.965e9 / 1e12
     cx.sampler = ClockSampler(local_rank)
     cx.sampler.start()
+    atexit.register(cx.sampler.stop)   # no nvidia-smi left running when a measurement raises
 
     head = measure(cx, args.workload, args.steps, args.warmup, want_e2e=not args.no_e2e,
-                   chains_override=args.chains_per_gpu, S_override=args.trials_per_step)
+                   chains_override=args.chains_per_gpu, S_override=args.trials_per_step, dump_dir=args.dump_outputs)
 
     extras = args.workload == "C2" and not args.no_extras and not args.chains_per_gpu and not args.trials_per_step
     workloads, strong, multi_abi = {}, {}, None

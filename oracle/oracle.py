@@ -12,6 +12,7 @@ import ctypes as C
 import math
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -353,14 +354,17 @@ _native = None
 
 def native_lib():
     """The `-O3 -march=native` build of the same source, compiled on THIS machine (timing only; bench.py).  Returns
-    (library, flags text); falls back to the portable build when the host has no compiler."""
+    (library, flags text); falls back to the portable build when the host has no compiler.  Built in a temporary
+    directory (the tree may be read-only) that is removed once the library is loaded."""
     global _native
     if _native is not None:
         return _native
-    path = os.path.join(_HERE, "_bench", "libpolymc_oracle_native.so")
     try:
-        subprocess.check_call(["make", "-C", _HERE, "-s", "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-        L = C.CDLL(path)
+        with tempfile.TemporaryDirectory(prefix="polymc_oracle_native_") as tmp:
+            path = os.path.join(tmp, "libpolymc_oracle_native.so")
+            subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"NATIVE_OUT={path}"],
+                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            L = C.CDLL(path)
         L.orc_bench.argtypes = [C.POINTER(OrcCase), C.c_uint64, C.c_int32, C.c_int32, C.c_int64, C.c_int32]
         L.orc_bench.restype = C.c_double
         _native = (L, "gcc -O3 -march=native, built on the timed host")

@@ -347,12 +347,16 @@ def test_host_formatting_reproduces_the_reference_text(runs):
             assert run["rolling_csv"].split("\n", 1)[0] == want
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/inc"), reason="the reference sources exist only in the build container")
+REFERENCE = os.environ.get("POLYMC_REFERENCE_DIR")
+
+
+@pytest.mark.skipif(not REFERENCE or not os.path.isdir(os.path.join(REFERENCE, "inc")),
+                    reason="needs the reference sources: set POLYMC_REFERENCE_DIR")
 def test_fixtures_regenerate_from_the_reference_sources(runs):
-    """Freshness: one driver run regenerated NOW from /root/reference equals the committed fixture (the GPU box has no
-    reference tree, so this runs in the build container only)."""
+    """Freshness: one driver run regenerated NOW from the reference sources equals the committed fixture."""
     name = "cluster_noninteracting_x0"
-    p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "golden", "make_ref_fixtures.py"), "--only", name],
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "golden", "make_ref_fixtures.py"), "--only", name,
+                        "--reference", REFERENCE],
                        capture_output=True, text=True, timeout=600)
     assert p.returncode == 0, p.stderr[-2000:]
     fresh = json.load(open(p.stdout.strip().split("\n")[-1]))["runs"][0]

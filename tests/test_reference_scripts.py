@@ -3,8 +3,11 @@ unchanged."  Checked literally: the UNMODIFIED reference script scripts/aggregat
 `<prefix>.out` files written by this package (the stdout block of the CLI twins under the launchers' file names) and must
 produce the table polymc.aggregate produces directly — byte for byte.
 
-Needs /root/reference (this container only; the GPU box has none): skipped elsewhere.  CPU only."""
+The files the reference scripts wrote for these inputs are stored in tests/golden/ref/script_tables.json, so the
+comparison runs on any machine.  With POLYMC_REFERENCE_DIR set to a checkout of the reference, the scripts are also run
+now and must write the same files.  CPU only."""
 import io
+import json
 import os
 import sys
 
@@ -14,9 +17,18 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 sys.path.insert(0, os.path.join(ROOT, "polymer-stats_b200"))
-SCRIPT = "/root/reference/scripts/aggregate_mcmc.jl"
+REF = os.environ.get("POLYMC_REFERENCE_DIR")
+SCRIPT = os.path.join(REF, "scripts", "aggregate_mcmc.jl") if REF else None
+with open(os.path.join(ROOT, "tests", "golden", "ref", "script_tables.json")) as _f:
+    STORED = json.load(_f)["tables"]
 
-pytestmark = pytest.mark.skipif(not os.path.exists(SCRIPT), reason="the reference tree is not on this machine")
+
+def assert_reference_agrees(key, ours, run_reference):
+    """ours: {file name: text} as polymc.aggregate writes it.  The reference script wrote STORED[key] for the same
+    inputs; with the reference tree at hand, run_reference() runs it now and returns its files."""
+    if REF:
+        assert run_reference() == ours
+    assert STORED[key] == ours
 
 
 def run_reference_aggregate(argv):
@@ -54,9 +66,13 @@ def test_reference_aggregate_script_reads_our_out_files(tmp_path, chain_type, ka
     ag.write_table(str(ours), *ag.aggregate_table(entries, chain_type, kappaflag, runflag, 3))
     theirs = tmp_path / "theirs.csv"
     argv = [str(theirs), str(outdir), "*.out", chain_type, "3D", "true" if kappaflag else "false"] + (["true"] if runflag else [])
-    log = run_reference_aggregate(argv)
-    assert log.count("processing") == 5
-    assert theirs.read_text() == ours.read_text()
+
+    def run_reference():
+        log = run_reference_aggregate(argv)
+        assert log.count("processing") == 5
+        return {"table.csv": theirs.read_text()}
+    assert_reference_agrees(f"aggregate_mcmc/{chain_type}-{kappaflag}-{runflag}", {"table.csv": ours.read_text()},
+                            run_reference)
 
 
 def test_reference_aggregate_script_reads_our_2d_out_files(tmp_path):
@@ -71,8 +87,11 @@ def test_reference_aggregate_script_reads_our_2d_out_files(tmp_path):
     ag.write_out_files(str(outdir), text)
     ours, theirs = tmp_path / "ours.csv", tmp_path / "theirs.csv"
     ag.write_table(str(ours), *ag.aggregate_table(entries, "dielectric", False, False, 2))
-    run_reference_aggregate([str(theirs), str(outdir), "*.out", "dielectric", "2D"])
-    assert theirs.read_text() == ours.read_text()
+
+    def run_reference():
+        run_reference_aggregate([str(theirs), str(outdir), "*.out", "dielectric", "2D"])
+        return {"table.csv": theirs.read_text()}
+    assert_reference_agrees("aggregate_mcmc/2D", {"table.csv": ours.read_text()}, run_reference)
 
 
 def test_reference_aggregate_script_on_the_plain_drivers_ten_lines(tmp_path):
@@ -89,14 +108,13 @@ def test_reference_aggregate_script_on_the_plain_drivers_ten_lines(tmp_path):
     ag.write_out_files(str(outdir), text)
     ours, theirs = tmp_path / "ours.csv", tmp_path / "theirs.csv"
     ag.write_table(str(ours), *ag.aggregate_table(entries, "dielectric", False, False, 3))
-    run_reference_aggregate([str(theirs), str(outdir), "*.out", "dielectric"])
-    assert theirs.read_text() == ours.read_text()
+
+    def run_reference():
+        run_reference_aggregate([str(theirs), str(outdir), "*.out", "dielectric"])
+        return {"table.csv": theirs.read_text()}
+    assert_reference_agrees("aggregate_mcmc/ten_lines", {"table.csv": ours.read_text()}, run_reference)
 
 
-REDUCE = "/root/reference/scripts/reduce_tabular_data.jl"
-
-
-@pytest.mark.skipif(not os.path.exists(REDUCE), reason="the reference tree is not on this machine")
 @pytest.mark.parametrize("chain_type,kappaflag", [("dielectric", False), ("dielectric", True), ("polar", False)])
 def test_reference_reduce_script_on_our_tables(tmp_path, chain_type, kappaflag):
     """scripts/reduce_tabular_data.jl (unmodified, run by minijl) pools the repeated runs of a table written by
@@ -116,18 +134,17 @@ def test_reference_reduce_script_on_our_tables(tmp_path, chain_type, kappaflag):
     nparams = len(ag.input_headers(chain_type, kappaflag))
     ours = tmp_path / "ours.csv"
     ag.write_table(str(ours), *ag.reduce_table(header, rows, nparams))
-    it = Interp(argv=[str(indir), str(outdir), chain_type] + (["true"] if kappaflag else []))
-    sink = io.StringIO()
-    it.stdout = sink
-    it.genv.vars["stdout"] = sink
-    it.run_main(REDUCE)
-    assert (outdir / "study.csv").read_text() == ours.read_text()
+
+    def run_reference():
+        it = Interp(argv=[str(indir), str(outdir), chain_type] + (["true"] if kappaflag else []))
+        sink = io.StringIO()
+        it.stdout = sink
+        it.genv.vars["stdout"] = sink
+        it.run_main(os.path.join(REF, "scripts", "reduce_tabular_data.jl"))
+        return {"study.csv": (outdir / "study.csv").read_text()}
+    assert_reference_agrees(f"reduce_tabular_data/{chain_type}-{kappaflag}", {"study.csv": ours.read_text()}, run_reference)
 
 
-BY = "/root/reference/scripts/aggregate_by.jl"
-
-
-@pytest.mark.skipif(not os.path.exists(BY), reason="the reference tree is not on this machine")
 @pytest.mark.parametrize("param,runflag", [("E0", False), ("Fz", False), ("FxFz", False), ("E0", True)])
 def test_reference_aggregate_by_script_on_our_out_files(tmp_path, monkeypatch, param, runflag):
     """scripts/aggregate_by.jl (unmodified, run by minijl — including the `julia scripts/aggregate_mcmc.jl …` command it
@@ -148,27 +165,31 @@ def test_reference_aggregate_by_script_on_our_out_files(tmp_path, monkeypatch, p
                 entries.append((prefix, ag.output_values(avg, ar, 1.0, 100, ex)))
     indir, outdir = tmp_path / "study", tmp_path / "by"
     ag.write_out_files(str(indir), text)
-    monkeypatch.chdir("/root/reference")            # the script spawns `julia scripts/aggregate_mcmc.jl` relative to the tree
-    it = Interp(argv=[str(outdir), str(indir), param, "dielectric", "3D", "false"] + (["true"] if runflag else []))
-    sink = io.StringIO()
-    it.stdout = sink
-    it.genv.vars["stdout"] = sink
-    it.run_main(BY)
-    ours = ag.aggregate_by(entries, param, "dielectric", False, runflag, 3)
-    assert sorted(os.listdir(outdir)) == sorted(ours.keys()) and len(ours) >= 3
-    for name, (header, rows) in ours.items():
+    ours = {}
+    for name, (header, rows) in ag.aggregate_by(entries, param, "dielectric", False, runflag, 3).items():
         mine = tmp_path / ("ours_" + name)
         ag.write_table(str(mine), header, rows)
-        assert (outdir / name).read_text() == mine.read_text(), name
+        ours[name] = mine.read_text()
+    assert len(ours) >= 3
+
+    def run_reference():
+        monkeypatch.chdir(REF)            # the script spawns `julia scripts/aggregate_mcmc.jl` relative to the tree
+        it = Interp(argv=[str(outdir), str(indir), param, "dielectric", "3D", "false"] + (["true"] if runflag else []))
+        sink = io.StringIO()
+        it.stdout = sink
+        it.genv.vars["stdout"] = sink
+        it.run_main(os.path.join(REF, "scripts", "aggregate_by.jl"))
+        return {name: (outdir / name).read_text() for name in os.listdir(outdir)}
+    assert_reference_agrees(f"aggregate_by/{param}-{runflag}", ours, run_reference)
 
 
-LAUNCHERS = sorted(__import__("glob").glob("/root/reference/run/*.jl"))
+LAUNCHERS = sorted(__import__("glob").glob(os.path.join(REF, "run", "*.jl"))) if REF else []
 # two launchers draw their cases from Distributions.jl (no scripted stream here); one is not valid Julia upstream
 # (`zip(a, b; c; d)`: positional arguments after the semicolon)
 NOT_RUN = {"phases-random_2023-05-15.jl", "phases-random_2023-07-11.jl", "phases_2023-05-15.jl"}
 
 
-@pytest.mark.skipif(not LAUNCHERS, reason="the reference tree is not on this machine")
+@pytest.mark.skipif(not LAUNCHERS, reason="needs the reference's run/ launchers: set POLYMC_REFERENCE_DIR")
 def test_every_reference_launcher_command_is_accepted_by_the_cli_twins(tmp_path):
     """north_star: "It keeps the existing CLI options … so run/* sweep scripts … work unchanged."  Every launcher of the
     reference's run/ directory is executed UNMODIFIED by minijl with the `julia <driver>.jl …` commands it spawns
