@@ -243,6 +243,55 @@ int32_t pmc_checkpoint_load(pmc_handle* h, const void* buf, int64_t bytes);
  * clustering driver. */
 int32_t pmc_accumulators_dd(pmc_handle* h, double* hi, double* lo);
 
+/* ---- replica exchange (parallel tempering) across kT and force ladders of one handle --------- */
+/* A new capability: the reference has no exchange, and a handle without ladders runs exactly as before.
+ *
+ * Ladder.  An ordered list of case indices of this handle, the rungs.  Replica r of rung k pairs with replica r of
+ * rung k+1, so R replicas per case hold R independent copies of every ladder.  A case is in at most one ladder; cases
+ * outside every ladder run as usual.  The rungs of a ladder agree on every field that enters the energy or the target
+ * density (E0, K1, K2, mu, b, n, chain_type, energy_type, kappa, psi0, cutoff_radius, cutoff_full, clustering, planar)
+ * and may differ in kT, Fz, Fx and the proposal / protocol fields (step sizes, adj_*, steps_per_adjust, do_flips,
+ * cluster_prob, accum_mode, alpha_carry, force_init).  PMC_ERR_INVALID, with a message, for umbrella = 1 (its weight
+ * function depends on kT and F), for rungs whose Fz / Fx differ under PMC_ENERGY_CUTOFF with cutoff_full = 0 (F is then
+ * not part of the energy), for a case index out of range or repeated, for a ladder of fewer than two rungs and for any
+ * mismatch in the fields above.  Ladders are a single-handle feature: pmc_multi_* has no exchange, and on a
+ * pmc_multi_shard handle the rungs are that shard's own case indices.
+ *
+ * Exchange rule.  Slot s samples π_s(x) ∝ exp(−U_s(x)/kT_s)·Ω(x), U_s the running energy of the run kernels
+ * (U_s(x) = U₀(x) − r(x)·F_s when F enters the energy).  A swap of slots a and b is accepted iff Δ ≥ 0 (no draw) or
+ * ε < exp(Δ), Δ = β_a [U_a(x_a) − U_a(x_b)] + β_b [U_b(x_b) − U_b(x_a)], U_a(x_b) = U_b(x_b) + r_b·(F_b − F_a),
+ * β = 1/kT of the stage (pmc_begin_stage's scale included).  Ω and the bending energy cancel.
+ *
+ * Pairing.  Round k (counted per handle from 0) attempts the pairs (rung i, rung i+1) with i ≡ k (mod 2) in every
+ * ladder and replica column.  ε comes from Philox stream 7 at position k of the lower-rung chain (DESIGN.md §4); the
+ * trial streams are untouched, a slot keeps drawing its own stream whatever configuration it holds.
+ *
+ * What moves.  With the configuration: the monomer records, Ω, Σu, r, p, the clustering driver's Σψ and Σcos²θ, and
+ * U (re-expressed for the new slot by the formula above).  With the slot (its temperature or force): accumulators,
+ * step sizes, counters, drift_max and cluster statistics, so the averages of a case are the averages of its rung.
+ * The acceptor is re-bound to the slot's new configuration (α carry 0, the rule for alpha_carry = 1), as
+ * pmc_begin_stage does.  pmc_reinit and pmc_begin_stage leave ladders, labels and statistics as they are.
+ *
+ * pmc_set_ladders: rungs = case indices in rung order, ladders separated by -1 (a trailing -1 is allowed); len 0
+ * clears.  Resets the round counter and the diagnostics.
+ * pmc_exchange: one round.  accepted [chains] (may be NULL): 1 at the lower slot of each accepted pair, else 0.
+ * pmc_run_tempering / _ex: pmc_run / pmc_run_ex (exchange_every) followed by pmc_exchange, nsteps / exchange_every
+ * times, bit-identical to that loop, rows included, without host synchronisation between the chunks.  exchange_every
+ * must divide nsteps and stepout must divide exchange_every (or be <= 0: no rows).  Rows as pmc_run / pmc_run_ex over
+ * all nsteps.
+ * pmc_exchange_stats, any pointer may be NULL: pair_stats [ncases][2] = attempts, accepts of (case, its next rung),
+ * summed over replicas (0 for top rungs and cases outside ladders); walker [chains] = the global chain id whose initial
+ * configuration the slot now holds (a permutation within every ladder column); round_trips [chains], by walker (index =
+ * label − chain_id_base) = completed bottom → top → bottom trips.
+ * With ladders set, pmc_checkpoint_save appends the ladders, the round counter, the statistics and the walker labels
+ * and round-trip state; pmc_checkpoint_load requires the same ladders.  Without ladders checkpoints are unchanged. */
+int32_t pmc_set_ladders(pmc_handle* h, const int32_t* rungs, int64_t len);
+int32_t pmc_exchange(pmc_handle* h, int32_t* accepted);
+int32_t pmc_run_tempering(pmc_handle* h, int64_t nsteps, int64_t exchange_every, int64_t stepout, double* traj, double* roll);
+int32_t pmc_run_tempering_ex(pmc_handle* h, int64_t nsteps, int64_t exchange_every, int64_t stepout,
+                             double* traj, double* roll19, double* state);
+int32_t pmc_exchange_stats(pmc_handle* h, double* pair_stats, int64_t* walker, int64_t* round_trips);
+
 /* ---- one ensemble over several GPUs of one box (ABI v3) ------------------------------------ */
 /* Replaces the fan-out of the reference's launchers — `julia -p N run/interacting_dielectric_study.jl workdir`,
  * run/interacting_dielectric_study.jl:37-47 (pmap over cases, one single-threaded process per case).  The

@@ -21,6 +21,11 @@
 
 using namespace pmc;
 
+namespace pmc {
+struct ExPair;        // exchange.cuh
+struct ExchangeArgs;
+}  // namespace pmc
+
 // sets the calling thread's pmc_last_error() text and returns `code`
 int pmc_fail(int code, const std::string& msg);
 
@@ -104,6 +109,17 @@ struct pmc_handle {
   int* pair_next = nullptr;
   const char* kernel_name = "";  // the MCMC kernel the last (dry or real) launch decision picked, pmc_kernel_name
   int dry_run = 0;               // launch helpers only record their decision
+  // replica exchange (exchange.cuh), set by pmc_set_ladders
+  std::vector<int32_t> ladder;          // the rungs as given, ladders separated by -1; empty: no ladders
+  pmc::ExPair* ex_pairs = nullptr;      // candidate pairs, those of even rounds first
+  int64_t ex_count[2] = {0, 0};         // pairs of even / odd rounds
+  unsigned long long* ex_stats = nullptr;   // [ncases][2] attempts, accepts with the next rung
+  long long* ex_walker = nullptr;       // [chains] walker label of each slot
+  int* ex_wstate = nullptr;             // [chains] round-trip state by walker
+  long long* ex_trips = nullptr;        // [chains] round trips by walker
+  int64_t ex_round = 0;                 // exchange rounds since pmc_set_ladders
+  double* tt_out[3] = {nullptr, nullptr, nullptr};   // traj, roll, state rows of a whole pmc_run_tempering*
+  size_t tt_cap[3] = {0, 0, 0};
 };
 
 // Device memory of the handles comes from a per-device cache of freed blocks: a study creates and destroys one handle
@@ -153,3 +169,6 @@ int launch_run_lane(pmc_handle* h, const pmc::RunArgs& a);                   // 
 int launch_run_cluster_cta(pmc_handle* h, const pmc::RunArgs& a);            // run_cluster_cta.cu
 int launch_delta_segment_cta(pmc_handle* h, const pmc::SegDeltaArgs& a);     // run_cluster_cta.cu
 int launch_run_cluster_lane(pmc_handle* h, const pmc::RunArgs& a);           // run_cluster_lane.cu
+int launch_exchange(pmc_handle* h, const pmc::ExchangeArgs& a, int64_t npairs);   // exchange.cu
+int launch_place_rows(pmc_handle* h, double* dst, const double* src, int64_t rows, int64_t rows_total, int64_t row0,
+                      int cols);                                             // exchange.cu

@@ -3,6 +3,7 @@
 // No CPU fallback: every compute entry point needs a CUDA device and reports
 // PMC_ERR_NO_DEVICE / PMC_ERR_CUDA otherwise.
 #include "handle.h"
+#include "exchange.cuh"
 
 namespace {
 
@@ -504,6 +505,9 @@ void pmc_destroy(pmc_handle* h) {
   if (h->pair_work) pmc_pool_free(h->pair_work);
   if (h->pair_order) pmc_pool_free(h->pair_order);
   if (h->pair_next) pmc_pool_free(h->pair_next);
+  for (void* p : {(void*)h->ex_pairs, (void*)h->ex_stats, (void*)h->ex_walker, (void*)h->ex_wstate, (void*)h->ex_trips,
+                  (void*)h->tt_out[0], (void*)h->tt_out[1], (void*)h->tt_out[2]})
+    if (p) pmc_pool_free(p);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   delete h;
@@ -737,6 +741,45 @@ int32_t pmc_run_ex(pmc_handle* h, int64_t nsteps, int64_t stepout, double* traj,
   return run_impl(h, nsteps, stepout, traj, roll19, 19, state);
 }
 
+// The shared step counter (one copy, so the row counts of the next launches are known on the host).
+static int fetch_step0(pmc_handle* h) {
+  ChainDyn d0;
+  PMC_CU(cudaMemcpyAsync(&d0, h->dyn, sizeof(ChainDyn), cudaMemcpyDeviceToHost, h->stream));
+  PMC_CU(cudaStreamSynchronize(h->stream));
+  if (h->host_dyn.empty()) h->host_dyn.resize((size_t)h->nchains);
+  h->host_dyn[0] = d0;
+  return PMC_OK;
+}
+
+static int grow(double** buf, size_t* cap, size_t doubles) {
+  if (doubles <= *cap) return PMC_OK;
+  if (*buf) pmc_pool_free(*buf);
+  *buf = nullptr; *cap = 0;
+  PMC_CU(pool_alloc(buf, doubles * sizeof(double)));
+  *cap = doubles;
+  return PMC_OK;
+}
+
+// Device row buffers of one launch of `rows` rows and the launch arguments of the run kernels.
+static int run_args(pmc_handle* h, int64_t nsteps, int64_t stepout, int64_t rows, int roll_cols, bool want_state,
+                    RunArgs& a) {
+  const size_t ntraj = (size_t)h->nchains * (size_t)rows * 8, nroll = (size_t)h->nchains * (size_t)rows * roll_cols;
+  const size_t nstate = want_state ? (size_t)h->nchains * (size_t)rows * 2 * (size_t)h->n : 0;
+  int rc;
+  if ((rc = grow(&h->state, &h->state_cap, nstate))) return rc;
+  if ((rc = grow(&h->traj, &h->traj_cap, ntraj))) return rc;
+  if ((rc = grow(&h->roll, &h->roll_cap, nroll))) return rc;
+  a = RunArgs{};
+  a.mono = h->mono; a.par = h->par; a.dyn = h->dyn;
+  a.traj = h->traj; a.roll = h->roll;
+  a.nsteps = nsteps; a.stepout = stepout; a.rows = rows;
+  a.seed = h->seed; a.chain_id_base = h->chain_id_base;
+  a.n = h->n; a.nchains = (int)h->nchains; a.energy_type = h->energy_type;
+  a.dynx = h->dynx; a.state = nstate ? h->state : nullptr; a.roll_cols = roll_cols;
+  a.compensated = h->compensated;
+  return PMC_OK;
+}
+
 static int run_impl(pmc_handle* h, int64_t nsteps, int64_t stepout, double* traj, double* roll, int roll_cols,
                     double* state) {
   int rc = check_handle(h);
@@ -747,42 +790,12 @@ static int run_impl(pmc_handle* h, int64_t nsteps, int64_t stepout, double* traj
   // re-synchronise running scalars against a full recompute (records drift, SURVEY §7 "hard parts")
   if ((rc = refresh(h, false))) return rc;
   // step0 (shared by all chains) decides the row count
-  {
-    ChainDyn d0;
-    PMC_CU(cudaMemcpyAsync(&d0, h->dyn, sizeof(ChainDyn), cudaMemcpyDeviceToHost, h->stream));
-    PMC_CU(cudaStreamSynchronize(h->stream));
-    if (h->host_dyn.empty()) h->host_dyn.resize((size_t)h->nchains);
-    h->host_dyn[0] = d0;
-  }
+  if ((rc = fetch_step0(h))) return rc;
   const int64_t rows = pmc_rows_for(h, nsteps, stepout);
   const size_t ntraj = (size_t)h->nchains * (size_t)rows * 8, nroll = (size_t)h->nchains * (size_t)rows * roll_cols;
   const size_t nstate = state ? (size_t)h->nchains * (size_t)rows * 2 * (size_t)h->n : 0;
-  if (nstate > h->state_cap) {
-    if (h->state) pmc_pool_free(h->state);
-    h->state = nullptr; h->state_cap = 0;
-    PMC_CU(pool_alloc(&h->state, nstate * sizeof(double)));
-    h->state_cap = nstate;
-  }
-  if (ntraj > h->traj_cap) {
-    if (h->traj) pmc_pool_free(h->traj);
-    h->traj = nullptr; h->traj_cap = 0;
-    PMC_CU(pool_alloc(&h->traj, ntraj * sizeof(double)));
-    h->traj_cap = ntraj;
-  }
-  if (nroll > h->roll_cap) {
-    if (h->roll) pmc_pool_free(h->roll);
-    h->roll = nullptr; h->roll_cap = 0;
-    PMC_CU(pool_alloc(&h->roll, nroll * sizeof(double)));
-    h->roll_cap = nroll;
-  }
-  RunArgs a{};
-  a.mono = h->mono; a.par = h->par; a.dyn = h->dyn;
-  a.traj = h->traj; a.roll = h->roll;
-  a.nsteps = nsteps; a.stepout = stepout; a.rows = rows;
-  a.seed = h->seed; a.chain_id_base = h->chain_id_base;
-  a.n = h->n; a.nchains = (int)h->nchains; a.energy_type = h->energy_type;
-  a.dynx = h->dynx; a.state = nstate ? h->state : nullptr; a.roll_cols = roll_cols;
-  a.compensated = h->compensated;
+  RunArgs a;
+  if ((rc = run_args(h, nsteps, stepout, rows, roll_cols, state != nullptr, a))) return rc;
   PMC_CU(cudaEventRecord(h->ev0, h->stream));
   if ((rc = dispatch_run(h, a))) return rc;
   // FP32 rectangle: the running energy is the sum of FP32-rounded ΔU of the accepted moves; put it back on the exact
@@ -1009,6 +1022,206 @@ int32_t pmc_cluster_stats(pmc_handle* h, double* out) {
   return PMC_OK;
 }
 
+// ---- replica exchange ---------------------------------------------------------------------------------------
+namespace {
+
+// PMC_CU that yields the status instead of returning it (for clean-up on failure)
+int cu_rc(cudaError_t e, const char* what) {
+  if (e == cudaSuccess) return PMC_OK;
+  cudaGetLastError();
+  return fail(e == cudaErrorMemoryAllocation ? PMC_ERR_NOMEM : PMC_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
+}
+#define PMC_CU_RC(expr) cu_rc((expr), #expr)
+
+void ladder_clear(pmc_handle* h) {
+  for (void* p : {(void*)h->ex_pairs, (void*)h->ex_stats, (void*)h->ex_walker, (void*)h->ex_wstate, (void*)h->ex_trips})
+    if (p) pmc_pool_free(p);
+  h->ex_pairs = nullptr; h->ex_stats = nullptr; h->ex_walker = nullptr; h->ex_wstate = nullptr; h->ex_trips = nullptr;
+  h->ex_count[0] = h->ex_count[1] = 0;
+  h->ex_round = 0;
+  h->ladder.clear();
+}
+
+// The name of the first field in which two rungs of one ladder differ although it enters the energy or the target
+// density, or nullptr.
+const char* rung_mismatch(const pmc_case& x, const pmc_case& y) {
+#define PMC_SAME(f) if (x.f != y.f) return #f;
+  PMC_SAME(E0) PMC_SAME(K1) PMC_SAME(K2) PMC_SAME(mu) PMC_SAME(b) PMC_SAME(n) PMC_SAME(chain_type) PMC_SAME(energy_type)
+  PMC_SAME(kappa) PMC_SAME(psi0) PMC_SAME(cutoff_radius) PMC_SAME(cutoff_full) PMC_SAME(clustering) PMC_SAME(planar)
+#undef PMC_SAME
+  return nullptr;
+}
+
+// One round: the pairs of parity round & 1 of every ladder and replica column.
+int exchange_round(pmc_handle* h) {
+  const int parity = (int)(h->ex_round & 1);
+  ExchangeArgs a{};
+  a.mono = h->mono; a.par = h->par; a.dyn = h->dyn; a.dynx = h->dynx;
+  a.pairs = h->ex_pairs + (parity ? h->ex_count[0] : 0);
+  a.stats = h->ex_stats; a.walker = h->ex_walker; a.wstate = h->ex_wstate; a.trips = h->ex_trips;
+  a.accepted = h->flags;
+  a.seed = h->seed; a.chain_id_base = h->chain_id_base; a.n = h->n; a.round = h->ex_round;
+  int rc = launch_exchange(h, a, h->ex_count[parity]);
+  if (rc) return rc;
+  h->ex_round += 1;
+  h->dyn_fresh = h->dynx_fresh = false;
+  return PMC_OK;
+}
+
+int tempering_impl(pmc_handle* h, int64_t nsteps, int64_t every, int64_t stepout, double* traj, double* roll,
+                   int roll_cols, double* state) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (h->ladder.empty()) return fail(PMC_ERR_INVALID, "no ladders set (pmc_set_ladders)");
+  if (nsteps < 0) return fail(PMC_ERR_INVALID, "nsteps must be >= 0");
+  if (nsteps == 0) return PMC_OK;
+  if (nsteps >= (1LL << 40)) return fail(PMC_ERR_INVALID, "nsteps must stay below 2^40");
+  if (every < 1 || nsteps % every != 0) return fail(PMC_ERR_INVALID, "exchange_every must divide nsteps");
+  if (stepout > 0 && every % stepout != 0) return fail(PMC_ERR_INVALID, "stepout must divide exchange_every, or be 0");
+  if ((rc = fetch_step0(h))) return rc;   // the only copy to the host before the results
+  const int64_t rows_total = pmc_rows_for(h, nsteps, stepout), rows = stepout > 0 ? every / stepout : 0;
+  const size_t per_row[3] = {8, (size_t)roll_cols, 2 * (size_t)h->n};
+  double* host_out[3] = {traj, roll, state};
+  for (int k = 0; k < 3; ++k)
+    if (host_out[k] && rows_total > 0 &&
+        (rc = grow(&h->tt_out[k], &h->tt_cap[k], (size_t)h->nchains * (size_t)rows_total * per_row[k])))
+      return rc;
+  RunArgs a;
+  if ((rc = run_args(h, every, stepout, rows, roll_cols, state != nullptr, a))) return rc;
+  const double* chunk_out[3] = {h->traj, h->roll, h->state};
+  PMC_CU(cudaEventRecord(h->ev0, h->stream));
+  for (int64_t k = 0; k < nsteps / every; ++k) {   // exactly pmc_run(every) followed by pmc_exchange, k times
+    if ((rc = refresh(h, false))) return rc;
+    if ((rc = dispatch_run(h, a))) return rc;
+    if (use_f32_rect(h) && (rc = refresh(h, /*rebind_gauge=*/false))) return rc;
+    for (int j = 0; j < 3; ++j)
+      if (host_out[j] && rows > 0 &&
+          (rc = launch_place_rows(h, h->tt_out[j], chunk_out[j], rows, rows_total, k * rows, (int)per_row[j])))
+        return rc;
+    if ((rc = exchange_round(h))) return rc;
+  }
+  PMC_CU(cudaEventRecord(h->ev1, h->stream));
+  for (int k = 0; k < 3; ++k)
+    if (host_out[k] && rows_total > 0)
+      PMC_CU(cudaMemcpyAsync(host_out[k], h->tt_out[k], (size_t)h->nchains * (size_t)rows_total * per_row[k] * sizeof(double),
+                             cudaMemcpyDeviceToHost, h->stream));
+  PMC_CU(cudaStreamSynchronize(h->stream));
+  PMC_CU(cudaEventElapsedTime(&h->last_ms, h->ev0, h->ev1));
+  h->host_dyn[0].step += nsteps;
+  return PMC_OK;
+}
+
+}  // namespace
+
+int32_t pmc_set_ladders(pmc_handle* h, const int32_t* rungs, int64_t len) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (len < 0 || (len > 0 && !rungs)) return fail(PMC_ERR_INVALID, "null or negative-length rung list");
+  const int64_t ncases = (int64_t)h->cases.size(), R = h->replicas;
+  std::vector<std::vector<int32_t>> ladders(1);
+  for (int64_t i = 0; i < len; ++i) {
+    if (rungs[i] == -1) {
+      if (ladders.back().empty()) return fail(PMC_ERR_INVALID, "empty ladder in the rung list");
+      if (i + 1 < len) ladders.emplace_back();
+      continue;
+    }
+    if (rungs[i] < 0 || rungs[i] >= ncases) return fail(PMC_ERR_INVALID, "rung " + std::to_string(rungs[i]) +
+                                                                             " is not a case index of this handle");
+    ladders.back().push_back(rungs[i]);
+  }
+  if (len == 0) ladders.clear();
+  std::vector<char> seen((size_t)ncases, 0);
+  for (const auto& L : ladders) {
+    if (L.size() < 2) return fail(PMC_ERR_INVALID, "a ladder needs at least two rungs");
+    for (int32_t c : L) {
+      if (seen[(size_t)c]) return fail(PMC_ERR_INVALID, "case " + std::to_string(c) + " appears more than once in the ladders");
+      seen[(size_t)c] = 1;
+      const pmc_case& x = h->cases[(size_t)c];
+      const pmc_case& y = h->cases[(size_t)L[0]];
+      if (x.umbrella) return fail(PMC_ERR_INVALID, "umbrella sampling cannot be tempered: its weights depend on kT and F");
+      if (const char* f = rung_mismatch(x, y))
+        return fail(PMC_ERR_INVALID, std::string("rungs of one ladder must agree on ") + f + " (cases " +
+                                         std::to_string(L[0]) + " and " + std::to_string(c) + ")");
+      if (x.energy_type == PMC_ENERGY_CUTOFF && !x.cutoff_full && (x.Fz != y.Fz || x.Fx != y.Fx))
+        return fail(PMC_ERR_INVALID, "a force ladder needs F in the energy: the cut-off energy without cutoff_full has no -r.F");
+    }
+  }
+  // pairs of even rounds first, then those of odd rounds; both lists are walked in ladder, rung, replica order
+  std::vector<ExPair> pairs[2];
+  std::vector<int> wstate((size_t)h->nchains, 0);
+  for (const auto& L : ladders) {
+    const int m = (int)L.size();
+    for (int64_t r = 0; r < R; ++r) wstate[(size_t)(L[0] * R + r)] = 1;
+    for (int i = 0; i + 1 < m; ++i)
+      for (int64_t r = 0; r < R; ++r)
+        pairs[i & 1].push_back(ExPair{(int)(L[i] * R + r), (int)(L[i + 1] * R + r), L[i],
+                                      (i == 0 ? 1 : 0) | (i + 2 == m ? 2 : 0)});
+  }
+  ladder_clear(h);
+  if (ladders.empty()) return PMC_OK;
+  const size_t c = (size_t)h->nchains, np = pairs[0].size() + pairs[1].size();
+  std::vector<long long> walker(c);
+  for (size_t i = 0; i < c; ++i) walker[i] = (long long)h->chain_id_base + (long long)i;
+  pairs[0].insert(pairs[0].end(), pairs[1].begin(), pairs[1].end());
+  auto undo = [&](int code) { ladder_clear(h); return code; };
+  if ((rc = PMC_CU_RC(pool_alloc(&h->ex_pairs, np * sizeof(ExPair))))) return undo(rc);
+  if ((rc = PMC_CU_RC(pool_alloc(&h->ex_stats, (size_t)ncases * 2 * sizeof(unsigned long long))))) return undo(rc);
+  if ((rc = PMC_CU_RC(pool_alloc(&h->ex_walker, c * sizeof(long long))))) return undo(rc);
+  if ((rc = PMC_CU_RC(pool_alloc(&h->ex_wstate, c * sizeof(int))))) return undo(rc);
+  if ((rc = PMC_CU_RC(pool_alloc(&h->ex_trips, c * sizeof(long long))))) return undo(rc);
+  if ((rc = PMC_CU_RC(cudaMemcpyAsync(h->ex_pairs, pairs[0].data(), np * sizeof(ExPair), cudaMemcpyHostToDevice, h->stream))) ||
+      (rc = PMC_CU_RC(cudaMemsetAsync(h->ex_stats, 0, (size_t)ncases * 2 * sizeof(unsigned long long), h->stream))) ||
+      (rc = PMC_CU_RC(cudaMemcpyAsync(h->ex_walker, walker.data(), c * sizeof(long long), cudaMemcpyHostToDevice, h->stream))) ||
+      (rc = PMC_CU_RC(cudaMemcpyAsync(h->ex_wstate, wstate.data(), c * sizeof(int), cudaMemcpyHostToDevice, h->stream))) ||
+      (rc = PMC_CU_RC(cudaMemsetAsync(h->ex_trips, 0, c * sizeof(long long), h->stream))) ||
+      (rc = PMC_CU_RC(cudaStreamSynchronize(h->stream))))   // the host vectors are pageable and local
+    return undo(rc);
+  h->ex_count[0] = (int64_t)(np - pairs[1].size());
+  h->ex_count[1] = (int64_t)pairs[1].size();
+  h->ladder.assign(rungs, rungs + len);
+  return PMC_OK;
+}
+
+int32_t pmc_exchange(pmc_handle* h, int32_t* accepted) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (h->ladder.empty()) return fail(PMC_ERR_INVALID, "no ladders set (pmc_set_ladders)");
+  PMC_CU(cudaMemsetAsync(h->flags, 0, (size_t)h->nchains * sizeof(int), h->stream));
+  if ((rc = exchange_round(h))) return rc;
+  if (accepted)
+    PMC_CU(cudaMemcpyAsync(accepted, h->flags, (size_t)h->nchains * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  PMC_CU(cudaStreamSynchronize(h->stream));
+  return PMC_OK;
+}
+
+int32_t pmc_run_tempering(pmc_handle* h, int64_t nsteps, int64_t exchange_every, int64_t stepout, double* traj,
+                          double* roll) {
+  return tempering_impl(h, nsteps, exchange_every, stepout, traj, roll, 17, nullptr);
+}
+
+int32_t pmc_run_tempering_ex(pmc_handle* h, int64_t nsteps, int64_t exchange_every, int64_t stepout, double* traj,
+                             double* roll19, double* state) {
+  if (h && !h->cluster_mode)
+    return fail(PMC_ERR_INVALID, "pmc_run_tempering_ex needs a clustering-driver handle (clustering, bend-mod or cutoff case)");
+  return tempering_impl(h, nsteps, exchange_every, stepout, traj, roll19, 19, state);
+}
+
+int32_t pmc_exchange_stats(pmc_handle* h, double* pair_stats, int64_t* walker, int64_t* round_trips) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (h->ladder.empty()) return fail(PMC_ERR_INVALID, "no ladders set (pmc_set_ladders)");
+  const size_t ncases = h->cases.size(), c = (size_t)h->nchains;
+  std::vector<unsigned long long> st(ncases * 2);
+  PMC_CU(cudaMemcpyAsync(st.data(), h->ex_stats, st.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
+  static_assert(sizeof(long long) == sizeof(int64_t), "walker labels are 64-bit");
+  if (walker) PMC_CU(cudaMemcpyAsync(walker, h->ex_walker, c * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+  if (round_trips) PMC_CU(cudaMemcpyAsync(round_trips, h->ex_trips, c * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+  PMC_CU(cudaStreamSynchronize(h->stream));
+  if (pair_stats)
+    for (size_t i = 0; i < st.size(); ++i) pair_stats[i] = (double)st[i];
+  return PMC_OK;
+}
+
 // ---- checkpoint / resume ---------------------------------------------------------------------------------
 namespace {
 struct CkptHeader {
@@ -1021,12 +1234,30 @@ struct CkptHeader {
   int64_t host_step;
 };
 constexpr uint64_t kCkptMagic = 0x3354504b43434d50ull;
+// Trailing block of a handle with ladders: this header, the rung list (int32), the pair statistics ([ncases][2] uint64),
+// the walker labels (int64), the round-trip states (int32) and counts (int64) of every chain.
+struct LadderHeader {
+  uint64_t magic;        // "PMCLADR1"
+  int64_t len, ncases, nchains, round;
+};
+constexpr uint64_t kLadderMagic = 0x315244414c434d50ull;
+
+size_t ckpt_base_bytes(const pmc_handle* h) {
+  const size_t c = (size_t)h->nchains;
+  return sizeof(CkptHeader) + c * (size_t)h->n * sizeof(MonoRec) + c * sizeof(ChainDyn) + c * sizeof(ChainDynX);
+}
+
+size_t ladder_block_bytes(const pmc_handle* h) {
+  if (h->ladder.empty()) return 0;
+  const size_t c = (size_t)h->nchains;
+  return sizeof(LadderHeader) + h->ladder.size() * sizeof(int32_t) + h->cases.size() * 2 * sizeof(unsigned long long) +
+         c * (sizeof(long long) + sizeof(int) + sizeof(long long));
+}
 }  // namespace
 
 int64_t pmc_checkpoint_bytes(const pmc_handle* h) {
   if (!h) return 0;
-  const size_t c = (size_t)h->nchains;
-  return (int64_t)(sizeof(CkptHeader) + c * (size_t)h->n * sizeof(MonoRec) + c * sizeof(ChainDyn) + c * sizeof(ChainDynX));
+  return (int64_t)(ckpt_base_bytes(h) + ladder_block_bytes(h));
 }
 
 int32_t pmc_checkpoint_save(pmc_handle* h, void* buf, int64_t bytes) {
@@ -1045,6 +1276,22 @@ int32_t pmc_checkpoint_save(pmc_handle* h, void* buf, int64_t bytes) {
   PMC_CU(cudaMemcpyAsync(p, h->mono, nm, cudaMemcpyDeviceToHost, h->stream));
   PMC_CU(cudaMemcpyAsync(p + nm, h->dyn, c * sizeof(ChainDyn), cudaMemcpyDeviceToHost, h->stream));
   PMC_CU(cudaMemcpyAsync(p + nm + c * sizeof(ChainDyn), h->dynx, c * sizeof(ChainDynX), cudaMemcpyDeviceToHost, h->stream));
+  if (!h->ladder.empty()) {
+    unsigned char* q = static_cast<unsigned char*>(buf) + ckpt_base_bytes(h);
+    const LadderHeader lh{kLadderMagic, (int64_t)h->ladder.size(), (int64_t)h->cases.size(), h->nchains, h->ex_round};
+    std::memcpy(q, &lh, sizeof(lh));
+    q += sizeof(lh);
+    std::memcpy(q, h->ladder.data(), h->ladder.size() * sizeof(int32_t));
+    q += h->ladder.size() * sizeof(int32_t);
+    const size_t ns = h->cases.size() * 2 * sizeof(unsigned long long);
+    PMC_CU(cudaMemcpyAsync(q, h->ex_stats, ns, cudaMemcpyDeviceToHost, h->stream));
+    q += ns;
+    PMC_CU(cudaMemcpyAsync(q, h->ex_walker, c * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+    q += c * sizeof(long long);
+    PMC_CU(cudaMemcpyAsync(q, h->ex_wstate, c * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    q += c * sizeof(int);
+    PMC_CU(cudaMemcpyAsync(q, h->ex_trips, c * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
+  }
   PMC_CU(cudaStreamSynchronize(h->stream));
   return PMC_OK;
 }
@@ -1059,9 +1306,22 @@ int32_t pmc_checkpoint_load(pmc_handle* h, const void* buf, int64_t bytes) {
   if (hd.n != h->n || hd.nchains != h->nchains || hd.energy_type != h->energy_type || hd.cluster_mode != h->cluster_mode ||
       hd.planar != h->planar || hd.seed != h->seed || hd.chain_id_base != h->chain_id_base)
     return fail(PMC_ERR_INVALID, "checkpoint belongs to a different ensemble (n, chains, energy type, seed or chain ids differ)");
-  if (bytes < pmc_checkpoint_bytes(h)) return fail(PMC_ERR_INVALID, "truncated checkpoint");
+  if (bytes < (int64_t)ckpt_base_bytes(h)) return fail(PMC_ERR_INVALID, "truncated checkpoint");
   const unsigned char* p = static_cast<const unsigned char*>(buf) + sizeof(hd);
   const size_t c = (size_t)h->nchains, nm = c * (size_t)h->n * sizeof(MonoRec);
+  // the ladder block, validated before anything is loaded
+  const unsigned char* q = static_cast<const unsigned char*>(buf) + ckpt_base_bytes(h);
+  LadderHeader lh{};
+  if (bytes >= (int64_t)(ckpt_base_bytes(h) + sizeof(lh))) std::memcpy(&lh, q, sizeof(lh));
+  if (h->ladder.empty() && lh.magic == kLadderMagic)
+    return fail(PMC_ERR_INVALID, "checkpoint holds replica-exchange ladders; set the same ladders before loading it");
+  if (!h->ladder.empty()) {
+    if (lh.magic != kLadderMagic) return fail(PMC_ERR_INVALID, "checkpoint has no replica-exchange ladders; this handle has");
+    if (bytes < pmc_checkpoint_bytes(h)) return fail(PMC_ERR_INVALID, "truncated checkpoint");
+    if (lh.len != (int64_t)h->ladder.size() || lh.ncases != (int64_t)h->cases.size() || lh.nchains != h->nchains ||
+        std::memcmp(q + sizeof(lh), h->ladder.data(), h->ladder.size() * sizeof(int32_t)) != 0)
+      return fail(PMC_ERR_INVALID, "checkpoint ladders differ from this handle's (pmc_set_ladders)");
+  }
   if (hd.kT_scale != h->kT_scale) {  // the stage temperature lives in the per-chain constants
     std::vector<ChainParams> par(c);
     for (size_t i = 0; i < c; ++i) par[i] = params_of(h->cases[i / (size_t)h->replicas], hd.kT_scale);
@@ -1072,6 +1332,18 @@ int32_t pmc_checkpoint_load(pmc_handle* h, const void* buf, int64_t bytes) {
   PMC_CU(cudaMemcpyAsync(h->mono, p, nm, cudaMemcpyHostToDevice, h->stream));
   PMC_CU(cudaMemcpyAsync(h->dyn, p + nm, c * sizeof(ChainDyn), cudaMemcpyHostToDevice, h->stream));
   PMC_CU(cudaMemcpyAsync(h->dynx, p + nm + c * sizeof(ChainDyn), c * sizeof(ChainDynX), cudaMemcpyHostToDevice, h->stream));
+  if (!h->ladder.empty()) {
+    q += sizeof(lh) + h->ladder.size() * sizeof(int32_t);
+    const size_t ns = h->cases.size() * 2 * sizeof(unsigned long long);
+    PMC_CU(cudaMemcpyAsync(h->ex_stats, q, ns, cudaMemcpyHostToDevice, h->stream));
+    q += ns;
+    PMC_CU(cudaMemcpyAsync(h->ex_walker, q, c * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    q += c * sizeof(long long);
+    PMC_CU(cudaMemcpyAsync(h->ex_wstate, q, c * sizeof(int), cudaMemcpyHostToDevice, h->stream));
+    q += c * sizeof(int);
+    PMC_CU(cudaMemcpyAsync(h->ex_trips, q, c * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
+    h->ex_round = lh.round;
+  }
   PMC_CU(cudaStreamSynchronize(h->stream));
   h->init = hd.init;
   h->dyn_fresh = h->dynx_fresh = false;

@@ -41,6 +41,8 @@ EXPORTS = [
     "pmc_multi_set_state_all", "pmc_multi_get_state_all", "pmc_multi_rows_for", "pmc_multi_run", "pmc_multi_run_ex",
     "pmc_multi_run_async", "pmc_multi_wait", "pmc_multi_gather", "pmc_multi_last_run_ms", "pmc_multi_launch_count",
     "pmc_release_cached_memory",
+    # replica exchange across kT / force ladders of one handle
+    "pmc_set_ladders", "pmc_exchange", "pmc_run_tempering", "pmc_run_tempering_ex", "pmc_exchange_stats",
 ]
 RESULT_COLS = 24
 RESULT_NAMES = AVG_NAMES + ["acc_rate", "normalizer", "phi_step", "theta_step", "trials", "U_running", "Ealign", "psi"]
@@ -230,6 +232,12 @@ def load():
     L.pmc_multi_last_run_ms.argtypes = [hp, C.POINTER(C.c_float)]
     L.pmc_multi_launch_count.argtypes = [hp]
     L.pmc_multi_launch_count.restype = C.c_int64
+    i64p = C.POINTER(C.c_int64)
+    L.pmc_set_ladders.argtypes = [hp, C.POINTER(C.c_int32), C.c_int64]
+    L.pmc_exchange.argtypes = [hp, C.POINTER(C.c_int32)]
+    L.pmc_run_tempering.argtypes = [hp, C.c_int64, C.c_int64, C.c_int64, dp, dp]
+    L.pmc_run_tempering_ex.argtypes = [hp, C.c_int64, C.c_int64, C.c_int64, dp, dp, dp]
+    L.pmc_exchange_stats.argtypes = [hp, dp, i64p, i64p]
     for name in EXPORTS:
         f = getattr(L, name)
         if f.restype is C.c_int:  # default restype: every status-returning entry point
@@ -491,6 +499,58 @@ class Ensemble:
         o = np.empty((self.nchains, 3))
         _check(load().pmc_cluster_stats(self._h, _dp(o)))
         return o
+
+    # ---- replica exchange across kT / force ladders (include/polymc.h, DESIGN.md §12) ----
+    def set_ladders(self, ladders):
+        """ladders: a list of lists of case indices, each in rung order (e.g. by increasing kT); [] clears.  Resets
+        the round counter and the exchange diagnostics."""
+        flat = []
+        for lad in ladders:
+            flat += [int(c) for c in lad] + [-1]
+        arr = (C.c_int32 * max(1, len(flat)))(*flat)
+        _check(load().pmc_set_ladders(self._h, arr, len(flat)))
+
+    def exchange(self):
+        """One exchange round; returns accepted [chains] (1 at the lower slot of every accepted pair)."""
+        flags = (C.c_int32 * self.nchains)()
+        _check(load().pmc_exchange(self._h, flags))
+        return np.frombuffer(flags, dtype=np.int32).copy()
+
+    def _tempering_rows(self, nsteps, exchange_every, stepout, fetch_rows, cols, want_state):
+        if exchange_every < 1 or nsteps % exchange_every:
+            raise PolymcError(-1, "exchange_every must divide nsteps")
+        rows = self.rows_for(nsteps, stepout)
+        if not (fetch_rows and rows > 0):
+            return None, None, None
+        return (np.empty((self.nchains, rows, 8)), np.empty((self.nchains, rows, cols)),
+                np.empty((self.nchains, rows, 2 * self.n)) if want_state else None)
+
+    def run_tempering(self, nsteps, exchange_every, stepout=0, fetch_rows=True):
+        """run(exchange_every) followed by exchange(), nsteps / exchange_every times, on the device without host
+        synchronisation between the chunks.  Returns (traj [chains][rows][8], roll [chains][rows][17]) as run()."""
+        traj, roll, _ = self._tempering_rows(nsteps, exchange_every, stepout, fetch_rows, 17, False)
+        _check(load().pmc_run_tempering(self._h, nsteps, exchange_every, stepout, _dp(traj), _dp(roll)))
+        return traj, roll
+
+    def run_tempering_ex(self, nsteps, exchange_every, stepout=0, fetch_rows=True, want_state=False):
+        """The clustering driver's run_ex(exchange_every) followed by exchange(), repeated; rows as run_ex()."""
+        traj, roll, state = self._tempering_rows(nsteps, exchange_every, stepout, fetch_rows, 19, want_state)
+        _check(load().pmc_run_tempering_ex(self._h, nsteps, exchange_every, stepout, _dp(traj), _dp(roll), _dp(state)))
+        return traj, roll, state
+
+    def exchange_stats(self):
+        """-> dict(attempts [ncases], accepts [ncases]: with the next rung, summed over replicas; walker [chains]:
+        global chain id of the initial configuration each slot holds; round_trips [chains]: by walker)."""
+        ncases = len(self.cases)
+        if ncases * self.replicas != self.nchains:
+            raise PolymcError(-1, "exchange_stats needs the handle's case list (a MultiEnsemble shard has none)")
+        ps = np.empty((ncases, 2))
+        walker = np.empty(self.nchains, dtype=np.int64)
+        trips = np.empty(self.nchains, dtype=np.int64)
+        i64p = C.POINTER(C.c_int64)
+        _check(load().pmc_exchange_stats(self._h, _dp(ps), walker.ctypes.data_as(i64p), trips.ctypes.data_as(i64p)))
+        return {"attempts": ps[:, 0].astype(np.int64), "accepts": ps[:, 1].astype(np.int64), "walker": walker,
+                "round_trips": trips}
 
 
 class _Shard(Ensemble):

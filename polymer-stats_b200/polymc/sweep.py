@@ -40,6 +40,35 @@ def bucket_cases(cases):
     return buckets
 
 
+TEMPER_FIELDS = ("kT", "Fz", "Fx")
+
+
+def tempering_ladders(cases, temper: str):
+    """Replica-exchange ladders of a sweep: cases that agree on every field except `temper` ("kT", "Fz" or "Fx")
+    form one ladder, ordered by increasing `temper`.  -> list of lists of case indices.  Refuses umbrella sampling
+    (its weights depend on kT and F), a ladder of one rung and two rungs with the same value."""
+    if temper not in TEMPER_FIELDS:
+        raise lib.PolymcError(-1, f"temper must be one of {', '.join(TEMPER_FIELDS)} (got {temper!r})")
+    rec = cases.rec if isinstance(cases, lib.CaseTable) else lib.CaseTable(cases).rec
+    if np.any(rec["umbrella"] != 0):
+        raise lib.PolymcError(-1, "umbrella sampling cannot be tempered: its weights depend on kT and F")
+    rest = rec.copy()
+    rest[temper] = 0.0           # every other field, byte for byte, is the key of the ladder
+    groups = OrderedDict()
+    for i in range(rest.shape[0]):
+        groups.setdefault(rest[i].tobytes(), []).append(i)
+    ladders = []
+    for idx in groups.values():
+        vals = rec[temper][idx]
+        if len(idx) < 2:
+            raise lib.PolymcError(-1, f"case {idx[0]} has no partner that differs only in {temper}: a ladder needs at "
+                                      "least two rungs")
+        if len(np.unique(vals)) != len(vals):
+            raise lib.PolymcError(-1, f"cases {idx} repeat a value of {temper}: every rung of a ladder needs its own")
+        ladders.append([idx[k] for k in np.argsort(vals, kind="stable")])
+    return ladders
+
+
 def _dist():
     try:
         import torch.distributed as dist
@@ -110,16 +139,56 @@ def _segments(mine: np.ndarray, replicas: int):
                 pos += ncases * replicas
 
 
+def _local_ladders(ladders, case0: int, ncases: int):
+    """The ladders of a handle holding cases [case0, case0 + ncases), as its own case indices."""
+    local = []
+    for lad in ladders:
+        inside = [case0 <= c < case0 + ncases for c in lad]
+        if any(inside) and not all(inside):
+            raise lib.PolymcError(-1, f"the ladder of cases {lad} spans two handles (cases of different num-monomers "
+                                      "or energy-type interleave): list the tempered option's grid last")
+        if all(inside):
+            local.append([c - case0 for c in lad])
+    return local
+
+
+def _collect_exchange(exchange, st, ladders, case0: int, ncases: int, nrep: int):
+    exchange["attempts"][case0:case0 + ncases] += st["attempts"]
+    exchange["accepts"][case0:case0 + ncases] += st["accepts"]
+    for k, lad in enumerate(ladders):
+        if case0 <= lad[0] < case0 + ncases:    # walkers by their starting case: label − chain_id_base = chain index
+            walkers = np.concatenate([np.arange((c - case0) * nrep, (c - case0 + 1) * nrep) for c in lad])
+            exchange["round_trips"][k] += int(st["round_trips"][walkers].sum())
+
+
 def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0, device: int = 0,
-              rank: int = 0, world: int = 1, protocol=None, bit_identical: bool = False, pair_precision: str = "fp64"):
+              rank: int = 0, world: int = 1, protocol=None, bit_identical: bool = False, pair_precision: str = "fp64",
+              temper=None, exchange_every: int = 100, exchange=None):
     """Run this rank's contiguous block of every (n, energy) bucket.  Returns a list of
     (global chain ids of the bucket, lo, block [hi-lo][NCOL]).  No communication.
 
     protocol None: `nsteps` trials of mcmc_eap_chain.jl's loop.  protocol = dict(burn_in=…, schedule=[…]):
     the clustering driver's ladder (mcmc_clustering_eap_chain.jl:365-386) — a burn-in stage per kT
-    multiplier, then `nsteps` production trials at kT."""
+    multiplier, then `nsteps` production trials at kT.
+
+    temper "kT" / "Fz" / "Fx": replica exchange every `exchange_every` trials along the ladders of
+    tempering_ladders() in every run of the protocol (each init, each burn-in stage).  A ladder lives in one
+    handle, so this needs a single rank.  `exchange`, a dict, receives the ladders, the per-case attempts and
+    accepts with the next rung and the round trips of every ladder."""
     if not isinstance(cases, lib.CaseTable):
         cases = list(cases)
+    ladders = None
+    if temper is not None:
+        if world > 1:
+            raise lib.PolymcError(-1, "replica exchange needs a single rank: a ladder must live in one handle")
+        exchange_every = int(exchange_every)
+        lengths = [nsteps] + ([int(protocol.get("burn_in", 0))] if protocol and not protocol.get("plain") else [])
+        if exchange_every < 1 or any(k % exchange_every for k in lengths):
+            raise lib.PolymcError(-1, f"--exchange-every ({exchange_every}) must divide --num-steps and --burn-in")
+        ladders = tempering_ladders(cases, temper)
+        if exchange is not None:
+            exchange.update(ladders=ladders, attempts=np.zeros(len(cases), np.int64),
+                            accepts=np.zeros(len(cases), np.int64), round_trips=np.zeros(len(ladders), np.int64))
     out = []
     for (_, _), idxs in bucket_cases(cases).items():
         # global chain ids of this bucket, case-major
@@ -137,11 +206,22 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
                               chain_id_base=int(mine[pos]), ensemble_chains=len(gids) if bit_identical else 0) as ens:
                 if pair_precision != "fp64":   # opt-in FP32 rectangle where a kernel serves it (include/polymc.h)
                     ens.set_pair_precision(pair_precision)
+                local = None
+                if ladders is not None:
+                    local = _local_ladders(ladders, case0, ncases)
+                    ens.set_ladders(local)
+                run, run_ex = ens.run, ens.run_ex
+                if local:
+                    def run(k, so, fetch_rows):
+                        return ens.run_tempering(k, exchange_every, so, fetch_rows=fetch_rows)
+
+                    def run_ex(k, so, fetch_rows):
+                        return ens.run_tempering_ex(k, exchange_every, so, fetch_rows=fetch_rows)
                 if protocol is None or protocol.get("plain"):
                     # mcmc_eap_chain.jl:276-361: num-inits passes of nsteps trials with the re-initialisation rule between
                     inits = int(protocol.get("num_inits", 1)) if protocol else 1
                     for init in range(inits):
-                        ens.run(nsteps, stepout, fetch_rows=False)
+                        run(nsteps, stepout, fetch_rows=False)
                         if init + 1 < inits:
                             ens.reinit()
                 else:
@@ -149,10 +229,12 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
                         ens.init_x0(protocol["x0"], protocol["dx0"])
                     for mult in protocol.get("schedule", []):
                         ens.begin_stage(float(mult))
-                        ens.run_ex(int(protocol.get("burn_in", 0)), 0, fetch_rows=False)
+                        run_ex(int(protocol.get("burn_in", 0)), 0, fetch_rows=False)
                     ens.begin_stage(1.0)
-                    ens.run_ex(nsteps, 0, fetch_rows=False)
+                    run_ex(nsteps, 0, fetch_rows=False)
                     block[pos:end, 35:37] = ens.extra_accumulators()
+                if local and exchange is not None:
+                    _collect_exchange(exchange, ens.exchange_stats(), ladders, case0, ncases, nrep)
                 avg, ar, nrm = ens.averages()
                 block[pos:end, :16] = avg
                 block[pos:end, 16] = ar
@@ -183,29 +265,37 @@ def assemble(total: int, parts):
 
 
 def run_sweep(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0, device: int = 0,
-              torch_device=None, protocol=None, bit_identical: bool = False, pair_precision: str = "fp64"):
+              torch_device=None, protocol=None, bit_identical: bool = False, pair_precision: str = "fp64",
+              temper=None, exchange_every: int = 100):
     """Run every (case, replica) chain of a sweep for nsteps trials, sharded over the ranks of the
     current torch.distributed group (or a single process), then gather the final per-chain results on
-    every rank.  Chain order = case-major: avg [ncases*replicas][16], acc_rate, normalizer, sums [..][17]."""
+    every rank.  Chain order = case-major: avg [ncases*replicas][16], acc_rate, normalizer, sums [..][17].
+    With temper (run_shard), "exchange" holds the ladders and their exchange statistics."""
     dist = _dist()
     rank = dist.get_rank() if dist else 0
     world = dist.get_world_size() if dist else 1
     if not isinstance(cases, lib.CaseTable):
         cases = list(cases)
-    parts = []
+    parts, exchange = [], {}
     for gids, lo, block in run_shard(cases, replicas, nsteps, stepout, seed, device, rank, world, protocol, bit_identical,
-                                     pair_precision):
+                                     pair_precision, temper, exchange_every, exchange):
         parts.append((gids, gather_rows(block, len(gids), lo, device=torch_device)))
-    return assemble(len(cases) * replicas, parts)
+    res = assemble(len(cases) * replicas, parts)
+    if temper is not None:
+        res["exchange"] = exchange
+    return res
 
 
 def sweep_table(pargs_list, driver: str = "plain", runs: int = 1, seed: int = 0, device: int = 0, torch_device=None,
-                kappaflag: bool = False, pooled: bool = False, with_entries: bool = False, bit_identical: bool = False):
+                kappaflag: bool = False, pooled: bool = False, with_entries: bool = False, bit_identical: bool = False,
+                temper=None, exchange_every: int = 100, exchange=None):
     """A whole launcher + aggregate_mcmc.jl (+ reduce_tabular_data.jl) pipeline in one call (SURVEY §8f
     rank 3): every pargs dict of `pargs_list` is one case (one launcher command line), run `runs` times as
     independent replica chains (the launchers' `run-NNN` cases); the result is the aggregated table the
     reference's scripts would build from the `.out` files.  Returns (header, rows, entries) with entries =
-    [(prefix, stdout text)] for optional `.out` emission."""
+    [(prefix, stdout text)] for optional `.out` emission.  temper / exchange_every: replica exchange along the
+    ladders of the sweep (run_shard); the table keeps its format, a row per case being a row per rung.  `exchange`,
+    a dict, receives the ladders and their statistics (see exchange_rows)."""
     from . import aggregate as agg
     from . import mcmc as plain_host
     from . import mcmc_clustering as cl_host
@@ -251,7 +341,9 @@ def sweep_table(pargs_list, driver: str = "plain", runs: int = 1, seed: int = 0,
                                       "part of the file-name tokens (aggregate_mcmc.jl:40-57; use --kappaflag for bend-mod)")
         seen[pre] = i
     res = run_sweep(cases, runs, p0["num-steps"], 0, seed, device, torch_device, protocol, bit_identical,
-                    p0.get("pair-precision", "fp64"))
+                    p0.get("pair-precision", "fp64"), temper, exchange_every)
+    if exchange is not None and temper is not None:
+        exchange.update(res["exchange"])
     runflag = runs > 1
     entries, texts = [], []
     for i, p in enumerate(pargs_list):
@@ -272,3 +364,34 @@ def sweep_table(pargs_list, driver: str = "plain", runs: int = 1, seed: int = 0,
     if with_entries:  # [(prefix, output values)]: the input of agg.aggregate_by (scripts/aggregate_by.jl)
         return header, rows, texts, entries
     return header, rows, texts
+
+
+def exchange_rows(pargs_list, temper: str, exchange: dict, fixed=()):
+    """The replica-exchange table of a tempered sweep: one row per adjacent rung pair with the ladder's `fixed` options
+    (e.g. the other grid axes), the two rung values, attempts, accepts, acceptance rate and the ladder's round trips
+    (bottom → top → bottom, summed over its walkers).  -> (header, rows)."""
+    header = list(fixed) + [f"{temper}_lo", f"{temper}_hi", "attempts", "accepts", "rate", "round_trips"]
+    rows = []
+    for k, lad in enumerate(exchange["ladders"]):
+        p = pargs_list[lad[0]]
+        for lo, hi in zip(lad[:-1], lad[1:]):
+            att, acc = int(exchange["attempts"][lo]), int(exchange["accepts"][lo])
+            rows.append([p[f] for f in fixed] + [pargs_list[lo][temper], pargs_list[hi][temper], att, acc,
+                                                 acc / att if att else float("nan"), int(exchange["round_trips"][k])])
+    return header, rows
+
+
+def write_exchange_csv(path: str, header, rows):
+    """exchange_rows() as CSV: counts as integers, other numbers as Julia prints Float64, anything else as text."""
+    from .output import julia_float
+
+    def cell(x):
+        if isinstance(x, (bool, str)):
+            return str(x)
+        if isinstance(x, (int, np.integer)):
+            return str(int(x))
+        return julia_float(x)
+    with open(path, "w") as f:
+        f.write(",".join(header) + "\n")
+        for row in rows:
+            f.write(",".join(cell(x) for x in row) + "\n")

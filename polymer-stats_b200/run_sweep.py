@@ -44,7 +44,15 @@ def main(argv=None) -> int:
                     help="choose the launch shapes from the whole study instead of this rank's share: results are then the same "
                          "bit for bit for any number of GPUs (a share runs up to ~15 %% slower than in its own shape)")
     ap.add_argument("--device", type=int, default=0)
+    ap.add_argument("--temper", choices=["kT", "Fz", "Fx"], default=None,
+                    help="replica exchange (parallel tempering): cases that differ only in this option form one ladder, "
+                         "and neighbouring rungs swap configurations every --exchange-every trials")
+    ap.add_argument("--exchange-every", type=int, default=100, help="trials between two exchange rounds")
+    ap.add_argument("--exchange-out", default=None,
+                    help="CSV of the exchange statistics: one row per adjacent rung pair (needs --temper)")
     a = ap.parse_args(argv)
+    if a.exchange_out and not a.temper:
+        ap.error("--exchange-out needs --temper")
     host = {"plain": mcmc, "clustering": mcmc_clustering, "clustering2d": mcmc_clustering_2d}[a.driver]
     axes = []
     for g in a.grid:
@@ -58,6 +66,8 @@ def main(argv=None) -> int:
         pargs_list.append(host.parse_args(common + extra))
     # under torchrun: one rank per GPU, chains sharded by global chain id, one all_gather of the results (NCCL)
     rank, world, torch_device = 0, int(os.environ.get("WORLD_SIZE", "1")), None
+    if a.temper and world > 1:
+        ap.error("--temper needs a single rank: a ladder must live in one handle (run without torchrun)")
     if world > 1:
         import torch
         import torch.distributed as dist
@@ -69,9 +79,11 @@ def main(argv=None) -> int:
         rank = dist.get_rank()
     if a.by and not a.by_outdir:
         ap.error("--by needs --by-outdir")
+    exchange = {}
     header, rows, texts, entries = sweep.sweep_table(pargs_list, driver=a.driver, runs=a.runs, seed=a.seed,
                                                      device=a.device, torch_device=torch_device,
-                                                     kappaflag=a.kappaflag, with_entries=True, bit_identical=a.bit_identical)
+                                                     kappaflag=a.kappaflag, with_entries=True, bit_identical=a.bit_identical,
+                                                     temper=a.temper, exchange_every=a.exchange_every, exchange=exchange)
     if world > 1:
         import torch.distributed as dist
         dist.destroy_process_group()
@@ -84,6 +96,9 @@ def main(argv=None) -> int:
         aggregate.write_table(a.pooled_out, h2, r2)
     if a.outdir:
         aggregate.write_out_files(a.outdir, texts)
+    if a.exchange_out:
+        fixed = [name for name, _ in axes if name != a.temper]
+        sweep.write_exchange_csv(a.exchange_out, *sweep.exchange_rows(pargs_list, a.temper, exchange, fixed))
     if a.by:
         os.makedirs(a.by_outdir, exist_ok=True)
         ct = pargs_list[0]["chain-type"]
