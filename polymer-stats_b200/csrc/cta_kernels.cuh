@@ -175,11 +175,16 @@ __device__ double cta_pair_energy(const CtaView& S, int n, int energy_type, doub
   return block_sum<T>(acc, S.part);
 }
 
-// The rectangle heads×tails, 43 FP64 instructions per pair (old and new energy of one pair):
-//   lane item L in registers (x_L, μ_L, −3μ_L, cL = −3μ_L·D), broadcast item B from shared memory
-//   (x_B, μ_B, eB = μ_B·D);  r = x_L − x_B,  r' = r − D;
+// The rectangle heads×tails, 39 FP64 instructions per pair (old and new energy of one pair):
+//   lane item L in registers (x_L, μ_L, −3μ_L, cL = −3μ_L·D, wL = −2p_L), broadcast item B from shared
+//   memory (x_B, μ_B, eB = μ_B·D, vB = |D|² + 2p_B);  r = x_L − x_B,  r' = r − D;
 //   μ_L·r' = μ_L·r − μ_L·D and μ_B·r' = μ_B·r − eB save two dot products;
+//   |r'|² = r² − 2r·D + |D|² = (r² + wL) + vB with r·D = p_L − p_B, p_k = (x_k − x_idx)·D the projection on
+//   the move measured from the rotated monomer: 2 DADD instead of forming r' (3 DADD + 1 DMUL + 2 DFMA).
+//   Measured from the pivot, the rounding error of |r'|² is of order eps·|x_k − x_idx|·|D|, the order r
+//   itself already carries;
 //   g = y³(μ_L·μ_B + (−3μ_L·r)(μ_B·r) y²),  y = 1/|r|.
+// -DPMC_RECT_Q2=0 builds the previous form (r' formed and squared, 43 FP64 instructions) for comparisons.
 // Shared-memory loads are not free next to the FP64 pipe (≈1.7 issue cycles per LDS.64 against 2 per
 // DFMA, tools/fp64_mix.cu), so each lane keeps NL=2 lane items and every broadcast item loaded from
 // shared memory serves two pairs; an odd last group of 32 lane items runs with NL=1.
@@ -212,11 +217,16 @@ struct WarpTeam {
   __device__ __forceinline__ static void sync() { __syncwarp(); }
 };
 
+#ifndef PMC_RECT_Q2
+#define PMC_RECT_Q2 1
+#endif
+
 struct LaneItem {
   double x, y, z;     // position
   double ax, ay, az;  // μ
   double tx, ty, tz;  // −3μ
   double c;           // −3μ·D
+  double w;           // −2(x − x_idx)·D (Q2 form only, see rect_lane_w)
 };
 
 __device__ __forceinline__ LaneItem load_lane_item(const CtaView& S, int L, double Dx, double Dy, double Dz) {
@@ -225,22 +235,57 @@ __device__ __forceinline__ LaneItem load_lane_item(const CtaView& S, int L, doub
   it.ax = S.mx[L]; it.ay = S.my[L]; it.az = S.mz[L];
   it.tx = -3.0 * it.ax; it.ty = -3.0 * it.ay; it.tz = -3.0 * it.az;
   it.c = fma(it.tz, Dz, fma(it.ty, Dy, it.tx * Dx));
+  it.w = 0.0;
   return it;
 }
 
-// new − old of one pair: lane item `it` against broadcast item (bx,by,bz; ux,uy,uz; e).
+// Projection of x on the move, measured from the pivot (px, py, pz) = x_idx: p = (x − x_idx)·D.
+__device__ __forceinline__ double rect_proj(double x, double y, double z, double px, double py, double pz, double Dx,
+                                            double Dy, double Dz) {
+  return fma(z - pz, Dz, fma(y - py, Dy, (x - px) * Dx));
+}
+
+// wL = −2p_L of a lane item.
+__device__ __forceinline__ void rect_lane_w(LaneItem& it, double px, double py, double pz, double Dx, double Dy,
+                                            double Dz) {
+  it.w = -2.0 * rect_proj(it.x, it.y, it.z, px, py, pz, Dx, Dy, Dz);
+}
+
+// Broadcast-side values of one trial, written by the pre-pass before rect_sum.  Q2 form: {eB, vB} of broadcast
+// item k (counted from the start of the broadcast side) interleaved at S.E[2k], S.E[2k+1] and read with one 16-byte
+// load, so the broadcast side must have at most n/2 items (S.E holds n doubles).  Otherwise eB at S.E[baseB + k].
+template <bool Q2>
+__device__ __forceinline__ void rect_prepass_item(const CtaView& S, int baseB, int k, double px, double py, double pz,
+                                                  double Dx, double Dy, double Dz) {
+  const int j = baseB + k;
+  const double e = fma(S.mz[j], Dz, fma(S.my[j], Dy, S.mx[j] * Dx));
+  if constexpr (Q2) {
+    const double dd = fma(Dz, Dz, fma(Dy, Dy, Dx * Dx));
+    reinterpret_cast<double2*>(S.E)[k] =
+        make_double2(e, fma(2.0, rect_proj(S.sx[j], S.sy[j], S.sz[j], px, py, pz, Dx, Dy, Dz), dd));
+  }
+  else
+    S.E[j] = e;
+}
+
+// new − old of one pair: lane item `it` against broadcast item (bx,by,bz; ux,uy,uz; e; p2 = vB, Q2 form only).
 // CUT: UCutoff (eap_chain.jl:176-187) — a term is zero when its own r² exceeds crad².
-template <bool CUT = false>
+template <bool CUT = false, bool Q2 = false>
 __device__ __forceinline__ double rect_pair(const LaneItem& it, double bx, double by, double bz, double ux,
-                                            double uy, double uz, double e, double Dx, double Dy, double Dz,
+                                            double uy, double uz, double e, double p2, double Dx, double Dy, double Dz,
                                             double acc, double crad2 = 0.0) {
   const double rx = it.x - bx, ry = it.y - by, rz = it.z - bz;
   const double mm = fma(it.az, uz, fma(it.ay, uy, it.ax * ux));
   const double r2 = fma(rz, rz, fma(ry, ry, rx * rx));
   const double a3 = fma(it.tz, rz, fma(it.ty, ry, it.tx * rx));
   const double bb = fma(uz, rz, fma(uy, ry, ux * rx));
-  const double qx = rx - Dx, qy = ry - Dy, qz = rz - Dz;
-  const double q2 = fma(qz, qz, fma(qy, qy, qx * qx));
+  double q2;
+  if constexpr (Q2) {
+    q2 = (r2 + it.w) + p2;
+  } else {
+    const double qx = rx - Dx, qy = ry - Dy, qz = rz - Dz;
+    q2 = fma(qz, qz, fma(qy, qy, qx * qx));
+  }
   const double a3n = a3 - it.c;
   const double bn = bb - e;
 #if PMC_RSQ_PAR
@@ -265,9 +310,12 @@ __device__ __forceinline__ double rect_pair(const LaneItem& it, double bx, doubl
 
 // EFLY: eB = μ_B·D is computed in the loop (3 DFMA per broadcast item) instead of being read from S.E —
 // saves the pre-pass and its barrier where barriers cost more than FP64 issue slots (short chains).
-template <class TEAM, int UNROLL = 2, bool CUT = false, bool EFLY = false>
+// Q2: |r'|² from the projections (rect_prepass_item<true> has filled S.E); `pivot` = idx, the rotated monomer.
+// The pivot is read from shared memory with each lane item: its index costs one register in the loop, its position six.
+template <class TEAM, int UNROLL = 2, bool CUT = false, bool EFLY = false, bool Q2 = false>
 __device__ __forceinline__ double rect_sum(const CtaView& S, int baseA, int A, int baseB, int B, double Dx,
-                                           double Dy, double Dz, double crad2 = 0.0) {
+                                           double Dy, double Dz, double crad2 = 0.0, int pivot = 0) {
+  static_assert(!(Q2 && EFLY), "the Q2 form reads 2p_B from the pre-pass");
   constexpr int W = TEAM::kWarps;
   const int lane = TEAM::lane(), warp = TEAM::warp();
   const int G = (A + 31) >> 5;
@@ -278,6 +326,28 @@ __device__ __forceinline__ double rect_sum(const CtaView& S, int baseA, int A, i
   const double* __restrict__ myp = S.my + baseB;
   const double* __restrict__ mzp = S.mz + baseB;
   const double* __restrict__ ep = S.E + baseB;
+  const double2* __restrict__ e2p = reinterpret_cast<const double2*>(S.E);
+  auto lane_item = [&](int L) {
+    LaneItem it = load_lane_item(S, L, Dx, Dy, Dz);
+    if (Q2) {
+      rect_lane_w(it, S.sx[pivot], S.sy[pivot], S.sz[pivot], Dx, Dy, Dz);
+      // With wL the two lane items fill the 128 registers of k_run_cta_win<128,4,2>, and ptxas would recompute
+      // −3μ inside the pair loop (5 DMUL per 4 pairs) rather than spill per-trial values outside it.  Hiding how −3μ
+      // was made keeps it in registers: 39 FP64 per pair in the loop (profiles/r04_rect_q2_sass.txt).
+      asm("" : "+d"(it.tx), "+d"(it.ty), "+d"(it.tz));
+    }
+    return it;
+  };
+  // eB (and vB) of broadcast item k, whose μ is (ux, uy, uz)
+  auto bvals = [&](int k, double ux, double uy, double uz, double& e, double& p2) {
+    if constexpr (Q2) {
+      const double2 v = e2p[k];
+      e = v.x; p2 = v.y;
+    } else {
+      e = EFLY ? fma(uz, Dz, fma(uy, Dy, ux * Dx)) : ep[k];
+      p2 = 0.0;
+    }
+  };
   double acc = 0.0;
   // phase 1: group pairs (64 lane items per warp pass), two pairs per broadcast load
   const int G2 = G >> 1;
@@ -291,8 +361,8 @@ __device__ __forceinline__ double rect_sum(const CtaView& S, int baseA, int A, i
       while (u < u1) {
         const int l0 = g * 64 + lane, l1 = l0 + 32;
         const bool v0 = l0 < A, v1 = l1 < A;
-        const LaneItem i0 = load_lane_item(S, baseA + min(l0, A - 1), Dx, Dy, Dz);
-        const LaneItem i1 = load_lane_item(S, baseA + min(l1, A - 1), Dx, Dy, Dz);
+        const LaneItem i0 = lane_item(baseA + min(l0, A - 1));
+        const LaneItem i1 = lane_item(baseA + min(l1, A - 1));
         const int kend = min(B, k + (u1 - u));
         u += kend - k;
         double a0 = 0.0, a1 = 0.0;
@@ -300,9 +370,10 @@ __device__ __forceinline__ double rect_sum(const CtaView& S, int baseA, int A, i
         for (; k < kend; ++k) {
           const double bx = bxp[k], by = byp[k], bz = bzp[k];
           const double ux = mxp[k], uy = myp[k], uz = mzp[k];
-          const double e = EFLY ? fma(uz, Dz, fma(uy, Dy, ux * Dx)) : ep[k];
-          a0 = rect_pair<CUT>(i0, bx, by, bz, ux, uy, uz, e, Dx, Dy, Dz, a0, crad2);
-          a1 = rect_pair<CUT>(i1, bx, by, bz, ux, uy, uz, e, Dx, Dy, Dz, a1, crad2);
+          double e, p2;
+          bvals(k, ux, uy, uz, e, p2);
+          a0 = rect_pair<CUT, Q2>(i0, bx, by, bz, ux, uy, uz, e, p2, Dx, Dy, Dz, a0, crad2);
+          a1 = rect_pair<CUT, Q2>(i1, bx, by, bz, ux, uy, uz, e, p2, Dx, Dy, Dz, a1, crad2);
         }
         acc += (v0 ? a0 : 0.0) + (v1 ? a1 : 0.0);
         k = 0;
@@ -317,18 +388,19 @@ __device__ __forceinline__ double rect_sum(const CtaView& S, int baseA, int A, i
     if (k < kend) {
       const int li = (G - 1) * 32 + lane;
       const bool valid = li < A;
-      const LaneItem it = load_lane_item(S, baseA + min(li, A - 1), Dx, Dy, Dz);
+      const LaneItem it = lane_item(baseA + min(li, A - 1));
       double a0 = 0.0, a1 = 0.0;
-      auto eb = [&](int kk) {
-        return EFLY ? fma(mzp[kk], Dz, fma(myp[kk], Dy, mxp[kk] * Dx)) : ep[kk];
+      auto pair = [&](int kk, double a) {
+        double e, p2;
+        bvals(kk, mxp[kk], myp[kk], mzp[kk], e, p2);
+        return rect_pair<CUT, Q2>(it, bxp[kk], byp[kk], bzp[kk], mxp[kk], myp[kk], mzp[kk], e, p2, Dx, Dy, Dz, a,
+                                  crad2);
       };
       for (; k + 1 < kend; k += 2) {
-        a0 = rect_pair<CUT>(it, bxp[k], byp[k], bzp[k], mxp[k], myp[k], mzp[k], eb(k), Dx, Dy, Dz, a0, crad2);
-        a1 = rect_pair<CUT>(it, bxp[k + 1], byp[k + 1], bzp[k + 1], mxp[k + 1], myp[k + 1], mzp[k + 1], eb(k + 1),
-                            Dx, Dy, Dz, a1, crad2);
+        a0 = pair(k, a0);
+        a1 = pair(k + 1, a1);
       }
-      if (k < kend)
-        a0 = rect_pair<CUT>(it, bxp[k], byp[k], bzp[k], mxp[k], myp[k], mzp[k], eb(k), Dx, Dy, Dz, a0, crad2);
+      if (k < kend) a0 = pair(k, a0);
       acc += valid ? (a0 + a1) : 0.0;
     }
   }
@@ -353,19 +425,22 @@ __device__ __forceinline__ double delta_pairs_partial(const CtaView& S, int n, i
     const long long costH = (long long)((H + 31) >> 5) * Tl;
     const long long costT = (long long)((Tl + 31) >> 5) * H;
     lanes_are_heads = costH <= costT;
+    // {eB, 2p_B} of the broadcast side fill 2B of the n doubles of S.E: at most one side (H + Tl = n − 1) has more
+    // than n/2 items, and it goes on the lanes
+    if (PMC_RECT_Q2 && 2 * (lanes_are_heads ? Tl : H) > n) lanes_are_heads = !lanes_are_heads;
   }
   // D_eff: r = x_L − x_B.  L=head,B=tail: r' = r − D.  L=tail,B=head: r' = r + D.
   const double sgn = lanes_are_heads ? 1.0 : -1.0;
   const double ex = sgn * Dx, ey = sgn * Dy, ez = sgn * Dz;
   const int baseA = lanes_are_heads ? 0 : idx + 1, A = lanes_are_heads ? H : Tl;
   const int baseB = lanes_are_heads ? idx + 1 : 0, B = lanes_are_heads ? Tl : H;
+  const double xi = S.sx[idx], yi = S.sy[idx], zi = S.sz[idx];  // the pivot of the Q2 projections
   if (rect)  // every copy of the staged chain needs its own E
     for (int k = TEAM::ltid(); k < B; k += TEAM::kLocalThreads)
-      S.E[baseB + k] = fma(S.mz[baseB + k], ez, fma(S.my[baseB + k], ey, S.mx[baseB + k] * ex));
+      rect_prepass_item<PMC_RECT_Q2>(S, baseB, k, xi, yi, zi, ex, ey, ez);
   // row {idx}×rest: both μ_idx and the separation change.
   double acc = 0.0;
   {
-    const double xi = S.sx[idx], yi = S.sy[idx], zi = S.sz[idx];
     const double ox = S.mx[idx], oy = S.my[idx], oz = S.mz[idx];
     int jlo = 0, jhi = n - 1;
     if (energy_type == 2) { jlo = max(0, idx - 1); jhi = min(n - 1, idx + 1); }
@@ -380,7 +455,7 @@ __device__ __forceinline__ double delta_pairs_partial(const CtaView& S, int n, i
     }
   }
   TEAM::sync();  // E visible
-  if (rect) acc += rect_sum<TEAM, UNROLL>(S, baseA, A, baseB, B, ex, ey, ez);
+  if (rect) acc += rect_sum<TEAM, UNROLL, false, false, PMC_RECT_Q2>(S, baseA, A, baseB, B, ex, ey, ez, 0.0, idx);
   return acc;
 }
 
@@ -688,8 +763,12 @@ struct SpecTrial {
   int accept, pad;
 };
 
+// The E arrays of teams 1…G−1 start 16-byte aligned (rect_prepass_item reads S.E as double2).
+__host__ __device__ inline int spec_e_stride(int n) { return (n + 1) & ~1; }
+
 __host__ __device__ inline size_t cta_smem_bytes_spec(int n, int groups) {
-  return cta_smem_bytes_win(n) + (((size_t)(groups - 1) * n * sizeof(double) + (size_t)groups * sizeof(SpecTrial) + 15) & ~(size_t)15);
+  return cta_smem_bytes_win(n) +
+         (((size_t)(groups - 1) * spec_e_stride(n) * sizeof(double) + (size_t)groups * sizeof(SpecTrial) + 15) & ~(size_t)15);
 }
 
 template <int G, int MINB>
@@ -700,13 +779,13 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_win_spec(const RunArgs
   Proposal* win = reinterpret_cast<Proposal*>(smem_raw + cta_smem_bytes(a.n));
   unsigned* dirty = reinterpret_cast<unsigned*>(win + kWin);
   double* extraE = reinterpret_cast<double*>(smem_raw + cta_smem_bytes_win(a.n));
-  SpecTrial* res = reinterpret_cast<SpecTrial*>(extraE + (size_t)(G - 1) * a.n);
+  SpecTrial* res = reinterpret_cast<SpecTrial*>(extraE + (size_t)(G - 1) * spec_e_stride(a.n));
   const int c = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, g = tid >> 5;
   const int n = a.n;
   MonoRec* mono = a.mono + (size_t)c * n;
   CtaView Sg = S;                       // this team's view: its own E array, everything else shared
-  if (g > 0) Sg.E = extraE + (size_t)(g - 1) * n;
+  if (g > 0) Sg.E = extraE + (size_t)(g - 1) * spec_e_stride(n);
   if (tid == 0) {
     *S.par = a.par[c];
     *S.dyn = a.dyn[c];
