@@ -46,11 +46,8 @@ static __device__ __noinline__ double log_shared(double x) { return log(x); }
 static __device__ __noinline__ double exp_shared(double x) { return exp(x); }
 static __device__ __noinline__ double acos_shared(double x) { return acos(x); }
 
-// Default of a translation unit: -DPMC_SH_DEFAULT=true makes every call site without an explicit choice use the shared copies.
-#ifndef PMC_SH_DEFAULT
-#define PMC_SH_DEFAULT false
-#endif
-constexpr bool kSharedLib = PMC_SH_DEFAULT;
+// Call sites without an explicit choice use the inlined versions.
+constexpr bool kSharedLib = false;
 
 template <bool SH>
 struct Lib {
@@ -205,26 +202,6 @@ __device__ __forceinline__ double rsqrt_fast(double x) { return rsqrt_mixed(x); 
 __device__ __forceinline__ double rsqrt_fast(double x) { return rsqrt_cubic(x); }
 #endif
 
-// y = 1/sqrt(x) and y² for a pair term.  Experiment PMC_RSQ_PAR (off in the product build): y² = s(1 + e + e²) from the seed
-// (s = y0², e = 1 − x s; relative error e³ ≲ 2^-57) next to y instead of y·y after it — one FP64 instruction more per 1/sqrt,
-// one step less in the dependent chain seed → s → e → y → y² → term → sum that the `wait` stalls of the composite-trial
-// kernel sit on (profiles/r02h_ncu_full_k_run_cta_cluster_K1.txt).
-#ifndef PMC_RSQ_PAR
-#define PMC_RSQ_PAR 0
-#endif
-#if PMC_RSQ_PAR
-__device__ __forceinline__ void rsqrt_y_y2(double x, double& y, double& y2) {
-  double y0;
-  asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y0) : "d"(x));
-  const double s = y0 * y0;
-  const double e = fma(-x, s, 1.0);
-  const double t = fma(e, 0.375, 0.5);
-  const double p = fma(e, e, e);
-  y = fma(y0 * e, t, y0);
-  y2 = fma(s, p, s);
-}
-#endif
-
 // 4π × one dipole-dipole pair term (eap_chain.jl:200-207): μa·μb/r³ − 3(μa·r)(μb·r)/r⁵.
 __device__ __forceinline__ double pair_g(double ax, double ay, double az, double bx, double by, double bz,
                                          double rx, double ry, double rz) {
@@ -232,13 +209,8 @@ __device__ __forceinline__ double pair_g(double ax, double ay, double az, double
   const double mm = fma(az, bz, fma(ay, by, ax * bx));
   const double a = fma(az, rz, fma(ay, ry, ax * rx));
   const double b = fma(bz, rz, fma(by, ry, bx * rx));
-#if PMC_RSQ_PAR
-  double y, y2;
-  rsqrt_y_y2(r2, y, y2);
-#else
   const double y = rsqrt_fast(r2);
   const double y2 = y * y;
-#endif
   const double t = fma(-3.0 * a * b, y2, mm);
   return t * (y2 * y);
 }

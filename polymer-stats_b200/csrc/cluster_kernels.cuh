@@ -16,10 +16,6 @@
 
 #include "lane_kernels.cuh"
 
-#ifndef PMC_UR_SHORT
-#define PMC_UR_SHORT 1   // rectangle unroll of the one- and two-warp teams (experiments: -DPMC_UR_SHORT=2)
-#endif
-
 namespace pmc {
 
 // Sums reduced over the CTA for one composite trial.
@@ -42,15 +38,13 @@ struct ClProposal {
   int idx, reflect;
 };
 
-constexpr int kClWin = 32;  // proposals built at once, one per lane of warp 0
-
 struct ClView {
   double *nhx, *nhy, *nhz;  // n̂_i of the current state (eap_chain.jl:27)
   double *nnx, *nny, *nnz;  // n̂'_i of the trial, valid on the segment
   double *xnx, *xny, *xnz;  // x'_i of the trial, valid on the segment
   double *psi, *psn;        // bond angles ψ_i of the current state (eap_chain.jl:29) and of the trial (bonds lo−1..hi)
   double* red;              // [kNumRed][warps] warp partials
-  ClProposal* win;          // [kClWin]
+  ClProposal* win;          // [kWin]
   ClusterCtl* ctl;
   ChainDynX* dx;
 };
@@ -58,7 +52,7 @@ struct ClView {
 // Bytes of the composite-trial arrays that follow the CtaView part.
 __host__ __device__ inline size_t cluster_extra_bytes(int n, int threads) {
   size_t b = (size_t)11 * n * sizeof(double) + (size_t)kNumRed * (threads / 32) * sizeof(double);
-  b += kClWin * sizeof(ClProposal) + sizeof(ClusterCtl) + sizeof(ChainDynX);
+  b += kWin * sizeof(ClProposal) + sizeof(ClusterCtl) + sizeof(ChainDynX);
   return (b + 15) & ~(size_t)15;
 }
 // run kernel (compact CtaView) / parity-seam kernel (full CtaView with its Proposal slots)
@@ -78,7 +72,7 @@ __device__ __forceinline__ ClView carve_cluster(unsigned char* base, int n, int 
   X.psi = d + 9 * n; X.psn = d + 10 * n;
   X.red = d + 11 * n;
   X.win = reinterpret_cast<ClProposal*>(X.red + kNumRed * (threads / 32));
-  X.ctl = reinterpret_cast<ClusterCtl*>(X.win + kClWin);
+  X.ctl = reinterpret_cast<ClusterCtl*>(X.win + kWin);
   X.dx = reinterpret_cast<ChainDynX*>(X.ctl + 1);
   return X;
 }
@@ -362,7 +356,7 @@ __device__ __forceinline__ void segment_sums(const CtaView& S, const ClView& X, 
                                              int energy_type, int lo, int hi, double Dx, double Dy, double Dz,
                                              double* acc, double* sums) {
   constexpr int W = T / 32;
-  using TEAM = typename std::conditional<T == 32, WarpTeam, Team<W, 0>>::type;
+  using TEAM = typename std::conditional<T == 32, WarpTeam, Team<W>>::type;
   const int tid = team_tid<T>(), lane = tid & 31, warp = tid >> 5;
   // ---- bonds lo−1..hi: ψ and bending energy (eap_chain.jl:45-47,54-58,246-251) ---------------------------
   {
@@ -386,7 +380,7 @@ __device__ __forceinline__ void segment_sums(const CtaView& S, const ClView& X, 
     // short chains (≤ 2 warps): eB = μ_B·D on the fly — a barrier costs more than 3 DFMA per broadcast item;
     // longer chains: the pre-pass into S.E and its barrier are amortised, and the rectangle loop is unrolled
     constexpr bool EFLY = (T <= 64);
-    constexpr int UR = (T <= 64) ? PMC_UR_SHORT : 2;
+    constexpr int UR = (T <= 64) ? 1 : 2;   // rectangle unroll
     const bool rect = H > 0 && Tl > 0;
     // lane side = the one that wastes fewer lanes; r = x_L − x_B, so r' = r − D (L = head) or r + D (L = tail)
     const long long costH = (long long)((H + 31) >> 5) * Tl;
@@ -512,12 +506,86 @@ __device__ __forceinline__ void stage_row_cluster(const ChainDyn& D, const Chain
 
 constexpr int kRowDoublesCluster = 28;
 
+// The team, thread tid: output row `row` after trial `step`, with the two extra averagers and, if a.state, the angles of
+// every monomer.  Starts with a team barrier (the records of the trial are visible).
+template <int T>
+__device__ __forceinline__ void emit_row_cluster(const RunArgs& a, const ChainDyn& D, const ChainDynX& DX,
+                                                 const MonoRec* mono, int c, long long row, long long step,
+                                                 double* rowbuf, int tid) {
+  team_sync<T>();
+  if (row < a.rows) {
+    if (tid == 0) stage_row_cluster(D, DX, step, rowbuf);
+    if (a.state) {
+      double* st = a.state + ((size_t)c * a.rows + row) * 2 * (size_t)a.n;
+      for (int m = tid; m < a.n; m += T) {
+        const MonoRec r = mono[m];
+        st[2 * m] = r.phi; st[2 * m + 1] = r.theta;
+      }
+    }
+    team_sync<T>();
+    if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = rowbuf[tid];
+    if (tid < a.roll_cols) a.roll[((size_t)c * a.rows + row) * a.roll_cols + tid] = rowbuf[8 + tid];
+  }
+}
+
+// The trial chain becomes the chain (mcmc_clustering_eap_chain.jl:274-275), threads tid, tid + T, …: monomers lo … hi
+// take the records, n̂, x and μ of the trial from the arrays of the team that evaluated it (St.E = sinθ', Xt), the tail
+// j > hi moves by D, and the bond angles lo−1 … hi follow.
+template <int T>
+__device__ __forceinline__ void commit_segment(const CtaView& S, const ClView& X, const CtaView& St, const ClView& Xt,
+                                               MonoRec* mono, const ChainParams& P, const ClProposal& q, int n, int lo,
+                                               int hi, bool reflect, double Dx, double Dy, double Dz, int tid) {
+  for (int m = lo + tid; m <= hi; m += T) {
+    double phi, theta, sb;
+    segment_angles(mono, q, m, reflect, P.planar, phi, theta, sb);
+    MonoRec rec;
+    rec.phi = phi; rec.theta = theta;
+    rec.nx = Xt.nnx[m]; rec.ny = Xt.nny[m]; rec.nz = Xt.nnz[m];
+    rec.sth = (St.E[m] == kKeepSinTheta) ? sb : St.E[m];
+    mono[m] = rec;
+    X.nhx[m] = rec.nx; X.nhy[m] = rec.ny; X.nhz[m] = rec.nz;
+    S.sx[m] = Xt.xnx[m]; S.sy[m] = Xt.xny[m]; S.sz[m] = Xt.xnz[m];
+    double ux, uy, uz;
+    mu_of(P, rec.nx, rec.ny, rec.nz, ux, uy, uz);
+    S.mx[m] = ux; S.my[m] = uy; S.mz[m] = uz;
+  }
+  shift_tail(S, hi + 1, n, Dx, Dy, Dz, tid, T);
+  for (int i = max(lo - 1, 0) + tid; i <= min(hi, n - 2); i += T) X.psi[i] = Xt.psn[i];
+}
+
+// Thread 0 (lane kernel: every thread): the increments of an accepted composite trial and its α carry, the trial
+// counters and the cluster statistics.
+__device__ __forceinline__ void commit_trial(const ChainParams& P, ChainDyn& D, ChainDynX& DX, bool accept,
+                                             long long step, double dU, double dOmega, double dsu, double Dx,
+                                             double Dy, double Dz, double dpx, double dpy, double dpz, double dpsi,
+                                             double dcos2, double la, bool reflect, int lo, int hi) {
+  if (accept) {
+    D.U += dU;
+    D.Omega += dOmega;
+    D.su += dsu;
+    D.r[0] += Dx; D.r[1] += Dy; D.r[2] += Dz;
+    D.p[0] += dpx; D.p[1] += dpy; D.p[2] += dpz;
+    DX.spsi += dpsi;
+    DX.scos2 += dcos2;
+    DX.carry = P.alpha_carry ? la : 0.0;  // logπ_prev = logπ + log α (acceptance.jl:32-33)
+    D.nacc += 1;
+    D.nacc_total += 1;
+  }
+  D.natt += 1;
+  D.steps_total += 1;
+  D.step = step;
+  if (reflect) {
+    const double sz = (double)(hi - lo + 1);
+    DX.ncluster += 1.0; DX.cluster_sum += sz; DX.cluster_max = fmax(DX.cluster_max, sz);
+  }
+}
+
 // The hot loop of mcmc_clustering_eap_chain.jl:267-336 for one chain per CTA (T = 32: a one-warp CTA, the team
 // barriers are __syncwarp).
 //
 // Proposal window, as in k_run_cta_win: the serial head of a trial (3 Philox blocks, 2 sincos, log, the record
 // read from HBM/L2) is taken off the per-trial critical path by building the single-monomer moves and the gate
-// decisions of the next kClWin trials at once, one trial per lane of warp 0.  A window entry depends on the
+// decisions of the next kWin trials at once, one trial per lane of warp 0.  A window entry depends on the
 // chain only through the record of its own monomer: an accepted trial marks the later entries whose monomer
 // lies in its segment [lo, hi] dirty and those are rebuilt when their turn comes.  Windows never cross a
 // step-size adaptation boundary.  The cluster growth reads the neighbours' current directions and stays per trial.
@@ -552,18 +620,11 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_cluster(const RunArgs a) {
   long long s = 1;
   while (s <= a.nsteps) {
     // ---- window [s, s+wlen) ------------------------------------------------------------------------------
-    long long wl = a.nsteps - s + 1;
-    if (wl > kClWin) wl = kClWin;
-    long long to_boundary = 0;  // trials until the adaptation rule runs (0: never)
-    if (adapt_on) {
-      to_boundary = P.steps_per_adjust - ((step0 + s - 1) % P.steps_per_adjust);  // ≥ 1
-      if (wl > to_boundary) wl = to_boundary;
-    }
-    const int wlen = (int)wl;
-    if (tid < 32) {
-      if (tid < wlen) make_window_entry(a, P, *S.dyn, mono, chain_id, step0 + s + tid, X.win[tid]);
-      if (tid == 0) X.ctl->dirty = 0u;
-    }
+    long long to_boundary;
+    const int wlen = window_len(a, P, adapt_on, step0, s, to_boundary);
+    if (tid < 32)
+      build_window(step0 + s, wlen, X.ctl->dirty, tid,
+                   [&](int e, long long st) { make_window_entry(a, P, *S.dyn, mono, chain_id, st, X.win[e]); });
     team_sync<T>();  // window visible
     for (int k = 0; k < wlen; ++k) {
       const long long step = step0 + s + k;
@@ -592,74 +653,16 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_cluster(const RunArgs a) {
       const double la = reflect ? cluster_log_alpha(X, n, lo, hi, X.ctl->up, X.ctl->lp) : 0.0;
       const SegDecision dec = segment_decision(P, a.energy_type, sums, Dx, Dz, la, carry);
       const bool accept = metropolis(dec.dlogpi, q->eps);
-      if (accept) {  // the trial chain becomes the chain (mcmc_clustering_eap_chain.jl:274-275)
-        for (int m = lo + tid; m <= hi; m += T) {
-          double phi, theta, sb;
-          segment_angles(mono, *q, m, reflect, P.planar, phi, theta, sb);
-          MonoRec rec;
-          rec.phi = phi; rec.theta = theta;
-          rec.nx = X.nnx[m]; rec.ny = X.nny[m]; rec.nz = X.nnz[m];
-          rec.sth = (S.E[m] == kKeepSinTheta) ? sb : S.E[m];
-          mono[m] = rec;
-          X.nhx[m] = rec.nx; X.nhy[m] = rec.ny; X.nhz[m] = rec.nz;
-          S.sx[m] = X.xnx[m]; S.sy[m] = X.xny[m]; S.sz[m] = X.xnz[m];
-          double ux, uy, uz;
-          mu_of(P, rec.nx, rec.ny, rec.nz, ux, uy, uz);
-          S.mx[m] = ux; S.my[m] = uy; S.mz[m] = uz;
-        }
-        for (int j = hi + 1 + tid; j < n; j += T) {
-          S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-        }
-        for (int i = max(lo - 1, 0) + tid; i <= min(hi, n - 2); i += T) X.psi[i] = X.psn[i];
-        if (tid < 32) {  // later entries of the window on a monomer of the segment are stale now
-          const int widx = X.win[tid].idx;
-          const bool stale = tid > k && tid < wlen && widx >= lo && widx <= hi;
-          const unsigned m = __ballot_sync(0xffffffffu, stale);
-          if (tid == 0 && m) X.ctl->dirty |= m;
-        }
+      if (accept) {
+        commit_segment<T>(S, X, S, X, mono, P, *q, n, lo, hi, reflect, Dx, Dy, Dz, tid);
+        if (tid < 32) mark_stale(X.win, k, wlen, lo, hi, X.ctl->dirty, tid);
       }
       if (tid == 0) {
-        ChainDyn& D = *S.dyn;
-        ChainDynX& DX = *X.dx;
-        if (accept) {
-          D.U += dec.dU;
-          D.Omega += sums[R_OMEGA];
-          D.su += dec.dsu;
-          D.r[0] += Dx; D.r[1] += Dy; D.r[2] += Dz;
-          D.p[0] += sums[R_PX]; D.p[1] += sums[R_PY]; D.p[2] += sums[R_PZ];
-          DX.spsi += sums[R_PSI];
-          DX.scos2 += sums[R_COS2];
-          DX.carry = P.alpha_carry ? dec.la : 0.0;  // logπ_prev = logπ + log α (acceptance.jl:32-33)
-          D.nacc += 1;
-          D.nacc_total += 1;
-        }
-        D.natt += 1;
-        D.steps_total += 1;
-        D.step = step;
-        if (reflect) {
-          const double sz = (double)(hi - lo + 1);
-          DX.ncluster += 1.0; DX.cluster_sum += sz; DX.cluster_max = fmax(DX.cluster_max, sz);
-        }
-        bookkeep_cluster(P, D, DX, /*adapt_now=*/k + 1 == to_boundary, n, a.compensated != 0);
+        commit_trial(P, *S.dyn, *X.dx, accept, step, dec.dU, sums[R_OMEGA], dec.dsu, Dx, Dy, Dz, sums[R_PX], sums[R_PY],
+                     sums[R_PZ], sums[R_PSI], sums[R_COS2], dec.la, reflect, lo, hi);
+        bookkeep_cluster(P, *S.dyn, *X.dx, /*adapt_now=*/k + 1 == to_boundary, n, a.compensated != 0);
       }
-      const bool isrow = row_due.tick();
-      if (isrow) {
-        team_sync<T>();  // records of this trial are visible
-        if (row < a.rows) {
-          if (tid == 0) stage_row_cluster(*S.dyn, *X.dx, step, rowbuf);
-          if (a.state) {
-            double* st = a.state + ((size_t)c * a.rows + row) * 2 * (size_t)n;
-            for (int m = tid; m < n; m += T) {
-              const MonoRec r = mono[m];
-              st[2 * m] = r.phi; st[2 * m + 1] = r.theta;
-            }
-          }
-          team_sync<T>();
-          if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = rowbuf[tid];
-          if (tid < a.roll_cols) a.roll[((size_t)c * a.rows + row) * a.roll_cols + tid] = rowbuf[8 + tid];
-        }
-        ++row;
-      }
+      if (row_due.tick()) emit_row_cluster<T>(a, *S.dyn, *X.dx, mono, c, row++, step, rowbuf, tid);
       team_sync<T>();  // state, records and the dirty mask of this trial are visible
     }
     s += wlen;
@@ -712,20 +715,25 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_cluster_spec(const Run
   const int tid = threadIdx.x, lane = tid & 31, g = tid >> 5;
   const int n = a.n;
   MonoRec* mono = a.mono + (size_t)c * n;
-  // this team's views: the chain (x, μ, n̂, ψ) is shared and read-only while trials are evaluated; sinθ'/E, n̂', x', ψ',
+  // team t's views: the chain (x, μ, n̂, ψ) is shared and read-only while trials are evaluated; sinθ'/E, n̂', x', ψ',
   // the reduction slots and the cluster control block are the team's own
-  CtaView Sg = S;
-  ClView Xg = X;
-  Sg.part = S.part + 3 * g;
-  Xg.red = X.red + kNumRed * g;
-  if (g > 0) {
-    double* d = reinterpret_cast<double*>(extra + (size_t)(g - 1) * cluster_spec_group_bytes(n));
-    Sg.E = d;
-    Xg.nnx = d + n; Xg.nny = d + 2 * n; Xg.nnz = d + 3 * n;
-    Xg.xnx = d + 4 * n; Xg.xny = d + 5 * n; Xg.xnz = d + 6 * n;
-    Xg.psn = d + 7 * n;
-    Xg.ctl = reinterpret_cast<ClusterCtl*>(d + 8 * n);
-  }
+  auto team_arrays = [&](int t, CtaView& St, ClView& Xt) {
+    St = S;
+    Xt = X;
+    St.part = S.part + 3 * t;
+    Xt.red = X.red + kNumRed * t;
+    if (t > 0) {
+      double* d = reinterpret_cast<double*>(extra + (size_t)(t - 1) * cluster_spec_group_bytes(n));
+      St.E = d;
+      Xt.nnx = d + n; Xt.nny = d + 2 * n; Xt.nnz = d + 3 * n;
+      Xt.xnx = d + 4 * n; Xt.xny = d + 5 * n; Xt.xnz = d + 6 * n;
+      Xt.psn = d + 7 * n;
+      Xt.ctl = reinterpret_cast<ClusterCtl*>(d + 8 * n);
+    }
+  };
+  CtaView Sg;
+  ClView Xg;
+  team_arrays(g, Sg, Xg);
   if (tid == 0) {
     *S.par = a.par[c];
     *S.dyn = a.dyn[c];
@@ -740,21 +748,17 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_cluster_spec(const Run
   const uint32_t init = (uint32_t)S.dyn->init;
   const bool adapt_on = P.adj_scale != 1.0 && P.steps_per_adjust > 0;
   long long row = 0;
-  Countdown row_due, adapt_due;
+  Countdown row_due;
   row_due.start(step0, a.stepout);
-  adapt_due.start(step0, adapt_on ? P.steps_per_adjust : 0);
 
   long long s = 1;
   while (s <= a.nsteps) {
-    // ---- window [s, s+wlen): never across an adaptation boundary --------------------------------------------
-    long long wl = a.nsteps - s + 1;
-    if (wl > kClWin) wl = kClWin;
-    if (adapt_on && wl > adapt_due.left) wl = adapt_due.left;
-    const int wlen = (int)wl;
-    if (tid < 32) {
-      if (tid < wlen) make_window_entry(a, P, *S.dyn, mono, chain_id, step0 + s + tid, X.win[tid]);
-      if (tid == 0) X.ctl->dirty = 0u;
-    }
+    // ---- window [s, s+wlen) --------------------------------------------------------------------------------
+    long long to_boundary;
+    const int wlen = window_len(a, P, adapt_on, step0, s, to_boundary);
+    if (tid < 32)
+      build_window(step0 + s, wlen, X.ctl->dirty, tid,
+                   [&](int e, long long st) { make_window_entry(a, P, *S.dyn, mono, chain_id, st, X.win[e]); });
     __syncthreads();  // window visible
     int k = 0;
     while (k < wlen) {
@@ -804,83 +808,19 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_cluster_spec(const Run
         const ClProposal* q = &X.win[kk];
         const bool accept = R.accept != 0, reflect = R.reflect != 0;
         const int lo = R.lo, hi = R.hi;
-        if (accept) {  // the trial chain of team b becomes the chain (mcmc_clustering_eap_chain.jl:274-275)
-          const double* bE = S.E;
-          const double *bnx = X.nnx, *bny = X.nny, *bnz = X.nnz, *bxx = X.xnx, *bxy = X.xny, *bxz = X.xnz, *bps = X.psn;
-          if (b > 0) {
-            const double* d = reinterpret_cast<const double*>(extra + (size_t)(b - 1) * cluster_spec_group_bytes(n));
-            bE = d; bnx = d + n; bny = d + 2 * n; bnz = d + 3 * n; bxx = d + 4 * n; bxy = d + 5 * n; bxz = d + 6 * n;
-            bps = d + 7 * n;
-          }
-          const double Dx = R.Dx, Dy = R.Dy, Dz = R.Dz;
-          for (int m = lo + tid; m <= hi; m += T) {
-            double phi, theta, sb;
-            segment_angles(mono, *q, m, reflect, P.planar, phi, theta, sb);
-            MonoRec rec;
-            rec.phi = phi; rec.theta = theta;
-            rec.nx = bnx[m]; rec.ny = bny[m]; rec.nz = bnz[m];
-            rec.sth = (bE[m] == kKeepSinTheta) ? sb : bE[m];
-            mono[m] = rec;
-            X.nhx[m] = rec.nx; X.nhy[m] = rec.ny; X.nhz[m] = rec.nz;
-            S.sx[m] = bxx[m]; S.sy[m] = bxy[m]; S.sz[m] = bxz[m];
-            double ux, uy, uz;
-            mu_of(P, rec.nx, rec.ny, rec.nz, ux, uy, uz);
-            S.mx[m] = ux; S.my[m] = uy; S.mz[m] = uz;
-          }
-          for (int j = hi + 1 + tid; j < n; j += T) {
-            S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-          }
-          for (int i = max(lo - 1, 0) + tid; i <= min(hi, n - 2); i += T) X.psi[i] = bps[i];
-          if (tid < 32) {  // later entries of the window on a monomer of the segment are stale now
-            const int widx = X.win[tid].idx;
-            const bool stale = tid > kk && tid < wlen && widx >= lo && widx <= hi;
-            const unsigned m = __ballot_sync(0xffffffffu, stale);
-            if (tid == 0 && m) X.ctl->dirty |= m;
-          }
+        if (accept) {  // the trial chain of team b becomes the chain
+          CtaView Sb;
+          ClView Xb;
+          team_arrays(b, Sb, Xb);
+          commit_segment<T>(S, X, Sb, Xb, mono, P, *q, n, lo, hi, reflect, R.Dx, R.Dy, R.Dz, tid);
+          if (tid < 32) mark_stale(X.win, kk, wlen, lo, hi, X.ctl->dirty, tid);
         }
         if (tid == 0) {
-          ChainDyn& D = *S.dyn;
-          ChainDynX& DX = *X.dx;
-          if (accept) {
-            D.U += R.dec.dU;
-            D.Omega += R.sums[R_OMEGA];
-            D.su += R.dec.dsu;
-            D.r[0] += R.Dx; D.r[1] += R.Dy; D.r[2] += R.Dz;
-            D.p[0] += R.sums[R_PX]; D.p[1] += R.sums[R_PY]; D.p[2] += R.sums[R_PZ];
-            DX.spsi += R.sums[R_PSI];
-            DX.scos2 += R.sums[R_COS2];
-            DX.carry = P.alpha_carry ? R.dec.la : 0.0;  // logπ_prev = logπ + log α (acceptance.jl:32-33)
-            D.nacc += 1;
-            D.nacc_total += 1;
-          }
-          D.natt += 1;
-          D.steps_total += 1;
-          D.step = step;
-          if (reflect) {
-            const double sz = (double)(hi - lo + 1);
-            DX.ncluster += 1.0; DX.cluster_sum += sz; DX.cluster_max = fmax(DX.cluster_max, sz);
-          }
+          commit_trial(P, *S.dyn, *X.dx, accept, step, R.dec.dU, R.sums[R_OMEGA], R.dec.dsu, R.Dx, R.Dy, R.Dz,
+                       R.sums[R_PX], R.sums[R_PY], R.sums[R_PZ], R.sums[R_PSI], R.sums[R_COS2], R.dec.la, reflect, lo, hi);
+          bookkeep_cluster(P, *S.dyn, *X.dx, /*adapt_now=*/kk + 1 == to_boundary, n, a.compensated != 0);
         }
-        const bool adapt_now = adapt_due.tick();   // every thread keeps the same countdowns
-        if (tid == 0) bookkeep_cluster(P, *S.dyn, *X.dx, adapt_now, n, a.compensated != 0);
-        const bool isrow = row_due.tick();
-        if (isrow) {
-          __syncthreads();  // records of this trial are visible
-          if (row < a.rows) {
-            if (tid == 0) stage_row_cluster(*S.dyn, *X.dx, step, rowbuf);
-            if (a.state) {
-              double* st = a.state + ((size_t)c * a.rows + row) * 2 * (size_t)n;
-              for (int m = tid; m < n; m += T) {
-                const MonoRec r = mono[m];
-                st[2 * m] = r.phi; st[2 * m + 1] = r.theta;
-              }
-            }
-            __syncthreads();
-            if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = rowbuf[tid];
-            if (tid < a.roll_cols) a.roll[((size_t)c * a.rows + row) * a.roll_cols + tid] = rowbuf[8 + tid];
-          }
-          ++row;
-        }
+        if (row_due.tick()) emit_row_cluster<T>(a, *S.dyn, *X.dx, mono, c, row++, step, rowbuf, tid);
         ++committed;
         if (accept) break;  // the speculations behind this trial saw the chain before it
       }
@@ -1002,7 +942,7 @@ template <bool SH = kSharedLib>
 __device__ __forceinline__ void lane_idx_record(const ChainParams& P, const Proposal& q, bool reflect, MonoRec& nrec,
                                                 double& dOmega) {
   if (!reflect) {
-    nrec.phi = q.phi; nrec.theta = q.theta; nrec.nx = q.nx; nrec.ny = q.ny; nrec.nz = q.nz; nrec.sth = q.sth;
+    nrec = record_of(q);
     dOmega = q.dOmega;
     return;
   }
@@ -1168,18 +1108,9 @@ __global__ void __launch_bounds__(T, MINB) k_run_lane_cluster(const RunArgs a) {
           mono[k] = r;
         }
       mono[d.idx] = nrec;
-      D.U += dU; D.Omega += g.dOmega; D.su += dsu;
-      D.r[0] += Dx; D.r[1] += Dy; D.r[2] += Dz;
-      D.p[0] += g.dpx; D.p[1] += g.dpy; D.p[2] += g.dpz;
-      DX.spsi += g.dpsi; DX.scos2 += g.dcos2;
-      DX.carry = P.alpha_carry ? la : 0.0;
-      D.nacc += 1; D.nacc_total += 1;
     }
-    D.natt += 1; D.steps_total += 1; D.step = step;
-    if (reflect) {
-      const double sz = (double)(hi - lo + 1);
-      DX.ncluster += 1.0; DX.cluster_sum += sz; DX.cluster_max = fmax(DX.cluster_max, sz);
-    }
+    commit_trial(P, D, DX, accept, step, dU, g.dOmega, dsu, Dx, Dy, Dz, g.dpx, g.dpy, g.dpz, g.dpsi, g.dcos2, la, reflect,
+                 lo, hi);
     bookkeep<COMP>(P, D, step);
     record_extras<COMP>(P, DX, D.su, D.log_gauge, n);
     if (a.stepout > 0 && (step % a.stepout) == 0) {

@@ -148,10 +148,7 @@ __device__ __forceinline__ float2 rect_pair_f32x2(const LanePairF& it, const flo
   return __ffma2_rn(neg2(t), __fmul2_rn(y2, y), acc);
 }
 
-#ifndef PMC_KFLUSH
-#define PMC_KFLUSH 32
-#endif
-constexpr int kFlush = PMC_KFLUSH;
+constexpr int kFlush = 32;
 
 // One pass over bundles of NL groups of 32 lane items (groups g0, g0+NL, …: `nb` bundles) against the B broadcast
 // items; the (bundle, broadcast item) space is split evenly over the team's warps.  Returns this thread's share.
@@ -311,7 +308,7 @@ template <int T>
 __device__ __forceinline__ double cta_delta_pairs_f32(const CtaView& S, const F32View& F, int n, double b, int idx,
                                                       double npx, double npy, double npz, double dnx, double dny,
                                                       double dnz) {
-  const double acc = delta_pairs_partial_f32<Team<T / 32, 0>>(S, F, n, b, idx, npx, npy, npz, dnx, dny, dnz);
+  const double acc = delta_pairs_partial_f32<Team<T / 32>>(S, F, n, b, idx, npx, npy, npz, dnx, dny, dnz);
   return block_sum<T>(acc, S.part, /*trailing_sync=*/false);
 }
 

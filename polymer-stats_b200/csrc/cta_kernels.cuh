@@ -184,25 +184,20 @@ __device__ double cta_pair_energy(const CtaView& S, int n, int energy_type, doub
 //   Measured from the pivot, the rounding error of |r'|² is of order eps·|x_k − x_idx|·|D|, the order r
 //   itself already carries;
 //   g = y³(μ_L·μ_B + (−3μ_L·r)(μ_B·r) y²),  y = 1/|r|.
-// -DPMC_RECT_Q2=0 builds the previous form (r' formed and squared, 43 FP64 instructions) for comparisons.
 // Shared-memory loads are not free next to the FP64 pipe (≈1.7 issue cycles per LDS.64 against 2 per
 // DFMA, tools/fp64_mix.cu), so each lane keeps NL=2 lane items and every broadcast item loaded from
 // shared memory serves two pairs; an odd last group of 32 lane items runs with NL=1.
-// A team = the warps that share the pair work of one chain: the whole CTA (FIRST_WARP = 0, plain
-// __syncthreads) or the worker warps of the warp-specialised kernel (named barrier 1).
-template <int NW, int FIRST_WARP>
+// A team = the warps that share the pair work of one chain: here the whole CTA.
+template <int NW>
 struct Team {
   static constexpr int kWarps = NW;
   static constexpr int kThreads = NW * 32;
   static constexpr int kLocalThreads = NW * 32;   // threads that share ONE copy of the staged chain (see PairTeam)
-  __device__ __forceinline__ static int tid() { return (int)threadIdx.x - FIRST_WARP * 32; }
+  __device__ __forceinline__ static int tid() { return (int)threadIdx.x; }
   __device__ __forceinline__ static int ltid() { return tid(); }
-  __device__ __forceinline__ static int warp() { return (int)(threadIdx.x >> 5) - FIRST_WARP; }
+  __device__ __forceinline__ static int warp() { return (int)(threadIdx.x >> 5); }
   __device__ __forceinline__ static int lane() { return (int)(threadIdx.x & 31); }
-  __device__ __forceinline__ static void sync() {
-    if (FIRST_WARP == 0) __syncthreads();
-    else asm volatile("bar.sync 1, %0;" ::"n"(NW * 32) : "memory");
-  }
+  __device__ __forceinline__ static void sync() { __syncthreads(); }
 };
 
 // One warp as the team (chains of ≤ 160 monomers in the composite-trial kernel).
@@ -216,10 +211,6 @@ struct WarpTeam {
   __device__ __forceinline__ static int lane() { return (int)(threadIdx.x & 31); }
   __device__ __forceinline__ static void sync() { __syncwarp(); }
 };
-
-#ifndef PMC_RECT_Q2
-#define PMC_RECT_Q2 1
-#endif
 
 struct LaneItem {
   double x, y, z;     // position
@@ -288,15 +279,9 @@ __device__ __forceinline__ double rect_pair(const LaneItem& it, double bx, doubl
   }
   const double a3n = a3 - it.c;
   const double bn = bb - e;
-#if PMC_RSQ_PAR
-  double y, y2, yn, yn2;
-  rsqrt_y_y2(r2, y, y2);
-  rsqrt_y_y2(q2, yn, yn2);
-#else
   const double y = rsqrt_fast(r2);
   const double yn = rsqrt_fast(q2);
   const double y2 = y * y, yn2 = yn * yn;
-#endif
   const double t = fma(a3 * bb, y2, mm);
   const double tn = fma(a3n * bn, yn2, mm);
   if constexpr (CUT) {
@@ -427,7 +412,7 @@ __device__ __forceinline__ double delta_pairs_partial(const CtaView& S, int n, i
     lanes_are_heads = costH <= costT;
     // {eB, 2p_B} of the broadcast side fill 2B of the n doubles of S.E: at most one side (H + Tl = n − 1) has more
     // than n/2 items, and it goes on the lanes
-    if (PMC_RECT_Q2 && 2 * (lanes_are_heads ? Tl : H) > n) lanes_are_heads = !lanes_are_heads;
+    if (2 * (lanes_are_heads ? Tl : H) > n) lanes_are_heads = !lanes_are_heads;
   }
   // D_eff: r = x_L − x_B.  L=head,B=tail: r' = r − D.  L=tail,B=head: r' = r + D.
   const double sgn = lanes_are_heads ? 1.0 : -1.0;
@@ -437,7 +422,7 @@ __device__ __forceinline__ double delta_pairs_partial(const CtaView& S, int n, i
   const double xi = S.sx[idx], yi = S.sy[idx], zi = S.sz[idx];  // the pivot of the Q2 projections
   if (rect)  // every copy of the staged chain needs its own E
     for (int k = TEAM::ltid(); k < B; k += TEAM::kLocalThreads)
-      rect_prepass_item<PMC_RECT_Q2>(S, baseB, k, xi, yi, zi, ex, ey, ez);
+      rect_prepass_item<true>(S, baseB, k, xi, yi, zi, ex, ey, ez);
   // row {idx}×rest: both μ_idx and the separation change.
   double acc = 0.0;
   {
@@ -455,7 +440,7 @@ __device__ __forceinline__ double delta_pairs_partial(const CtaView& S, int n, i
     }
   }
   TEAM::sync();  // E visible
-  if (rect) acc += rect_sum<TEAM, UNROLL, false, false, PMC_RECT_Q2>(S, baseA, A, baseB, B, ex, ey, ez, 0.0, idx);
+  if (rect) acc += rect_sum<TEAM, UNROLL, false, false, true>(S, baseA, A, baseB, B, ex, ey, ez, 0.0, idx);
   return acc;
 }
 
@@ -464,7 +449,7 @@ template <int T, int UNROLL = 2>
 __device__ __forceinline__ double cta_delta_pairs(const CtaView& S, int n, int energy_type, double b, int idx,
                                                   double npx, double npy, double npz, double dnx, double dny,
                                                   double dnz) {
-  const double acc = delta_pairs_partial<Team<T / 32, 0>, UNROLL>(S, n, energy_type, b, idx, npx, npy, npz, dnx, dny, dnz);
+  const double acc = delta_pairs_partial<Team<T / 32>, UNROLL>(S, n, energy_type, b, idx, npx, npy, npz, dnx, dny, dnz);
   return block_sum<T>(acc, S.part, /*trailing_sync=*/false);
 }
 
@@ -498,11 +483,12 @@ struct RunArgs {
   int window;      // k_run_warp_cluster: trials per window (≤ 32)
 };
 
-// Thread 0: draw and build the proposal of trial `step`.
+// Thread 0 (window: lane k for trial step + k): draw and build the proposal of trial `step`.  `init` = D.init (the
+// window passes the copy it keeps in a register, the rebuild of a stale entry reads D).
 __device__ __forceinline__ void make_proposal(const RunArgs& a, const ChainParams& P, const ChainDyn& D,
-                                              const MonoRec* mono, uint32_t chain_id, long long step,
+                                              const MonoRec* mono, uint32_t chain_id, uint32_t init, long long step,
                                               Proposal& q) {
-  const Draws d = draw_step(a.seed, chain_id, (uint32_t)D.init, step, a.n);
+  const Draws d = draw_step(a.seed, chain_id, init, step, a.n);
   const MonoRec rec = mono[d.idx];
   double dphi, dtheta;
   increments(P, d, rec.theta, D.phi_step, D.theta_step, dphi, dtheta);
@@ -552,97 +538,93 @@ __device__ __forceinline__ void stage_row(const ChainDyn& D, long long step, dou
   for (int k = 0; k < 16; ++k) rowbuf[9 + k] = (D.acc[k] + D.comp[k]) / nrm;
 }
 
-// The hot loop (mcmc_eap_chain.jl:276-350) for one interacting chain per CTA.
-template <int T, int MINB, int UNROLL = 2>
-__global__ void __launch_bounds__(T, MINB) k_run_cta(const RunArgs a) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const CtaView S = carve(smem_raw, a.n);
-  const int c = blockIdx.x;
-  const int tid = threadIdx.x;
-  const int n = a.n;
-  MonoRec* mono = a.mono + (size_t)c * n;
-  if (tid == 0) {
-    *S.par = a.par[c];
-    *S.dyn = a.dyn[c];
+// Warp 0, lane = tid: output row `row` of chain c after trial `step`, staged by lane 0.
+__device__ __forceinline__ void emit_row(const RunArgs& a, const ChainDyn& D, int c, long long row, long long step,
+                                         double* rowbuf, int tid) {
+  if (tid == 0) stage_row(D, step, rowbuf);
+  __syncwarp();
+  if (row < a.rows) {
+    if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = rowbuf[tid];
+    if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = rowbuf[8 + tid];
   }
-  __syncthreads();
-  const ChainParams& P = *S.par;
-  load_chain<T>(mono, P, n, S);
-  const uint32_t chain_id = a.chain_id_base + (uint32_t)c;
-  const double b = P.b, inv_kT = P.inv_kT;
-  const long long step0 = S.dyn->step;
-  long long row = 0;
-  if (tid == 0) make_proposal(a, P, *S.dyn, mono, chain_id, step0 + 1, S.prop[1]);
-
-  for (long long s = 1; s <= a.nsteps; ++s) {
-    const long long step = step0 + s;
-    __syncthreads();  // (A) proposal of this trial and state updates of the previous one are visible
-    const Proposal* q = &S.prop[s & 1];
-    const int idx = q->idx;
-    const bool skip = q->skip;
-    const double dnx = q->dnx, dny = q->dny, dnz = q->dnz;
-    double dsum = 0.0;
-    bool accept = false;
-    if (!skip) {
-      dsum = kInv4Pi * cta_delta_pairs<T, UNROLL>(S, n, 1, b, idx, q->mx, q->my, q->mz, dnx, dny, dnz);
-      accept = metropolis(q->single - dsum * inv_kT, q->eps);
-    }
-    if (accept) {  // apply move!: x_idx += (b/2)Δn̂, x_{j>idx} += bΔn̂, μ_idx = μ'
-      const double Dx = b * dnx, Dy = b * dny, Dz = b * dnz;
-      for (int j = idx + 1 + tid; j < n; j += T) {
-        S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-      }
-    }
-    if (tid == 0) {
-      if (accept) {
-        S.sx[idx] += 0.5 * b * dnx; S.sy[idx] += 0.5 * b * dny; S.sz[idx] += 0.5 * b * dnz;
-        S.mx[idx] = q->mx; S.my[idx] = q->my; S.mz[idx] = q->mz;
-        MonoRec rec;
-        rec.phi = q->phi; rec.theta = q->theta;
-        rec.nx = q->nx; rec.ny = q->ny; rec.nz = q->nz; rec.sth = q->sth;
-        mono[idx] = rec;
-      }
-      after_decision(P, *S.dyn, *q, accept, dsum, step);
-    }
-    const bool isrow = a.stepout > 0 && (step % a.stepout) == 0;
-    if (isrow && tid < 32) {
-      if (tid == 0) stage_row(*S.dyn, step, S.rowbuf);
-      __syncwarp();
-      if (row < a.rows) {
-        if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-        if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-      }
-      __syncwarp();
-    }
-    if (isrow) ++row;
-    if (tid == 0 && s < a.nsteps) make_proposal(a, P, *S.dyn, mono, chain_id, step + 1, S.prop[(s + 1) & 1]);
-  }
-  __syncthreads();
-  if (tid == 0) a.dyn[c] = *S.dyn;
+  __syncwarp();
 }
 
-// The accept/reject decision from the summed pair partials; explicit rounding so that every call site
-// (control warp and workers) takes bit-identical decisions.
+// The record of monomer q.idx after the move of q.
+__device__ __forceinline__ MonoRec record_of(const Proposal& q) {
+  MonoRec rec;
+  rec.phi = q.phi; rec.theta = q.theta;
+  rec.nx = q.nx; rec.ny = q.ny; rec.nz = q.nz; rec.sth = q.sth;
+  return rec;
+}
+
+// move! of an accepted trial, tail part: x_j += D for j ≥ first, by threads tid, tid + stride, …
+__device__ __forceinline__ void shift_tail(const CtaView& S, int first, int n, double Dx, double Dy, double Dz, int tid,
+                                           int stride) {
+  for (int j = first + tid; j < n; j += stride) {
+    S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
+  }
+}
+
+// move! of an accepted single-monomer trial, by one thread: x_idx += (b/2)Δn̂, μ_idx = μ', and the record.
+__device__ __forceinline__ void move_pivot(const CtaView& S, MonoRec* mono, const Proposal& q, int idx, double b,
+                                           double dnx, double dny, double dnz) {
+  S.sx[idx] += 0.5 * b * dnx; S.sy[idx] += 0.5 * b * dny; S.sz[idx] += 0.5 * b * dnz;
+  S.mx[idx] = q.mx; S.my[idx] = q.my; S.mz[idx] = q.mz;
+  mono[idx] = record_of(q);
+}
+
+// The accept/reject decision from the summed pair partials; explicit rounding so that every kernel takes
+// bit-identical decisions.
 __device__ __forceinline__ bool decide(double single, double tsum, double inv_kT, double eps, double& dsum) {
   dsum = __dmul_rn(kInv4Pi, tsum);
   return metropolis(__fma_rn(-dsum, inv_kT, single), eps);
 }
 
-__device__ __forceinline__ void cta_sync() { asm volatile("bar.sync 0;" ::: "memory"); }
-
-// Windowed variant of the hot loop: the serial part of a trial (Philox, sincos, log, …) is taken off
-// the per-trial critical path by building the proposals of the next WIN trials at once, one trial
-// per lane of warp 0.  A proposal depends on the chain only through the record of its own monomer, so
-// it stays valid unless an earlier trial of the window moves the same monomer: accepted trials mark
-// later same-monomer proposals dirty and those are rebuilt (serially, rarely) when their turn comes.
-// A window never crosses a step-size adaptation boundary (mcmc_eap_chain.jl:301-322).
+// Proposal windows: the serial part of a trial (Philox, sincos, log, …) is taken off the per-trial critical path by
+// building the proposals of the next kWin trials at once, one trial per lane of warp 0.  A proposal depends on the
+// chain only through the record of its own monomer, so it stays valid unless an earlier trial of the window moves
+// that monomer: accepted trials mark later proposals on the monomers they moved stale, and those are rebuilt
+// (serially, rarely) when their turn comes.  A window never crosses a step-size adaptation boundary
+// (mcmc_eap_chain.jl:301-322).
 constexpr int kWin = 32;
+
+// Trials of the window that starts at trial s.  to_boundary = trials until the adaptation rule runs next (0: never).
+__device__ __forceinline__ int window_len(const RunArgs& a, const ChainParams& P, bool adapt_on, long long step0,
+                                          long long s, long long& to_boundary) {
+  long long wl = a.nsteps - s + 1;
+  if (wl > kWin) wl = kWin;
+  to_boundary = 0;
+  if (adapt_on) {
+    to_boundary = P.steps_per_adjust - ((step0 + s - 1) % P.steps_per_adjust);  // ≥ 1
+    if (wl > to_boundary) wl = to_boundary;
+  }
+  return (int)wl;
+}
+
+// Warp 0, lane = tid: entry `tid` of the window is trial step + tid, built by make(tid, step + tid); no entry is stale.
+template <class Make>
+__device__ __forceinline__ void build_window(long long step, int wlen, unsigned& dirty, int tid, Make&& make) {
+  if (tid < wlen) make(tid, step + tid);
+  if (tid == 0) dirty = 0u;
+}
+
+// Warp 0, lane = tid: trial k of the window was accepted and moved monomers lo … hi; later entries on them are stale.
+template <class Entry>
+__device__ __forceinline__ void mark_stale(const Entry* win, int k, int wlen, int lo, int hi, unsigned& dirty,
+                                           int tid) {
+  const int widx = win[tid].idx;
+  const bool stale = tid > k && tid < wlen && widx >= lo && widx <= hi;
+  const unsigned m = __ballot_sync(0xffffffffu, stale);
+  if (tid == 0 && m) dirty |= m;
+}
 
 __host__ __device__ inline size_t cta_smem_bytes_win(int n) {
   return (cta_smem_bytes(n) + kWin * sizeof(Proposal) + 16 + 15) & ~(size_t)15;
 }
 __host__ __device__ inline size_t cta_smem_bytes_win_f32(int n) { return cta_smem_bytes_win(n) + f32_smem_bytes(n); }
 
+// The hot loop (mcmc_eap_chain.jl:276-350) for one interacting chain per CTA, with proposal windows.
 // PREC = 1: the rectangle of every trial in FP32 (cta_f32.cuh; pmc_set_pair_precision), everything else as PREC = 0.
 template <int T, int MINB, int UNROLL = 2, int PREC = 0>
 __global__ void __launch_bounds__(T, MINB) k_run_cta_win(const RunArgs a) {
@@ -662,7 +644,7 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_win(const RunArgs a) {
   __syncthreads();
   const ChainParams& P = *S.par;
   load_chain<T>(mono, P, n, S);
-  if (PREC) fill_mu_f32<Team<T / 32, 0>>(S, F, n);   // visible after the window barrier below
+  if (PREC) fill_mu_f32<Team<T / 32>>(S, F, n);   // visible after the window barrier below
   const uint32_t chain_id = a.chain_id_base + (uint32_t)c;
   const double b = P.b, inv_kT = P.inv_kT;
   const long long step0 = S.dyn->step;
@@ -673,28 +655,16 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_win(const RunArgs a) {
   long long s = 1;
   while (s <= a.nsteps) {
     // ---- window [s, s+wlen) ----------------------------------------------------------------------
-    long long wl = a.nsteps - s + 1;
-    if (wl > kWin) wl = kWin;
-    if (adapt_on) {
-      const long long to_boundary = P.steps_per_adjust - ((step0 + s - 1) % P.steps_per_adjust);  // ≥1
-      if (wl > to_boundary) wl = to_boundary;
-    }
-    const int wlen = (int)wl;
-    if (tid < 32) {
-      if (tid < wlen) {
-        const Draws d = draw_step(a.seed, chain_id, init, step0 + s + tid, n);
-        const MonoRec rec = mono[d.idx];
-        double dphi, dtheta;
-        increments(P, d, rec.theta, S.dyn->phi_step, S.dyn->theta_step, dphi, dtheta);
-        build_proposal(P, rec, d.idx, dphi, dtheta, d.eps, win[tid]);
-      }
-      if (tid == 0) *dirty = 0u;
-    }
+    long long to_boundary;
+    const int wlen = window_len(a, P, adapt_on, step0, s, to_boundary);
+    if (tid < 32)
+      build_window(step0 + s, wlen, *dirty, tid,
+                   [&](int e, long long st) { make_proposal(a, P, *S.dyn, mono, chain_id, init, st, win[e]); });
     __syncthreads();  // window visible
     for (int k = 0; k < wlen; ++k) {
       const long long step = step0 + s + k;
       if ((*dirty >> k) & 1u) {  // an earlier trial of this window moved the same monomer: rebuild
-        if (tid == 0) make_proposal(a, P, *S.dyn, mono, chain_id, step, win[k]);
+        if (tid == 0) make_proposal(a, P, *S.dyn, mono, chain_id, (uint32_t)S.dyn->init, step, win[k]);
         __syncthreads();
       }
       const Proposal* q = &win[k];
@@ -708,39 +678,19 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_win(const RunArgs a) {
                               : cta_delta_pairs<T, UNROLL>(S, n, 1, b, idx, q->mx, q->my, q->mz, dnx, dny, dnz);
         accept = decide(q->single, t, inv_kT, q->eps, dsum);
       }
-      if (accept) {  // apply move!: x_idx += (b/2)Δn̂, x_{j>idx} += bΔn̂, μ_idx = μ'
-        const double Dx = b * dnx, Dy = b * dny, Dz = b * dnz;
-        for (int j = idx + 1 + tid; j < n; j += T) {
-          S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-        }
-        if (tid < 32) {  // later proposals of the window on the same monomer are stale now
-          const bool stale = tid > k && tid < wlen && win[tid].idx == idx;
-          const unsigned m = __ballot_sync(0xffffffffu, stale);
-          if (tid == 0 && m) *dirty |= m;
-        }
+      if (accept) {
+        shift_tail(S, idx + 1, n, b * dnx, b * dny, b * dnz, tid, T);
+        if (tid < 32) mark_stale(win, k, wlen, idx, idx, *dirty, tid);
       }
       if (tid == 0) {
         if (accept) {
-          S.sx[idx] += 0.5 * b * dnx; S.sy[idx] += 0.5 * b * dny; S.sz[idx] += 0.5 * b * dnz;
-          S.mx[idx] = q->mx; S.my[idx] = q->my; S.mz[idx] = q->mz;
+          move_pivot(S, mono, *q, idx, b, dnx, dny, dnz);
           if (PREC) F.pb[idx] = make_float4((float)q->mx, (float)q->my, (float)q->mz, 0.0f);   // w is rebuilt per trial
-          MonoRec rec;
-          rec.phi = q->phi; rec.theta = q->theta;
-          rec.nx = q->nx; rec.ny = q->ny; rec.nz = q->nz; rec.sth = q->sth;
-          mono[idx] = rec;
         }
         after_decision(P, *S.dyn, *q, accept, dsum, step);
       }
       const bool isrow = a.stepout > 0 && (step % a.stepout) == 0;
-      if (isrow && tid < 32) {
-        if (tid == 0) stage_row(*S.dyn, step, S.rowbuf);
-        __syncwarp();
-        if (row < a.rows) {
-          if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-          if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-        }
-        __syncwarp();
-      }
+      if (isrow && tid < 32) emit_row(a, *S.dyn, c, row, step, S.rowbuf, tid);
       if (isrow) ++row;
       __syncthreads();  // state, records and dirty mask of this trial are visible
     }
@@ -799,26 +749,16 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_win_spec(const RunArgs
   const uint32_t init = (uint32_t)S.dyn->init;
   const bool adapt_on = P.adj_scale != 1.0 && P.steps_per_adjust > 0;
   long long row = 0;
-  Countdown row_due, adapt_due;
+  Countdown row_due;
   row_due.start(step0, a.stepout);
-  adapt_due.start(step0, adapt_on ? P.steps_per_adjust : 0);
 
   long long s = 1;
   while (s <= a.nsteps) {
-    long long wl = a.nsteps - s + 1;
-    if (wl > kWin) wl = kWin;
-    if (adapt_on && wl > adapt_due.left) wl = adapt_due.left;   // windows never cross an adaptation boundary
-    const int wlen = (int)wl;
-    if (tid < 32) {
-      if (tid < wlen) {
-        const Draws d = draw_step(a.seed, chain_id, init, step0 + s + tid, n);
-        const MonoRec rec = mono[d.idx];
-        double dphi, dtheta;
-        increments(P, d, rec.theta, S.dyn->phi_step, S.dyn->theta_step, dphi, dtheta);
-        build_proposal(P, rec, d.idx, dphi, dtheta, d.eps, win[tid]);
-      }
-      if (tid == 0) *dirty = 0u;
-    }
+    long long to_boundary;
+    const int wlen = window_len(a, P, adapt_on, step0, s, to_boundary);
+    if (tid < 32)
+      build_window(step0 + s, wlen, *dirty, tid,
+                   [&](int e, long long st) { make_proposal(a, P, *S.dyn, mono, chain_id, init, st, win[e]); });
     __syncthreads();  // window visible
     int k = 0;
     while (k < wlen) {
@@ -827,7 +767,7 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_win_spec(const RunArgs
       if (g < nb) {
         const int kk = k + g;
         if ((*dirty >> kk) & 1u) {  // an accepted trial of this window moved the same monomer: rebuild the entry
-          if (lane == 0) make_proposal(a, P, *S.dyn, mono, chain_id, step0 + s + kk, win[kk]);
+          if (lane == 0) make_proposal(a, P, *S.dyn, mono, chain_id, (uint32_t)S.dyn->init, step0 + s + kk, win[kk]);
           __syncwarp();
         }
         const Proposal* q = &win[kk];
@@ -851,43 +791,18 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_win_spec(const RunArgs
         const Proposal* q = &win[kk];
         const bool accept = res[bb].accept != 0;
         const int idx = q->idx;
-        if (accept) {  // apply move!: x_idx += (b/2)Δn̂, x_{j>idx} += bΔn̂, μ_idx = μ'
-          const double Dx = b * q->dnx, Dy = b * q->dny, Dz = b * q->dnz;
-          for (int j = idx + 1 + tid; j < n; j += T) {
-            S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-          }
-          if (tid < 32) {  // later proposals of the window on the same monomer are stale now
-            const bool stale = tid > kk && tid < wlen && win[tid].idx == idx;
-            const unsigned m = __ballot_sync(0xffffffffu, stale);
-            if (tid == 0 && m) *dirty |= m;
-          }
+        if (accept) {
+          shift_tail(S, idx + 1, n, b * q->dnx, b * q->dny, b * q->dnz, tid, T);
+          if (tid < 32) mark_stale(win, kk, wlen, idx, idx, *dirty, tid);
         }
         if (tid == 0) {
-          if (accept) {
-            S.sx[idx] += 0.5 * b * q->dnx; S.sy[idx] += 0.5 * b * q->dny; S.sz[idx] += 0.5 * b * q->dnz;
-            S.mx[idx] = q->mx; S.my[idx] = q->my; S.mz[idx] = q->mz;
-            MonoRec rec;
-            rec.phi = q->phi; rec.theta = q->theta;
-            rec.nx = q->nx; rec.ny = q->ny; rec.nz = q->nz; rec.sth = q->sth;
-            mono[idx] = rec;
-          }
+          if (accept) move_pivot(S, mono, *q, idx, b, q->dnx, q->dny, q->dnz);
           apply_decision(P, *S.dyn, *q, accept, res[bb].dsum, step);
-        }
-        const bool adapt_now = adapt_due.tick();   // every thread keeps the same countdowns
-        if (tid == 0) {
-          if (adapt_now) adapt_apply(P, S.dyn->phi_step, S.dyn->theta_step, S.dyn->nacc, S.dyn->natt);
+          if (kk + 1 == to_boundary) adapt_apply(P, S.dyn->phi_step, S.dyn->theta_step, S.dyn->nacc, S.dyn->natt);
           record_averages<true>(P, S.dyn->acc, S.dyn->comp, S.dyn->r, S.dyn->p, S.dyn->U, S.dyn->su, S.dyn->log_gauge);
         }
         const bool isrow = row_due.tick();
-        if (isrow && tid < 32) {
-          if (tid == 0) stage_row(*S.dyn, step, S.rowbuf);
-          __syncwarp();
-          if (row < a.rows) {
-            if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-            if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-          }
-          __syncwarp();
-        }
+        if (isrow && tid < 32) emit_row(a, *S.dyn, c, row, step, S.rowbuf, tid);
         if (isrow) ++row;
         ++committed;
         if (accept) break;  // the speculations behind this trial saw the chain before it
@@ -898,172 +813,6 @@ __global__ void __launch_bounds__(32 * G, MINB) k_run_cta_win_spec(const RunArgs
     s += wlen;
   }
   if (tid == 0) a.dyn[c] = *S.dyn;
-}
-
-// Warp-specialised variant of the hot loop: warp 0 is the control warp (RNG, proposal, bookkeeping,
-// output rows), warps 1..WK are the workers that own the pair sums.  The control warp prepares the
-// proposal of trial s+1 and does the bookkeeping of trial s−1 WHILE the workers evaluate trial s, so
-// the serial per-trial work leaves the critical path.  The proposal of trial s+1 depends on the
-// outcome of trial s only when both touch the same monomer, or when trial s ends an adaptation
-// window (step sizes may change): those cases are built after the decision instead.
-// Barriers per trial: two whole-CTA (proposal published / partial sums ready) + one workers-only.
-template <int WK, int MINB, int UNROLL = 2>
-__global__ void __launch_bounds__((WK + 1) * 32, MINB) k_run_cta_ws(const RunArgs a) {
-  using TEAM = Team<WK, 1>;
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const CtaView S = carve(smem_raw, a.n);
-  const int c = blockIdx.x;
-  const int tid = threadIdx.x;
-  const int n = a.n;
-  const bool control = tid < 32;
-  MonoRec* mono = a.mono + (size_t)c * n;
-  if (tid == 0) {
-    *S.par = a.par[c];
-    *S.dyn = a.dyn[c];
-  }
-  __syncthreads();
-  const ChainParams& P = *S.par;
-  load_chain<(WK + 1) * 32>(mono, P, n, S);
-  const uint32_t chain_id = a.chain_id_base + (uint32_t)c;
-  const double b = P.b, inv_kT = P.inv_kT;
-  const long long step0 = S.dyn->step;
-  const bool adapt_on = P.adj_scale != 1.0 && P.steps_per_adjust > 0;
-  double* part = S.part;  // [2][WK] ping-pong by trial parity
-
-  if (control) {
-    ChainDyn& D = *S.dyn;
-    long long row = 0;
-    bool booked = true;  // bookkeeping of the previous trial done?
-    if (tid == 0) make_proposal(a, P, D, mono, chain_id, step0 + 1, S.prop[1]);
-    cta_sync();  // (A) of trial 1
-    for (long long s = 1; s <= a.nsteps; ++s) {
-      const long long step = step0 + s;
-      const Proposal* q = &S.prop[s & 1];
-      // ---- overlapped with the workers' pair sums of trial s -------------------------------------
-      if (!booked) {  // bookkeeping of trial s−1
-        const long long pstep = step - 1;
-        if (tid == 0) bookkeep(P, D, pstep);
-        const bool isrow = a.stepout > 0 && (pstep % a.stepout) == 0;
-        if (isrow) {
-          if (tid == 0) stage_row(D, pstep, S.rowbuf);
-          __syncwarp();
-          if (row < a.rows) {
-            if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-            if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-          }
-          __syncwarp();
-          ++row;
-        }
-        booked = true;
-      }
-      const bool last = (s == a.nsteps);
-      const bool adapt_step = adapt_on && (step % P.steps_per_adjust) == 0;
-      bool deferred = false;
-      if (!last && tid == 0) {
-        const Draws d = draw_step(a.seed, chain_id, (uint32_t)D.init, step + 1, n);
-        if (d.idx == q->idx || adapt_step) {
-          deferred = true;
-        } else {
-          const MonoRec rec = mono[d.idx];
-          double dphi, dtheta;
-          increments(P, d, rec.theta, D.phi_step, D.theta_step, dphi, dtheta);
-          build_proposal(P, rec, d.idx, dphi, dtheta, d.eps, S.prop[(s + 1) & 1]);
-        }
-      }
-      cta_sync();  // (C) partial sums of trial s are in part[s&1]
-      // ---- decision (the workers take the same one) ----------------------------------------------
-      if (tid == 0) {
-        double dsum = 0.0;
-        bool accept = false;
-        if (!q->skip) {
-          const double* ps = part + (s & 1) * WK;
-          double t = 0.0;
-#pragma unroll
-          for (int w = 0; w < WK; ++w) t += ps[w];
-          accept = decide(q->single, t, inv_kT, q->eps, dsum);
-        }
-        if (accept) {
-          MonoRec rec;
-          rec.phi = q->phi; rec.theta = q->theta;
-          rec.nx = q->nx; rec.ny = q->ny; rec.nz = q->nz; rec.sth = q->sth;
-          mono[q->idx] = rec;
-        }
-        apply_decision(P, D, *q, accept, dsum, step);
-        if (deferred) {
-          bookkeep(P, D, step);  // adaptation must precede the next proposal
-          make_proposal(a, P, D, mono, chain_id, step + 1, S.prop[(s + 1) & 1]);
-        }
-      }
-      deferred = __shfl_sync(0xffffffffu, (int)deferred, 0) != 0;
-      booked = false;
-      if (deferred) {  // rows of a trial booked early
-        const bool isrow = a.stepout > 0 && (step % a.stepout) == 0;
-        if (isrow) {
-          if (tid == 0) stage_row(D, step, S.rowbuf);
-          __syncwarp();
-          if (row < a.rows) {
-            if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-            if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-          }
-          __syncwarp();
-          ++row;
-        }
-        booked = true;
-      }
-      cta_sync();  // (A) of trial s+1: proposal published
-    }
-    if (!booked) {  // bookkeeping of the last trial
-      const long long pstep = step0 + a.nsteps;
-      if (tid == 0) bookkeep(P, D, pstep);
-      const bool isrow = a.stepout > 0 && (pstep % a.stepout) == 0;
-      if (isrow) {
-        if (tid == 0) stage_row(D, pstep, S.rowbuf);
-        __syncwarp();
-        if (row < a.rows) {
-          if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-          if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-        }
-        __syncwarp();
-      }
-    }
-    if (tid == 0) a.dyn[c] = D;
-  } else {
-    // ---- workers ----------------------------------------------------------------------------------
-    const int wtid = TEAM::tid();
-    cta_sync();  // (A) of trial 1
-    for (long long s = 1; s <= a.nsteps; ++s) {
-      const Proposal* q = &S.prop[s & 1];
-      const int idx = q->idx;
-      const bool skip = q->skip;
-      const double dnx = q->dnx, dny = q->dny, dnz = q->dnz;
-      double* ps = part + (s & 1) * WK;
-      if (!skip) {
-        double acc = delta_pairs_partial<TEAM, UNROLL>(S, n, 1, b, idx, q->mx, q->my, q->mz, dnx, dny, dnz);
-        acc = warp_sum(acc);
-        if (TEAM::lane() == 0) ps[TEAM::warp()] = acc;
-      }
-      cta_sync();  // (C)
-      bool accept = false;
-      if (!skip) {
-        double t = 0.0;
-#pragma unroll
-        for (int w = 0; w < WK; ++w) t += ps[w];
-        double dsum;
-        accept = decide(q->single, t, inv_kT, q->eps, dsum);
-      }
-      if (accept) {  // apply move!: x_idx += (b/2)Δn̂, x_{j>idx} += bΔn̂, μ_idx = μ'
-        const double Dx = b * dnx, Dy = b * dny, Dz = b * dnz;
-        for (int j = idx + 1 + wtid; j < n; j += TEAM::kThreads) {
-          S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-        }
-        if (wtid == 0) {
-          S.sx[idx] += 0.5 * Dx; S.sy[idx] += 0.5 * Dy; S.sz[idx] += 0.5 * Dz;
-          S.mx[idx] = q->mx; S.my[idx] = q->my; S.mz[idx] = q->mz;
-        }
-      }
-      cta_sync();  // (A) of trial s+1
-    }
-  }
 }
 
 // Recompute {U, Σu, U_dd, Ω, r, p} of chains from their records (EAPChain ctor tail,
@@ -1097,6 +846,47 @@ __device__ __forceinline__ void bond_sums_partial(const MonoRec* __restrict__ mo
   }
 }
 
+// Totals of one chain, in every thread.
+struct ChainTotals {
+  double U, su, udd, om, ub, sp, c2;
+  double rx, ry, rz, px, py, pz;
+};
+
+// Stage the chain of records `mono` and sum its totals.
+template <int T>
+__device__ __forceinline__ ChainTotals chain_totals(const MonoRec* __restrict__ mono, const ChainParams& P, int n,
+                                                    int energy_type, const CtaView& S) {
+  const int tid = threadIdx.x;
+  load_chain<T>(mono, P, n, S);
+  ChainTotals t;
+  double su = 0, om = 0, px = 0, py = 0, pz = 0;
+  for (int i = tid; i < n; i += T) {
+    su += -0.5 * P.E0 * S.mz[i];
+    om += log(mono[i].sth);
+    px += S.mx[i]; py += S.my[i]; pz += S.mz[i];
+  }
+  double ub, sp, c2;
+  bond_sums_partial<T>(mono, P, n, ub, sp, c2);
+  t.su = block_sum<T>(su, S.part);
+  t.om = block_sum<T>(om, S.part);
+  t.px = block_sum<T>(px, S.part);
+  t.py = block_sum<T>(py, S.part);
+  t.pz = block_sum<T>(pz, S.part);
+  t.ub = block_sum<T>(ub, S.part);
+  t.sp = block_sum<T>(sp, S.part);
+  t.c2 = block_sum<T>(c2, S.part);
+  t.su += t.ub;  // us[i] = u + ubend (eap_chain.jl:130)
+  t.udd = kInv4Pi * cta_pair_energy<T>(S, n, energy_type, P.crad2);
+  // end_to_end (eap_chain.jl:405): x_n + (b/2) n̂_n
+  t.rx = S.sx[n - 1] + 0.5 * P.b * mono[n - 1].nx;
+  t.ry = S.sy[n - 1] + 0.5 * P.b * mono[n - 1].ny;
+  t.rz = S.sz[n - 1] + 0.5 * P.b * mono[n - 1].nz;
+  // energy.jl:7-23; the UCutoff functor (eap_chain.jl:171-192) is the bare pair sum unless cutoff_full
+  const bool bare = (energy_type == 3) && !P.cutoff_full;
+  t.U = bare ? t.udd : t.su + t.udd - (t.rx * P.Fx + t.rz * P.Fz);
+  return t;
+}
+
 template <int T>
 __global__ void __launch_bounds__(T) k_energy_cta(const EnergyArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1107,63 +897,39 @@ __global__ void __launch_bounds__(T) k_energy_cta(const EnergyArgs a) {
   if (tid == 0) *S.par = a.par[c];
   __syncthreads();
   const ChainParams& P = *S.par;
-  load_chain<T>(mono, P, n, S);
-  double su = 0, om = 0, px = 0, py = 0, pz = 0;
-  for (int i = tid; i < n; i += T) {
-    su += -0.5 * P.E0 * S.mz[i];
-    om += log(mono[i].sth);
-    px += S.mx[i]; py += S.my[i]; pz += S.mz[i];
-  }
-  double ub, sp, c2;
-  bond_sums_partial<T>(mono, P, n, ub, sp, c2);
-  su = block_sum<T>(su, S.part);
-  om = block_sum<T>(om, S.part);
-  px = block_sum<T>(px, S.part);
-  py = block_sum<T>(py, S.part);
-  pz = block_sum<T>(pz, S.part);
-  ub = block_sum<T>(ub, S.part);
-  sp = block_sum<T>(sp, S.part);
-  c2 = block_sum<T>(c2, S.part);
-  su += ub;  // us[i] = u + ubend (eap_chain.jl:130)
-  const double udd = kInv4Pi * cta_pair_energy<T>(S, n, a.energy_type, P.crad2);
+  const ChainTotals t = chain_totals<T>(mono, P, n, a.energy_type, S);
   if (tid == 0) {
-    // end_to_end (eap_chain.jl:405): x_n + (b/2) n̂_n
-    const double rx = S.sx[n - 1] + 0.5 * P.b * mono[n - 1].nx;
-    const double ry = S.sy[n - 1] + 0.5 * P.b * mono[n - 1].ny;
-    const double rz = S.sz[n - 1] + 0.5 * P.b * mono[n - 1].nz;
-    // energy.jl:7-23; the UCutoff functor (eap_chain.jl:171-192) is the bare pair sum unless cutoff_full
-    const bool bare = (a.energy_type == 3) && !P.cutoff_full;
-    const double U = bare ? udd : su + udd - (rx * P.Fx + rz * P.Fz);
     if (a.out4) {
       double* o = a.out4 + (size_t)blockIdx.x * 4;
-      o[0] = U; o[1] = su; o[2] = udd; o[3] = om;
+      o[0] = t.U; o[1] = t.su; o[2] = t.udd; o[3] = t.om;
     }
     if (a.out8) {
       double* o = a.out8 + (size_t)blockIdx.x * 8;
-      o[0] = U; o[1] = su; o[2] = udd; o[3] = om;
-      o[4] = ub; o[5] = sp / (double)(n - 1); o[6] = c2; o[7] = 0.0;
+      o[0] = t.U; o[1] = t.su; o[2] = t.udd; o[3] = t.om;
+      o[4] = t.ub; o[5] = t.sp / (double)(n - 1); o[6] = t.c2; o[7] = 0.0;
     }
     if (a.obs6) {
       double* o = a.obs6 + (size_t)blockIdx.x * 6;
-      o[0] = rx; o[1] = ry; o[2] = rz; o[3] = px; o[4] = py; o[5] = pz;
+      o[0] = t.rx; o[1] = t.ry; o[2] = t.rz; o[3] = t.px; o[4] = t.py; o[5] = t.pz;
     }
     if (a.update_dyn) {
       ChainDyn& D = a.dyn[c];
-      if (D.valid) D.drift_max = fmax(D.drift_max, fabs(D.U - U));
-      D.U = U; D.su = su; D.Omega = om;
-      D.r[0] = rx; D.r[1] = ry; D.r[2] = rz;
-      D.p[0] = px; D.p[1] = py; D.p[2] = pz;
-      if (a.rebind_gauge || !D.valid) D.log_gauge = P.gauge0 + om;
+      if (D.valid) D.drift_max = fmax(D.drift_max, fabs(D.U - t.U));
+      D.U = t.U; D.su = t.su; D.Omega = t.om;
+      D.r[0] = t.rx; D.r[1] = t.ry; D.r[2] = t.rz;
+      D.p[0] = t.px; D.p[1] = t.py; D.p[2] = t.pz;
+      if (a.rebind_gauge || !D.valid) D.log_gauge = P.gauge0 + t.om;
       D.valid = 1;
       if (a.dynx) {
-        a.dynx[c].spsi = sp;
-        a.dynx[c].scos2 = c2;
+        a.dynx[c].spsi = t.sp;
+        a.dynx[c].scos2 = t.c2;
       }
     }
   }
 }
 
-// Non-mutating ΔU of one scripted move on one interacting chain (same device code as k_run_cta).
+// Non-mutating ΔU of one scripted move on one interacting chain: what the run kernels evaluate for this move, with
+// the rectangle in FP32 (cta_f32.cuh) for PREC = 1.
 struct DeltaArgs {
   const MonoRec* mono;
   const ChainParams* par;
@@ -1172,46 +938,24 @@ struct DeltaArgs {
   double dphi, dtheta;
 };
 
-template <int T>
+template <int T, int PREC = 0>
 __global__ void __launch_bounds__(T) k_delta_cta(const DeltaArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const CtaView S = carve(smem_raw, a.n);
+  const F32View F = carve_f32(smem_raw + ((cta_smem_bytes(a.n) + 15) & ~(size_t)15), PREC ? a.n : 0, S.E);
   const int tid = threadIdx.x, n = a.n;
   const MonoRec* mono = a.mono + (size_t)a.chain * n;
   if (tid == 0) *S.par = a.par[a.chain];
   __syncthreads();
   const ChainParams& P = *S.par;
   load_chain<T>(mono, P, n, S);
+  if (PREC) fill_mu_f32<Team<T / 32>>(S, F, n);
   if (tid == 0) build_proposal(P, mono[a.idx], a.idx, a.dphi, a.dtheta, 0.0, S.prop[0]);
   __syncthreads();
   const Proposal* q = &S.prop[0];
   const double dsum =
-      kInv4Pi * cta_delta_pairs<T>(S, n, a.energy_type, P.b, a.idx, q->mx, q->my, q->mz, q->dnx, q->dny, q->dnz);
-  if (tid == 0) {
-    a.out[0] = q->du + q->drF + dsum;
-    a.out[1] = q->dOmega;
-    a.out[2] = (double)q->clamped;
-    a.out[3] = dsum;
-  }
-}
-
-// The same with the rectangle in FP32 (cta_f32.cuh): what k_run_cta_win<…, PREC = 1> evaluates for this move.
-template <int T>
-__global__ void __launch_bounds__(T) k_delta_cta_f32(const DeltaArgs a) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const CtaView S = carve(smem_raw, a.n);
-  const F32View F = carve_f32(smem_raw + ((cta_smem_bytes(a.n) + 15) & ~(size_t)15), a.n, S.E);
-  const int tid = threadIdx.x, n = a.n;
-  const MonoRec* mono = a.mono + (size_t)a.chain * n;
-  if (tid == 0) *S.par = a.par[a.chain];
-  __syncthreads();
-  const ChainParams& P = *S.par;
-  load_chain<T>(mono, P, n, S);
-  fill_mu_f32<Team<T / 32, 0>>(S, F, n);
-  if (tid == 0) build_proposal(P, mono[a.idx], a.idx, a.dphi, a.dtheta, 0.0, S.prop[0]);
-  __syncthreads();
-  const Proposal* q = &S.prop[0];
-  const double dsum = kInv4Pi * cta_delta_pairs_f32<T>(S, F, n, P.b, a.idx, q->mx, q->my, q->mz, q->dnx, q->dny, q->dnz);
+      kInv4Pi * (PREC ? cta_delta_pairs_f32<T>(S, F, n, P.b, a.idx, q->mx, q->my, q->mz, q->dnx, q->dny, q->dnz)
+                      : cta_delta_pairs<T>(S, n, a.energy_type, P.b, a.idx, q->mx, q->my, q->mz, q->dnx, q->dny, q->dnz));
   if (tid == 0) {
     a.out[0] = q->du + q->drF + dsum;
     a.out[1] = q->dOmega;
@@ -1242,42 +986,21 @@ __global__ void __launch_bounds__(T) k_reinit_cta(const ReinitArgs a) {
   if (tid == 0) *S.par = a.par[c];
   __syncthreads();
   const ChainParams& P = *S.par;
-  load_chain<T>(cand, P, n, S);
-  double su = 0, om = 0, px = 0, py = 0, pz = 0;
-  for (int i = tid; i < n; i += T) {
-    su += -0.5 * P.E0 * S.mz[i];
-    om += log(cand[i].sth);
-    px += S.mx[i]; py += S.my[i]; pz += S.mz[i];
-  }
-  double ub, sp, c2;
-  bond_sums_partial<T>(cand, P, n, ub, sp, c2);
-  su = block_sum<T>(su, S.part);
-  om = block_sum<T>(om, S.part);
-  px = block_sum<T>(px, S.part);
-  py = block_sum<T>(py, S.part);
-  pz = block_sum<T>(pz, S.part);
-  ub = block_sum<T>(ub, S.part);
-  su += ub;
-  const double udd = kInv4Pi * cta_pair_energy<T>(S, n, a.energy_type, P.crad2);
-  const double rx = S.sx[n - 1] + 0.5 * P.b * cand[n - 1].nx;
-  const double ry = S.sy[n - 1] + 0.5 * P.b * cand[n - 1].ny;
-  const double rz = S.sz[n - 1] + 0.5 * P.b * cand[n - 1].nz;
-  const bool bare = (a.energy_type == 3) && !P.cutoff_full;
-  const double U = bare ? udd : su + udd - (rx * P.Fx + rz * P.Fz);
+  const ChainTotals t = chain_totals<T>(cand, P, n, a.energy_type, S);
   const ChainDyn& D0 = a.dyn[c];
   const uint4 w = philox_at(a.seed, a.chain_id_base + (uint32_t)c, (uint32_t)a.new_init, SUB_REINIT, 0);
   const double eps = u53(w.x, w.y);
   // metropolis_acc (acceptance.jl:1-3) with Π sinθ written as exp(Σ log sinθ)
-  const bool take = P.force_init || (eps <= exp(-(U - D0.U) * P.inv_kT + (om - D0.Omega)));
+  const bool take = P.force_init || (eps <= exp(-(t.U - D0.U) * P.inv_kT + (t.om - D0.Omega)));
   __syncthreads();
   if (take)
     for (int i = tid; i < n; i += T) mono[i] = cand[i];
   if (tid == 0) {
     ChainDyn& D = a.dyn[c];
     if (take) {
-      D.U = U; D.su = su; D.Omega = om;
-      D.r[0] = rx; D.r[1] = ry; D.r[2] = rz;
-      D.p[0] = px; D.p[1] = py; D.p[2] = pz;
+      D.U = t.U; D.su = t.su; D.Omega = t.om;
+      D.r[0] = t.rx; D.r[1] = t.ry; D.r[2] = t.rz;
+      D.p[0] = t.px; D.p[1] = t.py; D.p[2] = t.pz;
     }
     D.init = a.new_init;
     D.step = 0;

@@ -80,7 +80,6 @@ struct pmc_handle {
   int cta_threads = 256;      // block size of the CTA-per-chain kernels
   int sm_count = 148;
   int64_t shape_chains = 0;   // ensemble size the launch shape is chosen for (0 = nchains), pmc_set_ensemble_hint
-  int ws_cfg = 0;             // warp-specialised run kernel variant (0 = classic kernel)
   // O(1)-ΔU chains of the plain driver: one chain per warp below this many chains, else one per lane.  Measured
   // crossover (profiles/r02c_tune_lane_vs_warp.txt): non-interacting 14.8 vs 12.6 G updates/s at 65 536 chains and 14.5 vs
   // 17.5 at 262 144; Ising level at 65 536.  Set from the energy type in launch_run_lane.
@@ -89,7 +88,6 @@ struct pmc_handle {
   int compensated = 0;        // Neumaier-compensated accumulators in the lane/warp kernels (CTA kernels: always)
   int spec_teams = 0;         // > 0: small ensemble of short interacting chains — one-warp teams on different trials (k_run_cta_win_spec)
   int pair_precision = 0;     // 0: FP64 everywhere; 1: the rectangle of single-monomer trials in FP32 where a kernel exists (cta_f32.cuh)
-  int use_win = 1;            // windowed run kernel (batched proposals) whenever shared memory allows
   std::vector<ChainDyn> host_dyn;
   bool dyn_fresh = false, dynx_fresh = false;   // the host copies equal the device's (no launch since they were fetched)
   // clustering driver (mcmc_clustering_eap_chain.jl)
@@ -162,7 +160,6 @@ inline int cluster_fit128(int n) {
 // ---- launch helpers, one translation unit per kernel family -------------------------------------------------
 int launch_run_cta(pmc_handle* h, const pmc::RunArgs& a);                    // run_cta.cu
 bool use_f32_rect(const pmc_handle* h);
-int launch_delta_cta_f32(pmc_handle* h, const DeltaArgs& a);
 int launch_run_pair(pmc_handle* h, const pmc::RunArgs& a);                   // run_pair.cu
 bool use_pair_kernel(const pmc_handle* h);                                   // run_pair.cu
 int launch_run_lane(pmc_handle* h, const pmc::RunArgs& a);                   // run_lane.cu

@@ -12,7 +12,7 @@
 //   * a cluster runs chain after chain from a global queue ordered by PREDICTED work, heaviest first (LPT): the
 //     monomer index of every trial is a counter-based draw that does not depend on the chain's state
 //     (mcmc_eap_chain.jl:277 `idx = rand(1:n)`), so Σ idx·(n−1−idx) of a launch is known before it starts.
-// The Markov chain, its Philox stream and the order of the pair-sum reduction inside a CTA are those of k_run_cta; only
+// The Markov chain, its Philox stream and the order of the pair-sum reduction inside a CTA are those of k_run_cta_win; only
 // the split of the pair set over 2·T threads differs (results agree with the one-CTA kernels to rounding, decisions are
 // the same: tests/test_gpu_round2.py::test_c5_run_kernel_trajectory_n4096).
 #pragma once
@@ -93,6 +93,7 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_pair(const RunArgs a, const
   int* xnext_peer = cluster.map_shared_rank(xnext, rank ^ 1);
   const int tid = threadIdx.x;
   const int n = a.n;
+  cluster.sync();   // both CTAs have started before either touches the other's shared memory
 
   for (;;) {
     // ---- next chain of the queue (both CTAs must agree) ---------------------------------------------------------
@@ -117,7 +118,7 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_pair(const RunArgs a, const
     const double b = P.b, inv_kT = P.inv_kT;
     const long long step0 = S.dyn->step;
     long long row = 0;
-    if (tid == 0) make_proposal(a, P, *S.dyn, mono, chain_id, step0 + 1, S.prop[1]);
+    if (tid == 0) make_proposal(a, P, *S.dyn, mono, chain_id, (uint32_t)S.dyn->init, step0 + 1, S.prop[1]);
 
     for (long long s = 1; s <= a.nsteps; ++s) {
       const long long step = step0 + s;
@@ -142,35 +143,17 @@ __global__ void __launch_bounds__(T, MINB) k_run_cta_pair(const RunArgs a, const
       // scope) and, two trials later, guarantees the peer has read a slot before it is written again.
       cluster.sync();
       if (!skip) accept = decide(pr->single, slot[0] + slot[1], inv_kT, pr->eps, dsum);
-      if (accept) {  // apply move! to this CTA's copy: x_idx += (b/2)Δn̂, x_{j>idx} += bΔn̂, μ_idx = μ'
-        const double Dx = b * dnx, Dy = b * dny, Dz = b * dnz;
-        for (int j = idx + 1 + tid; j < n; j += T) {
-          S.sx[j] += Dx; S.sy[j] += Dy; S.sz[j] += Dz;
-        }
-      }
+      if (accept) shift_tail(S, idx + 1, n, b * dnx, b * dny, b * dnz, tid, T);   // apply move! to this CTA's copy
       if (tid == 0) {
-        if (accept) {
-          S.sx[idx] += 0.5 * b * dnx; S.sy[idx] += 0.5 * b * dny; S.sz[idx] += 0.5 * b * dnz;
-          S.mx[idx] = pr->mx; S.my[idx] = pr->my; S.mz[idx] = pr->mz;
-          MonoRec rec;
-          rec.phi = pr->phi; rec.theta = pr->theta;
-          rec.nx = pr->nx; rec.ny = pr->ny; rec.nz = pr->nz; rec.sth = pr->sth;
-          mono[idx] = rec;   // both CTAs store the same record: each later reads back what its own SM wrote
-        }
+        // both CTAs store the same record: each later reads back what its own SM wrote
+        if (accept) move_pivot(S, mono, *pr, idx, b, dnx, dny, dnz);
         after_decision(P, *S.dyn, *pr, accept, dsum, step);
       }
       const bool isrow = a.stepout > 0 && (step % a.stepout) == 0;
-      if (isrow && tid < 32 && rank == 0) {
-        if (tid == 0) stage_row(*S.dyn, step, S.rowbuf);
-        __syncwarp();
-        if (row < a.rows) {
-          if (tid < 8) a.traj[((size_t)c * a.rows + row) * 8 + tid] = S.rowbuf[tid];
-          if (tid < 17) a.roll[((size_t)c * a.rows + row) * 17 + tid] = S.rowbuf[8 + tid];
-        }
-        __syncwarp();
-      }
+      if (isrow && tid < 32 && rank == 0) emit_row(a, *S.dyn, c, row, step, S.rowbuf, tid);
       if (isrow) ++row;
-      if (tid == 0 && s < a.nsteps) make_proposal(a, P, *S.dyn, mono, chain_id, step + 1, S.prop[(s + 1) & 1]);
+      if (tid == 0 && s < a.nsteps)
+        make_proposal(a, P, *S.dyn, mono, chain_id, (uint32_t)S.dyn->init, step + 1, S.prop[(s + 1) & 1]);
     }
     __syncthreads();
     if (tid == 0 && rank == 0) a.dyn[c] = *S.dyn;

@@ -132,73 +132,48 @@ int check_chain(const pmc_handle* h, int64_t chain) {
 }
 
 // Block size for the CTA-per-chain kernels: enough threads to cover the mean rectangle
-// (n²/6 pairs) without leaving most lanes idle on short chains.  PMC_CTA_THREADS overrides.
-int pick_cta_threads(int n) {
-  int t = n <= 128 ? 64 : n <= 1024 ? 128 : n <= 1536 ? 256 : 512;
-  int o = env_int("PMC_CTA_THREADS", 0);
-  const int cfg = env_int("PMC_RUN_CFG", 0);
-  if (cfg > 0) o = cfg / 100;
-  if (o == 64 || o == 128 || o == 256 || o == 512 || o == 1024) t = o;
-  return t;
+// (n²/6 pairs) without leaving most lanes idle on short chains.
+int pick_cta_threads(int n) { return n <= 128 ? 64 : n <= 1024 ? 128 : n <= 1536 ? 256 : 512; }
+
+// Launch pick(std::integral_constant<int, T>) for the block size T = h->cta_threads chosen at create time (T ≥ MIN_T).
+template <int MIN_T = 32, class Pick, class Args>
+static int launch_cta_kernel(pmc_handle* h, Pick pick, int nblocks, size_t smem, const Args& a) {
+  auto go = [&](auto t) -> int {
+    const auto kernel = pick(t);
+    int rc = set_smem(kernel, smem);
+    if (rc) return rc;
+    kernel<<<nblocks, decltype(t)::value, smem, h->stream>>>(a);
+    ++h->launches;
+    PMC_CU(cudaGetLastError());
+    return PMC_OK;
+  };
+  switch (h->cta_threads) {
+    case 32:
+      if constexpr (MIN_T <= 32) return go(std::integral_constant<int, 32>());
+      break;
+    case 64: return go(std::integral_constant<int, 64>());
+    case 128: return go(std::integral_constant<int, 128>());
+    case 256: return go(std::integral_constant<int, 256>());
+    case 512: return go(std::integral_constant<int, 512>());
+  }
+  return fail(PMC_ERR_INVALID, "bad cta_threads");
 }
 
-// Launch helpers: dispatch on the block size chosen at create time.
 int launch_energy(pmc_handle* h, const EnergyArgs& a, int nblocks) {
-  const size_t smem = cta_smem_bytes(h->n);
-#define PMC_CASE(TT)                                                        \
-  case TT: {                                                                \
-    int rc = set_smem(k_energy_cta<TT>, smem);                              \
-    if (rc) return rc;                                                      \
-    k_energy_cta<TT><<<nblocks, TT, smem, h->stream>>>(a);              \
-    ++h->launches;                  \
-    break;                                                                  \
-  }
-  switch (h->cta_threads) {
-    PMC_CASE(32) PMC_CASE(64) PMC_CASE(128) PMC_CASE(256) PMC_CASE(512) PMC_CASE(1024)
-    default: return fail(PMC_ERR_INVALID, "bad cta_threads");
-  }
-#undef PMC_CASE
-  PMC_CU(cudaGetLastError());
-  return PMC_OK;
+  return launch_cta_kernel(h, [](auto t) { return k_energy_cta<decltype(t)::value>; }, nblocks, cta_smem_bytes(h->n), a);
 }
 
+// ΔU of one scripted move with the rectangle precision the run kernel of this handle uses.
 int launch_delta_cta(pmc_handle* h, const DeltaArgs& a) {
-  const size_t smem = cta_smem_bytes(h->n);
-#define PMC_CASE(TT)                                                        \
-  case TT: {                                                                \
-    int rc = set_smem(k_delta_cta<TT>, smem);                               \
-    if (rc) return rc;                                                      \
-    k_delta_cta<TT><<<1, TT, smem, h->stream>>>(a);                     \
-    ++h->launches;                         \
-    break;                                                                  \
-  }
-  switch (h->cta_threads) {
-    PMC_CASE(32) PMC_CASE(64) PMC_CASE(128) PMC_CASE(256) PMC_CASE(512) PMC_CASE(1024)
-    default: return fail(PMC_ERR_INVALID, "bad cta_threads");
-  }
-#undef PMC_CASE
-  PMC_CU(cudaGetLastError());
-  return PMC_OK;
+  if (use_f32_rect(h))
+    return launch_cta_kernel<64>(h, [](auto t) { return k_delta_cta<decltype(t)::value, 1>; }, 1,
+                                 ((cta_smem_bytes(h->n) + 15) & ~(size_t)15) + f32_smem_bytes(h->n), a);
+  return launch_cta_kernel(h, [](auto t) { return k_delta_cta<decltype(t)::value>; }, 1, cta_smem_bytes(h->n), a);
 }
 
 int launch_reinit(pmc_handle* h, const ReinitArgs& a) {
-  const size_t smem = cta_smem_bytes(h->n);
-  const int nblocks = (int)h->nchains;
-#define PMC_CASE(TT)                                                        \
-  case TT: {                                                                \
-    int rc = set_smem(k_reinit_cta<TT>, smem);                              \
-    if (rc) return rc;                                                      \
-    k_reinit_cta<TT><<<nblocks, TT, smem, h->stream>>>(a);              \
-    ++h->launches;                  \
-    break;                                                                  \
-  }
-  switch (h->cta_threads) {
-    PMC_CASE(32) PMC_CASE(64) PMC_CASE(128) PMC_CASE(256) PMC_CASE(512) PMC_CASE(1024)
-    default: return fail(PMC_ERR_INVALID, "bad cta_threads");
-  }
-#undef PMC_CASE
-  PMC_CU(cudaGetLastError());
-  return PMC_OK;
+  return launch_cta_kernel(h, [](auto t) { return k_reinit_cta<decltype(t)::value>; }, (int)h->nchains,
+                           cta_smem_bytes(h->n), a);
 }
 
 // Recompute the running scalars of every chain from its records (re-synchronisation).
@@ -281,7 +256,7 @@ static int scaled_threads(int base, int minb, size_t smem, int tmax, int64_t cha
   return base * scale;
 }
 
-// (Re)choose cta_threads from n and the ensemble size.  Experiments pin it with PMC_CTA_THREADS / PMC_RUN_CFG.
+// (Re)choose cta_threads from n and the ensemble size.
 static void choose_shape(pmc_handle* h) {
   const int64_t chains = h->shape_chains > 0 ? h->shape_chains : h->nchains;
   const bool cta_pairs = h->energy_type == PMC_ENERGY_INTERACTING || h->energy_type == PMC_ENERGY_CUTOFF;
@@ -311,10 +286,6 @@ static void choose_shape(pmc_handle* h) {
     return;
   }
   const int base = pick_cta_threads(h->n);
-  if (env_int("PMC_CTA_THREADS", 0) > 0 || env_int("PMC_RUN_CFG", 0) > 0) {
-    h->cta_threads = base;
-    return;
-  }
   const int minb = base == 64 ? 8 : base == 128 ? 4 : base == 256 ? 2 : 1;
   h->cta_threads = scaled_threads(base, minb, cta_smem_bytes_win(h->n), 512, chains, h->sm_count);
   // Small ensembles of short interacting chains: one-warp teams on DIFFERENT trials of the window (k_run_cta_win_spec)
@@ -701,7 +672,7 @@ int32_t pmc_delta_u(pmc_handle* h, int64_t chain, int64_t idx0, double dphi, dou
   a.n = h->n; a.energy_type = h->energy_type; a.chain = (int)chain; a.idx = (int)idx0;
   a.dphi = dphi; a.dtheta = dtheta;
   if (h->energy_type == PMC_ENERGY_INTERACTING) {
-    if ((rc = use_f32_rect(h) ? launch_delta_cta_f32(h, a) : launch_delta_cta(h, a))) return rc;
+    if ((rc = launch_delta_cta(h, a))) return rc;
   } else {
     k_delta_lane<<<1, 32, 0, h->stream>>>(a);
     ++h->launches;

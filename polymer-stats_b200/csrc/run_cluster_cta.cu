@@ -28,7 +28,7 @@ int launch_run_cluster_cta(pmc_handle* h, const RunArgs& a) {
     // Small ensembles of short chains (one-warp teams, n ≤ 160): the extra warps choose_shape grants per chain evaluate
     // DIFFERENT trials at the same time (k_run_cta_cluster_spec) instead of sharing one; PMC_CLUSTER_SPEC=0: the shared-trial
     // kernels below (experiments)
-    if (pick_cluster_threads(h->n) == 32 && h->cta_threads > 32 && env_int("PMC_CLUSTER_SPEC", 1) && !env_int("PMC_CLUSTER_CFG", 0)) {
+    if (pick_cluster_threads(h->n) == 32 && h->cta_threads > 32 && env_int("PMC_CLUSTER_SPEC", 1)) {
       const int groups = h->cta_threads / 32;
       const size_t smem = cluster_spec_smem_bytes(h->n, groups);
       if (smem <= (size_t)kSmemMax) {
@@ -54,25 +54,6 @@ int launch_run_cluster_cta(pmc_handle* h, const RunArgs& a) {
 #undef PMC_SP
       }
     }
-    // PMC_CLUSTER_CFG = threads*100 + minblocks selects a tuning variant (experiments only)
-    const int ccfg = env_int("PMC_CLUSTER_CFG", 0);
-#ifdef PMC_TUNING_VARIANTS
-    if (ccfg == 3216) PMC_CL(32, 16)
-    else if (ccfg == 3214) PMC_CL(32, 14)
-    else if (ccfg == 3212) PMC_CL(32, 12)
-    else if (ccfg == 3210) PMC_CL(32, 10)
-    else if (ccfg == 3208) PMC_CL(32, 8)
-    else if (ccfg == 6408) PMC_CL(64, 8)
-    else if (ccfg == 6410) PMC_CL(64, 10)
-    else if (ccfg == 6406) PMC_CL(64, 6)
-    else if (ccfg == 6404) PMC_CL(64, 4)
-    else if (ccfg == 12804) PMC_CL(128, 4)
-    else if (ccfg == 12805) PMC_CL(128, 5)
-    else if (ccfg == 25602) PMC_CL(256, 2)
-    else
-#else
-    (void)ccfg;
-#endif
     switch (h->cta_threads > 256 ? 256 : h->cta_threads) {
       case 32:  // very short chains fit 16 per SM in shared memory: worth the 128-register build (+9 % at n=25)
         // registers beat occupancy for the one-warp teams (profiles/r02b_tune_k1.txt): 10 chains per SM at 204 registers are

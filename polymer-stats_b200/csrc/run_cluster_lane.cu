@@ -45,8 +45,6 @@ int launch_run_cluster_lane(pmc_handle* h, const RunArgs& a) {
       if (ising) k_run_lane_cluster<TB, 4, true, true><<<nb, TB, 0, h->stream>>>(a);
       else k_run_lane_cluster<TB, 4, false, true><<<nb, TB, 0, h->stream>>>(a);
     } else {
-      // PMC_LANE_CLUSTER_CFG = threads*100 + minblocks selects a tuning variant (experiments only)
-      const int lcfg = env_int("PMC_LANE_CLUSTER_CFG", 0);
 #define PMC_LC(TT, MB)                                                                                         \
   {                                                                                                            \
     PMC_PICK("k_run_lane_cluster<" #TT "," #MB ">");                                                           \
@@ -54,17 +52,6 @@ int launch_run_cluster_lane(pmc_handle* h, const RunArgs& a) {
     if (ising) k_run_lane_cluster<TT, MB, true, false><<<nbb, TT, 0, h->stream>>>(a);                          \
     else k_run_lane_cluster<TT, MB, false, false><<<nbb, TT, 0, h->stream>>>(a);                               \
   }
-#ifdef PMC_TUNING_VARIANTS
-      if (lcfg == 6403) PMC_LC(64, 3)
-      else if (lcfg == 6404) PMC_LC(64, 4)
-      else if (lcfg == 6408) PMC_LC(64, 8)
-      else if (lcfg == 3208) PMC_LC(32, 8)
-      else if (lcfg == 3212) PMC_LC(32, 12)
-      else if (lcfg == 3216) PMC_LC(32, 16)
-      else
-#else
-      (void)lcfg;
-#endif
       if (packing_chains(h) >= 32768) PMC_LC(64, 8)  // many chains: occupancy beats the spills of the 128-register build
       else PMC_LC(64, 4)
 #undef PMC_LC

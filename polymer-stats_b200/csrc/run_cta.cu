@@ -1,4 +1,5 @@
-// run_cta.cu — launches of the single-monomer-trial CTA-per-chain run kernels (cta_kernels.cuh): k_run_cta_win, k_run_cta, k_run_cta_ws.
+// run_cta.cu — launches of the single-monomer-trial CTA-per-chain run kernels (cta_kernels.cuh): k_run_cta_win,
+// k_run_cta_win_spec; chains whose windowed kernel does not fit one CTA go to k_run_cta_pair (run_pair.cu).
 #include "handle.h"
 
 namespace {
@@ -8,35 +9,15 @@ int fail(int code, const std::string& msg) { return pmc_fail(code, msg); }
 // FP32 rectangle (pmc_set_pair_precision): served by the windowed one-CTA kernel; every other launch stays FP64.
 bool use_f32_rect(const pmc_handle* h) {
   if (h->pair_precision != 1 || h->energy_type != PMC_ENERGY_INTERACTING || h->cluster_mode) return false;
-  if (use_pair_kernel(h) || !env_int("PMC_RUN_WIN", h->use_win) || env_int("PMC_RUN_CFG", 0)) return false;
+  if (use_pair_kernel(h)) return false;
   if (h->cta_threads != 64 && h->cta_threads != 128 && h->cta_threads != 256 && h->cta_threads != 512) return false;
   return cta_smem_bytes_win_f32(h->n) <= (size_t)kSmemMax;
 }
 
-int launch_delta_cta_f32(pmc_handle* h, const DeltaArgs& a) {
-  const size_t smem = ((cta_smem_bytes(h->n) + 15) & ~(size_t)15) + f32_smem_bytes(h->n);
-#define PMC_CASE(TT)                                            \
-  case TT: {                                                    \
-    int rc = set_smem(k_delta_cta_f32<TT>, smem);               \
-    if (rc) return rc;                                          \
-    k_delta_cta_f32<TT><<<1, TT, smem, h->stream>>>(a);         \
-    ++h->launches;                                              \
-    break;                                                      \
-  }
-  switch (h->cta_threads) {
-    PMC_CASE(64) PMC_CASE(128) PMC_CASE(256) PMC_CASE(512)
-    default: return fail(PMC_ERR_INVALID, "bad cta_threads");
-  }
-#undef PMC_CASE
-  PMC_CU(cudaGetLastError());
-  return PMC_OK;
-}
-
 int launch_run_cta(pmc_handle* h, const RunArgs& a) {
-  if (h->spec_teams > 0 && h->pair_precision == 0 && !env_int("PMC_RUN_CFG", 0) && env_int("PMC_RUN_WIN", h->use_win) &&
-      !env_int("PMC_RUN_WS", h->ws_cfg) && env_int("PMC_RUN_PAIR", 1) != 2) {
+  const int nb = (int)h->nchains;
+  if (h->spec_teams > 0 && h->pair_precision == 0 && env_int("PMC_RUN_PAIR", 1) != 2) {
     const size_t smem = cta_smem_bytes_spec(h->n, h->spec_teams);
-    const int nb = (int)h->nchains;
 #define PMC_LAUNCH_SPEC(GG, MB)                                                  \
   {                                                                              \
     PMC_PICK("k_run_cta_win_spec<" #GG "," #MB ">");                             \
@@ -53,129 +34,32 @@ int launch_run_cta(pmc_handle* h, const RunArgs& a) {
 #undef PMC_LAUNCH_SPEC
   }
   if (use_pair_kernel(h)) return launch_run_pair(h, a);
-  if (use_f32_rect(h)) {
-    const size_t smem32 = cta_smem_bytes_win_f32(h->n);
-    const int nb = (int)h->nchains;
-#define PMC_LAUNCH_F32(TT, MB)                                                   \
-  {                                                                              \
-    PMC_PICK("k_run_cta_win<" #TT "," #MB ",2,fp32>");                           \
-    int rc = set_smem(k_run_cta_win<TT, MB, 2, 1>, smem32);                      \
-    if (rc) return rc;                                                           \
-    k_run_cta_win<TT, MB, 2, 1><<<nb, TT, smem32, h->stream>>>(a);               \
-    ++h->launches;                                                               \
-    PMC_CU(cudaGetLastError());                                                  \
-    return PMC_OK;                                                               \
-  }
-    switch (h->cta_threads) {
-      case 64: PMC_LAUNCH_F32(64, 8)
-      case 128: PMC_LAUNCH_F32(128, 4)
-      case 256: PMC_LAUNCH_F32(256, 2)
-      default: PMC_LAUNCH_F32(512, 1)
-    }
-#undef PMC_LAUNCH_F32
-  }
-  const size_t smem = cta_smem_bytes(h->n);
-  const int nblocks = (int)h->nchains;
-  // PMC_RUN_CFG = threads*100 + minblocks*10 + unroll selects a tuning variant (experiments only)
-  const int cfg = env_int("PMC_RUN_CFG", 0);
-  // PMC_RUN_WS = workers*10 + minblocks selects the warp-specialised kernel (control warp + workers)
-  const int ws = env_int("PMC_RUN_WS", h->ws_cfg);
-#define PMC_LAUNCH_WS(WK, MB)                                               \
+  // windowed kernel (32 proposals built at once by warp 0), FP64 or FP32 rectangle
+  const bool f32 = use_f32_rect(h);
+  const size_t smem = f32 ? cta_smem_bytes_win_f32(h->n) : cta_smem_bytes_win(h->n);
+  if (smem > (size_t)kSmemMax) return fail(PMC_ERR_UNSUPPORTED, "chain too long for the one-CTA run kernel");
+#define PMC_LAUNCH_WIN(TT, MB, PREC, NAME)                                  \
   {                                                                         \
-    PMC_PICK("k_run_cta_ws<" #WK "," #MB ",2>");                            \
-    int rc = set_smem(k_run_cta_ws<WK, MB, 2>, smem);                       \
+    PMC_PICK(NAME);                                                         \
+    int rc = set_smem(k_run_cta_win<TT, MB, 2, PREC>, smem);                \
     if (rc) return rc;                                                      \
-    k_run_cta_ws<WK, MB, 2><<<nblocks, (WK + 1) * 32, smem, h->stream>>>(a); \
-    ++h->launches;                                                          \
-    PMC_CU(cudaGetLastError());                                             \
-    return PMC_OK;                                                          \
+    k_run_cta_win<TT, MB, 2, PREC><<<nb, TT, smem, h->stream>>>(a);         \
+    break;                                                                  \
   }
-#ifdef PMC_TUNING_VARIANTS  // measured negative result (profiles/r01c_tune_warp_specialised.txt): tuning builds only
-  if (cfg == 0) {
-    if (ws == 34) PMC_LAUNCH_WS(3, 4)
-    if (ws == 43) PMC_LAUNCH_WS(4, 3)
-    if (ws == 72) PMC_LAUNCH_WS(7, 2)
-    if (ws == 52) PMC_LAUNCH_WS(5, 2)
-    if (ws == 71) PMC_LAUNCH_WS(7, 1)
-    if (ws == 151) PMC_LAUNCH_WS(15, 1)
-    if (ws == 14) PMC_LAUNCH_WS(1, 4)
-    if (ws == 18) PMC_LAUNCH_WS(1, 8)
-  }
-#else
-  (void)ws;
-#endif
-#undef PMC_LAUNCH_WS
-  // windowed kernel (32 proposals built at once by warp 0): needs 6.7 KB more shared memory
-  const int use_win = env_int("PMC_RUN_WIN", h->use_win);
-  const size_t smem_win = cta_smem_bytes_win(h->n);
-#define PMC_LAUNCH_WIN(TT, MB)                                              \
-  {                                                                         \
-    PMC_PICK("k_run_cta_win<" #TT "," #MB ",2>");                           \
-    int rc = set_smem(k_run_cta_win<TT, MB, 2>, smem_win);                  \
-    if (rc) return rc;                                                      \
-    k_run_cta_win<TT, MB, 2><<<nblocks, TT, smem_win, h->stream>>>(a);      \
-    ++h->launches;                                                          \
-    PMC_CU(cudaGetLastError());                                             \
-    return PMC_OK;                                                          \
-  }
-  if (cfg == 0 && use_win && smem_win <= (size_t)kSmemMax) {
-#ifdef PMC_TUNING_VARIANTS
-    if (use_win == 648) PMC_LAUNCH_WIN(64, 8)
-    if (use_win == 1286) PMC_LAUNCH_WIN(128, 6)
-    if (use_win == 1283) PMC_LAUNCH_WIN(128, 3)
-    if (use_win == 1282) PMC_LAUNCH_WIN(128, 2)
-    if (use_win == 1285) PMC_LAUNCH_WIN(128, 5)
-    if (use_win == 2562) PMC_LAUNCH_WIN(256, 2)
-    if (use_win == 643) PMC_LAUNCH_WIN(64, 10)
-    if (use_win == 2563) PMC_LAUNCH_WIN(256, 3)
-#endif
-    switch (h->cta_threads) {
-      case 64: PMC_LAUNCH_WIN(64, 8)
-      case 128: PMC_LAUNCH_WIN(128, 4)
-      case 256: PMC_LAUNCH_WIN(256, 2)
-      case 512: PMC_LAUNCH_WIN(512, 1)
-      default: break;
-    }
-  }
-#undef PMC_LAUNCH_WIN
-#define PMC_LAUNCH(TT, MB, UR)                                              \
-  {                                                                         \
-    PMC_PICK("k_run_cta<" #TT "," #MB "," #UR ">");                         \
-    int rc = set_smem(k_run_cta<TT, MB, UR>, smem);                         \
-    if (rc) return rc;                                                      \
-    k_run_cta<TT, MB, UR><<<nblocks, TT, smem, h->stream>>>(a);             \
-    ++h->launches;                                                          \
-  }
-#ifdef PMC_TUNING_VARIANTS
-  if (cfg == 12842) PMC_LAUNCH(128, 4, 2)
-  else if (cfg == 12841) PMC_LAUNCH(128, 4, 1)
-  else if (cfg == 25621) PMC_LAUNCH(256, 2, 1)
-  else if (cfg == 51211) PMC_LAUNCH(512, 1, 1)
-  else if (cfg == 12862) PMC_LAUNCH(128, 6, 2)
-  else if (cfg == 12861) PMC_LAUNCH(128, 6, 1)
-  else if (cfg == 12882) PMC_LAUNCH(128, 8, 2)
-  else if (cfg == 12881) PMC_LAUNCH(128, 8, 1)
-  else if (cfg == 25632) PMC_LAUNCH(256, 3, 2)
-  else if (cfg == 25631) PMC_LAUNCH(256, 3, 1)
-  else if (cfg == 25642) PMC_LAUNCH(256, 4, 2)
-  else if (cfg == 25641) PMC_LAUNCH(256, 4, 1)
-  else if (cfg == 25622) PMC_LAUNCH(256, 2, 2)
-  else if (cfg == 51212) PMC_LAUNCH(512, 1, 2)
-  else if (cfg == 51222) PMC_LAUNCH(512, 2, 2)
-  else if (cfg == 102412) PMC_LAUNCH(1024, 1, 2)
-  else if (cfg == 102411) PMC_LAUNCH(1024, 1, 1)
-  else
-#endif
+#define PMC_LAUNCH_WIN2(TT, MB)                                                      \
+  case TT:                                                                           \
+    if (f32) PMC_LAUNCH_WIN(TT, MB, 1, "k_run_cta_win<" #TT "," #MB ",2,fp32>")     \
+    else PMC_LAUNCH_WIN(TT, MB, 0, "k_run_cta_win<" #TT "," #MB ",2>")
   switch (h->cta_threads) {
-    case 64: PMC_LAUNCH(64, 8, 2) break;
-    case 128: PMC_LAUNCH(128, 4, 2) break;
-    case 256: PMC_LAUNCH(256, 2, 2) break;
-    case 512: PMC_LAUNCH(512, 1, 2) break;
-    case 1024: PMC_LAUNCH(1024, 1, 2) break;
+    PMC_LAUNCH_WIN2(64, 8)
+    PMC_LAUNCH_WIN2(128, 4)
+    PMC_LAUNCH_WIN2(256, 2)
+    PMC_LAUNCH_WIN2(512, 1)
     default: return fail(PMC_ERR_INVALID, "bad cta_threads");
   }
-#undef PMC_LAUNCH
+#undef PMC_LAUNCH_WIN2
+#undef PMC_LAUNCH_WIN
+  ++h->launches;
   PMC_CU(cudaGetLastError());
   return PMC_OK;
 }
-

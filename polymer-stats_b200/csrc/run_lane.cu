@@ -11,10 +11,7 @@ int launch_run_lane(pmc_handle* h, const RunArgs& a) {
     const int mode = env_int("PMC_LANE_MODE", 0);  // 1 = lane, 2 = warp, 0 = by chain count
     const long long below = h->warp_mode_below > 0 ? h->warp_mode_below : (h->energy_type == PMC_ENERGY_ISING ? 65536 : 120000);
     const bool use_warp = mode == 2 || (mode == 0 && packing_chains(h) < below);
-    // PMC_LANE_CFG = minblocks*10 + compensated selects a tuning variant (experiments only)
-    const int lcfg = env_int("PMC_LANE_CFG", -1);
-    const bool comp = lcfg >= 0 ? (lcfg % 10) != 0 : h->compensated != 0;
-    const int mb = lcfg >= 0 ? lcfg / 10 : 0;
+    const bool comp = h->compensated != 0;
     if (use_warp) {
       const unsigned nb = (unsigned)((h->nchains + 3) / 4);
       const bool ising = h->energy_type == PMC_ENERGY_ISING;
@@ -30,16 +27,8 @@ int launch_run_lane(pmc_handle* h, const RunArgs& a) {
       k_run_warp<IS, MB, CP><<<nb, 128, 0, h->stream>>>(a);                         \
     }                                                                               \
   }
-#define PMC_WSEL(MB)                                                        \
-  {                                                                         \
-    if (ising) { if (comp) PMC_W(1, MB, true) else PMC_W(1, MB, false) }  \
-    else { if (comp) PMC_W(0, MB, true) else PMC_W(0, MB, false) }        \
-  }
-#ifdef PMC_TUNING_VARIANTS
-      if (mb == 3) PMC_WSEL(3) else if (mb == 2) PMC_WSEL(2) else if (mb == 5) PMC_WSEL(5) else if (mb == 6) PMC_WSEL(6) else
-#endif
-      PMC_WSEL(4)
-#undef PMC_WSEL
+      if (ising) { if (comp) PMC_W(1, 4, true) else PMC_W(1, 4, false) }
+      else { if (comp) PMC_W(0, 4, true) else PMC_W(0, 4, false) }
 #undef PMC_W
     } else {
       constexpr int TB = 64;
@@ -49,11 +38,7 @@ int launch_run_lane(pmc_handle* h, const RunArgs& a) {
     PMC_PICK("k_run_lane<64," #MB "," #CP ">");            \
     k_run_lane<TB, MB, CP><<<nb, TB, 0, h->stream>>>(a);  \
   }
-      if (mb == 6 || (mb == 0 && !comp)) { if (comp) PMC_L(6, true) else PMC_L(6, false) }
-#ifdef PMC_TUNING_VARIANTS
-      else if (mb == 8) { if (comp) PMC_L(8, true) else PMC_L(8, false) }
-#endif
-      else { if (comp) PMC_L(4, true) else PMC_L(4, false) }
+      if (comp) PMC_L(4, true) else PMC_L(6, false)
 #undef PMC_L
     }
     ++h->launches;

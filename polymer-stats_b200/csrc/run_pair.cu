@@ -15,11 +15,14 @@ int fail(int code, const std::string& msg) { return pmc_fail(code, msg); }
 //     elsewhere the windowed one-CTA kernel is ahead (its proposals are off the critical path);
 //   * shorter chains: never (the cluster barrier per trial is no longer small against the trial).
 // The ensemble size is the hint's (pmc_set_ensemble_hint), so a shard decides like the whole sweep.
-// PMC_RUN_PAIR=0 switches pairs off, PMC_RUN_PAIR=2 forces them for any chain length (tests and experiments).
+// Chains whose windowed one-CTA kernel does not fit shared memory (n ≳ 3900) always take pairs.  Otherwise PMC_RUN_PAIR=0
+// switches pairs off and PMC_RUN_PAIR=2 forces them for any chain length (tests and experiments).
 bool use_pair_kernel(const pmc_handle* h) {
-  const int mode = env_int("PMC_RUN_PAIR", 1);
-  if (mode == 0 || h->energy_type != PMC_ENERGY_INTERACTING || h->cluster_mode) return false;
+  if (h->energy_type != PMC_ENERGY_INTERACTING || h->cluster_mode) return false;
   if (h->cta_threads != 128 && h->cta_threads != 256 && h->cta_threads != 512) return false;
+  if (cta_smem_bytes_win(h->n) > (size_t)kSmemMax) return true;
+  const int mode = env_int("PMC_RUN_PAIR", 1);
+  if (mode == 0) return false;
   if (mode == 2) return true;
   if (cta_smem_bytes(h->n) > (size_t)kSmemMax / 2) return true;
   if (h->n > 768) return true;

@@ -7,7 +7,7 @@ distance of a pair from the rotated monomer and with |D|, so the states here put
 (hairpins), make |D| large, stretch a chain to n = 700 and run the n = 4096 shape of the two-SM kernel.
 The bound is 1e-13 of Σ|changed terms|, ten times tighter than the oracle gate of the other tests, except at n = 4096:
 there the staged positions (a block scan on the device, a sequential sum in the reference) already differ enough that
-r' formed and squared (-DPMC_RECT_Q2=0) measures 2.2e-13 on this state, as the projections do.
+r' formed and squared (the form before the projections) measures 2.2e-13 on this state, as the projections do.
 """
 import math
 

@@ -1,5 +1,5 @@
 // Microbenchmark of the rectangle loop (rect_sum, cta_kernels.cuh) alone, and accuracy of rsqrt_fast under
-// -DPMC_RSQRT_VARIANT=0|1, and of the two forms of |r'|² under -DPMC_RECT_Q2=0|1 (developer tool, not product code;
+// -DPMC_RSQRT_VARIANT=0|1, and of the two forms of |r'|² under -DRECT_Q2=0|1 (developer tool, not product code;
 // the Q2 form keeps the broadcast side at most n/2 long: both builds time the trials whose tails are that short).
 // Build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -DPMC_RSQRT_VARIANT=1 -o tools/rect_bench_v1 tools/rect_bench.cu
 #include <cstdio>
@@ -7,6 +7,9 @@
 #include <cuda_runtime.h>
 #include "../polymer-stats_b200/csrc/cta_kernels.cuh"
 using namespace pmc;
+#ifndef RECT_Q2
+#define RECT_Q2 1   // 0: r' formed and squared (the form before the projections)
+#endif
 
 template <int T, int MINB>
 __global__ void __launch_bounds__(T, MINB) k_rect(double* out, int n, int reps) {
@@ -20,7 +23,7 @@ __global__ void __launch_bounds__(T, MINB) k_rect(double* out, int n, int reps) 
   }
   __syncthreads();
   double acc = 0.0;
-  using TEAM = Team<T / 32, 0>;
+  using TEAM = Team<T / 32>;
   for (int r = 0; r < reps; ++r) {
     const int idx = (int)((r * 2654435761u + blockIdx.x * 40503u) % (unsigned)n);
     const double Dx = 0.1 + 1e-3 * (r & 7), Dy = -0.2, Dz = 0.15;
@@ -29,9 +32,9 @@ __global__ void __launch_bounds__(T, MINB) k_rect(double* out, int n, int reps) 
       // heads on the lanes: the tails' {eB, 2p_B} take 2·Tl doubles of S.E in the Q2 form
       if (2 * Tl > n) continue;
       const double px = S.sx[idx], py = S.sy[idx], pz = S.sz[idx];
-      for (int k = threadIdx.x; k < Tl; k += T) rect_prepass_item<PMC_RECT_Q2>(S, idx + 1, k, px, py, pz, Dx, Dy, Dz);
+      for (int k = threadIdx.x; k < Tl; k += T) rect_prepass_item<RECT_Q2>(S, idx + 1, k, px, py, pz, Dx, Dy, Dz);
       __syncthreads();
-      acc += rect_sum<TEAM, 2, false, false, PMC_RECT_Q2>(S, 0, H, idx + 1, Tl, Dx, Dy, Dz, 0.0, idx);
+      acc += rect_sum<TEAM, 2, false, false, RECT_Q2>(S, 0, H, idx + 1, Tl, Dx, Dy, Dz, 0.0, idx);
       __syncthreads();
     }
   }
@@ -79,7 +82,7 @@ int main() {
   cudaMemcpy(h, d, sizeof(double) * blocks * T, cudaMemcpyDeviceToHost);
   double cs = 0; for (int i = 0; i < blocks * T; ++i) cs += h[i];
   printf("q2 %d variant %d: rect loop %.3f ms, %.3e pairs -> %.2f G pairs/s = %.2f TFLOP/s algorithmic (68 flop/pair), checksum %.15e\n",
-         PMC_RECT_Q2, PMC_RSQRT_VARIANT, best, pairs, pairs / best / 1e6, pairs * 68 / best / 1e9, cs);
+         RECT_Q2, PMC_RSQRT_VARIANT, best, pairs, pairs / best / 1e6, pairs * 68 / best / 1e9, cs);
   const int TT = 256 * 148;
   double* e; cudaMalloc(&e, TT * sizeof(double));
   k_acc<<<148, 256>>>(e, 200000000);

@@ -20,11 +20,6 @@ if which in ("all", "plain"):
         ens.run(40, 10)
         print(ens.kernel_name(), ens.averages()[1][:2])
     del os.environ["PMC_LANE_MODE"]
-    os.environ["PMC_RUN_WIN"] = "0"                         # the classic (window-less) CTA kernel
-    with pm.Ensemble(pm.make_case(n=70, E0=1.0, Fz=0.5, energy_type="interacting"), replicas=3, seed=2) as ens:
-        ens.run(30, 10)
-        print(ens.kernel_name(), ens.averages()[1])
-    del os.environ["PMC_RUN_WIN"]
 if which in ("all", "pair"):
     os.environ["PMC_RUN_PAIR"] = "2"                        # two SMs per chain: cluster barrier + distributed shared memory
     for n, R in ((70, 3), (300, 5)):

@@ -38,28 +38,25 @@ for name, kw, R, steps, cl in CASES:
     ens.close()
 
 # Cross-kernel decision equality over long runs (compute-sanitizer is closed on this pool: a race in a barrier protocol
-# would show up as a different accept/reject sequence): the same ensemble through the windowed one-CTA kernel, the classic
-# one-CTA kernel and the CTA-pair kernel (cluster barrier + distributed shared memory) must count the same acceptances per
-# chain — the reduction orders differ, so only a decision within rounding of its threshold could legitimately differ.
+# would show up as a different accept/reject sequence): the same ensemble through the windowed one-CTA kernel and the
+# CTA-pair kernel (cluster barrier + distributed shared memory) must count the same acceptances per chain — the reduction orders differ, so only a decision within rounding of its threshold could legitimately differ.
 import os
 for n, R, steps in ((512, 444, 20000), (1024, 300, 6000), (200, 1000, 40000)):
     counts = {}
-    for tag, env in (("windowed", dict(PMC_RUN_PAIR="0", PMC_RUN_WIN="1")), ("classic", dict(PMC_RUN_PAIR="0", PMC_RUN_WIN="0")),
-                     ("pair", dict(PMC_RUN_PAIR="2", PMC_RUN_WIN="1"))):
+    for tag, env in (("windowed", dict(PMC_RUN_PAIR="0")), ("pair", dict(PMC_RUN_PAIR="2"))):
         os.environ.update(env)
         with pm.Ensemble(pm.make_case(n=n, E0=1.0, Fz=0.5, energy_type="interacting"), replicas=R, seed=4242) as ens:
             name = ens.kernel_name()
             t0 = time.time()
             ens.run(steps, 0, fetch_rows=False)
             counts[tag] = (ens.diagnostics()[:, 4].copy(), name, time.time() - t0)
-    same = all(np.array_equal(counts["windowed"][0], counts[k][0]) for k in ("classic", "pair"))
-    diff = max(int((counts["windowed"][0] != counts[k][0]).sum()) for k in ("classic", "pair"))
-    print("decision equality n=%d, %d chains x %d trials: %s (%s %.1f s, %s %.1f s, %s %.1f s); chains with a different acceptance "
-          "count: %d" % (n, R, steps, "ok " if same else "DIFF", counts["windowed"][1], counts["windowed"][2], counts["classic"][1],
-                         counts["classic"][2], counts["pair"][1], counts["pair"][2], diff), flush=True)
+    same = np.array_equal(counts["windowed"][0], counts["pair"][0])
+    diff = int((counts["windowed"][0] != counts["pair"][0]).sum())
+    print("decision equality n=%d, %d chains x %d trials: %s (%s %.1f s, %s %.1f s); chains with a different acceptance "
+          "count: %d" % (n, R, steps, "ok " if same else "DIFF", counts["windowed"][1], counts["windowed"][2], counts["pair"][1],
+                         counts["pair"][2], diff), flush=True)
     bad += not same
-for k in ("PMC_RUN_PAIR", "PMC_RUN_WIN"):
-    os.environ.pop(k, None)
+os.environ.pop("PMC_RUN_PAIR", None)
 
 # Chain per lane against chain per warp (32 speculative trials per window, resolved in order): both are the reference's
 # sequential Markov chain on the same Philox stream, so the final STATES must be equal bit for bit and the acceptance
