@@ -1,5 +1,5 @@
 // handle.h — what the translation units of libpolymc_b200.so share: the handle behind the C ABI, error
-// plumbing, and the launch helpers each kernel family's TU exports (one TU per family so that `make -j`
+// plumbing, and the launchers each kernel family's TU exports (one TU per family so that `make -j`
 // compiles them in parallel).
 #pragma once
 
@@ -14,10 +14,13 @@
 #include <algorithm>
 #include <chrono>
 #include <mutex>
+#include <type_traits>
 #include <unordered_map>
+#include <utility>
 #include <vector>
 
 #include "cluster_kernels.cuh"
+#include "plan.h"
 
 using namespace pmc;
 
@@ -48,13 +51,6 @@ inline int env_int(const char* name, int dflt) {
   return (v && *v) ? std::atoi(v) : dflt;
 }
 
-// Every launch helper records the kernel it picks; with dry_run set it stops there (pmc_kernel_name).
-#define PMC_PICK(name_literal)        \
-  do {                                \
-    h->kernel_name = name_literal;    \
-    if (h->dry_run) return PMC_OK;    \
-  } while (0)
-
 struct pmc_handle {
   int device = 0;
   int64_t nchains = 0;
@@ -77,16 +73,9 @@ struct pmc_handle {
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   float last_ms = 0.f;
   int64_t launches = 0;
-  int cta_threads = 256;      // block size of the CTA-per-chain kernels
   int sm_count = 148;
   int64_t shape_chains = 0;   // ensemble size the launch shape is chosen for (0 = nchains), pmc_set_ensemble_hint
-  // O(1)-ΔU chains of the plain driver: one chain per warp below this many chains, else one per lane.  Measured
-  // crossover (profiles/r02c_tune_lane_vs_warp.txt): non-interacting 14.8 vs 12.6 G updates/s at 65 536 chains and 14.5 vs
-  // 17.5 at 262 144; Ising level at 65 536.  Set from the energy type in launch_run_lane.
-  long long warp_mode_below = 0;
-  long long warp_cluster_below = 11000;  // composite trials: chain per warp below this many chains, else per lane
   int compensated = 0;        // Neumaier-compensated accumulators in the lane/warp kernels (CTA kernels: always)
-  int spec_teams = 0;         // > 0: small ensemble of short interacting chains — one-warp teams on different trials (k_run_cta_win_spec)
   int pair_precision = 0;     // 0: FP64 everywhere; 1: the rectangle of single-monomer trials in FP32 where a kernel exists (cta_f32.cuh)
   std::vector<ChainDyn> host_dyn;
   bool dyn_fresh = false, dynx_fresh = false;   // the host copies equal the device's (no launch since they were fetched)
@@ -105,8 +94,6 @@ struct pmc_handle {
   unsigned long long* pair_work = nullptr;
   int* pair_order = nullptr;
   int* pair_next = nullptr;
-  const char* kernel_name = "";  // the MCMC kernel the last (dry or real) launch decision picked, pmc_kernel_name
-  int dry_run = 0;               // launch helpers only record their decision
   // replica exchange (exchange.cuh), set by pmc_set_ladders
   std::vector<int32_t> ladder;          // the rungs as given, ladders separated by -1; empty: no ladders
   pmc::ExPair* ex_pairs = nullptr;      // candidate pairs, those of even rounds first
@@ -134,12 +121,33 @@ int set_smem(K kernel, size_t bytes) {
   return PMC_OK;
 }
 
-// Ensemble size the chain-per-lane / chain-per-warp packing is chosen for: like the block size it follows the
-// hint, so a shard of a sweep runs the kernel the whole ensemble would (the packings sum the per-trial averager
-// contributions in different orders; same kernel ⇒ results bit-identical however the sweep is sharded).
-inline int64_t packing_chains(const pmc_handle* h) { return h->shape_chains > 0 ? h->shape_chains : h->nchains; }
+// One launch on the handle's stream: the dynamic shared memory limit (when the kernel takes any), the launch, the count.
+template <typename K, typename... Args>
+int launch(pmc_handle* h, K kernel, unsigned grid, int block, size_t smem, const Args&... args) {
+  if (smem > (size_t)kSmemMax) return pmc_fail(PMC_ERR_UNSUPPORTED, "chain too long for this kernel's shared memory");
+  if (smem) {
+    int rc = set_smem(kernel, smem);
+    if (rc) return rc;
+  }
+  kernel<<<grid, block, smem, h->stream>>>(args...);
+  ++h->launches;
+  PMC_CU(cudaGetLastError());
+  return PMC_OK;
+}
 
-// Block size of the composite-trial CTA kernels.
+// f(std::integral_constant<int, V>()) for the V of the list that equals v: maps a planned value onto an instantiation.
+template <int... V, class F>
+int with(int v, F&& f) {
+  int rc = PMC_OK;
+  const bool hit = ((v == V && ((rc = f(std::integral_constant<int, V>())), true)) || ...);
+  return hit ? rc : pmc_fail(PMC_ERR_INVALID, "no kernel instantiated for this launch shape");
+}
+template <int LO, class F, int... I>
+int with_offset(int v, F&& f, std::integer_sequence<int, I...>) { return with<(LO + I)...>(v, f); }
+template <int LO, int HI, class F>   // v in LO … HI
+int with_range(int v, F&& f) { return with_offset<LO>(v, f, std::make_integer_sequence<int, HI - LO + 1>()); }
+
+// Block size of the composite-trial CTA kernels (and of their helper kernel k_delta_segment_cta).
 // Short chains are latency bound (one serial proposal/cluster/decision chain per trial), so one warp per
 // chain and many chains per SM; measured crossovers in profiles/r01e_tune_cluster.txt.  Chains whose shared-memory
 // footprint (18 n doubles) leaves room for a single CTA per SM get 256 threads instead of 128: at n = 800 … 1000 one
@@ -149,23 +157,13 @@ inline int pick_cluster_threads(int n) {
   if (n <= 256) return 64;
   return 2 * (pmc::cluster_smem_bytes(n, 128) + 1024) > (size_t)kSmemMax ? 256 : 128;
 }
-// CTAs of the 128-thread composite-trial kernel that fit one SM's shared memory (2 … 4): the launch bound follows it,
-// because a bound the shared memory cannot honour only takes registers away (n = 400: 3 per SM at 168 registers are
-// +8 % over a bound of 4 at 128; n = 640: 2 per SM +20 %).
-inline int cluster_fit128(int n) {
-  const int fit = (int)((size_t)kSmemMax / (pmc::cluster_smem_bytes(n, 128) + 1024));
-  return fit >= 4 ? 4 : fit >= 3 ? 3 : 2;
-}
-
-// ---- launch helpers, one translation unit per kernel family -------------------------------------------------
-int launch_run_cta(pmc_handle* h, const pmc::RunArgs& a);                    // run_cta.cu
-bool use_f32_rect(const pmc_handle* h);
-int launch_run_pair(pmc_handle* h, const pmc::RunArgs& a);                   // run_pair.cu
-bool use_pair_kernel(const pmc_handle* h);                                   // run_pair.cu
-int launch_run_lane(pmc_handle* h, const pmc::RunArgs& a);                   // run_lane.cu
-int launch_run_cluster_cta(pmc_handle* h, const pmc::RunArgs& a);            // run_cluster_cta.cu
-int launch_delta_segment_cta(pmc_handle* h, const pmc::SegDeltaArgs& a);     // run_cluster_cta.cu
-int launch_run_cluster_lane(pmc_handle* h, const pmc::RunArgs& a);           // run_cluster_lane.cu
+// ---- launchers of the run kernels, one translation unit per kernel family: each maps a plan onto instantiations ----
+int launch_run_cta(pmc_handle* h, const RunPlan& p, const pmc::RunArgs& a);           // run_cta.cu: cta_win, cta_win_spec
+int launch_run_pair(pmc_handle* h, const RunPlan& p, const pmc::RunArgs& a);          // run_pair.cu: cta_pair
+int launch_run_lane(pmc_handle* h, const RunPlan& p, const pmc::RunArgs& a);          // run_lane.cu: lane, warp
+int launch_run_cluster_cta(pmc_handle* h, const RunPlan& p, const pmc::RunArgs& a);   // run_cluster_cta.cu
+int launch_delta_segment_cta(pmc_handle* h, const pmc::SegDeltaArgs& a);              // run_cluster_cta.cu
+int launch_run_cluster_lane(pmc_handle* h, const RunPlan& p, const pmc::RunArgs& a);  // run_cluster_lane.cu
 int launch_exchange(pmc_handle* h, const pmc::ExchangeArgs& a, int64_t npairs);   // exchange.cu
 int launch_place_rows(pmc_handle* h, double* dst, const double* src, int64_t rows, int64_t rows_total, int64_t row0,
                       int cols);                                             // exchange.cu

@@ -131,32 +131,11 @@ int check_chain(const pmc_handle* h, int64_t chain) {
   return PMC_OK;
 }
 
-// Block size for the CTA-per-chain kernels: enough threads to cover the mean rectangle
-// (n²/6 pairs) without leaving most lanes idle on short chains.
-int pick_cta_threads(int n) { return n <= 128 ? 64 : n <= 1024 ? 128 : n <= 1536 ? 256 : 512; }
-
-// Launch pick(std::integral_constant<int, T>) for the block size T = h->cta_threads chosen at create time (T ≥ MIN_T).
-template <int MIN_T = 32, class Pick, class Args>
+// Launch pick(std::integral_constant<int, T>) at the planned block size T of the CTA helper kernels.
+template <class Pick, class Args>
 static int launch_cta_kernel(pmc_handle* h, Pick pick, int nblocks, size_t smem, const Args& a) {
-  auto go = [&](auto t) -> int {
-    const auto kernel = pick(t);
-    int rc = set_smem(kernel, smem);
-    if (rc) return rc;
-    kernel<<<nblocks, decltype(t)::value, smem, h->stream>>>(a);
-    ++h->launches;
-    PMC_CU(cudaGetLastError());
-    return PMC_OK;
-  };
-  switch (h->cta_threads) {
-    case 32:
-      if constexpr (MIN_T <= 32) return go(std::integral_constant<int, 32>());
-      break;
-    case 64: return go(std::integral_constant<int, 64>());
-    case 128: return go(std::integral_constant<int, 128>());
-    case 256: return go(std::integral_constant<int, 256>());
-    case 512: return go(std::integral_constant<int, 512>());
-  }
-  return fail(PMC_ERR_INVALID, "bad cta_threads");
+  return with<32, 64, 128, 256, 512>(plan_run(h).cta_threads,
+                                     [&](auto T) { return launch(h, pick(T), nblocks, T, smem, a); });
 }
 
 int launch_energy(pmc_handle* h, const EnergyArgs& a, int nblocks) {
@@ -165,10 +144,11 @@ int launch_energy(pmc_handle* h, const EnergyArgs& a, int nblocks) {
 
 // ΔU of one scripted move with the rectangle precision the run kernel of this handle uses.
 int launch_delta_cta(pmc_handle* h, const DeltaArgs& a) {
-  if (use_f32_rect(h))
-    return launch_cta_kernel<64>(h, [](auto t) { return k_delta_cta<decltype(t)::value, 1>; }, 1,
-                                 ((cta_smem_bytes(h->n) + 15) & ~(size_t)15) + f32_smem_bytes(h->n), a);
-  return launch_cta_kernel(h, [](auto t) { return k_delta_cta<decltype(t)::value>; }, 1, cta_smem_bytes(h->n), a);
+  const RunPlan p = plan_run(h);
+  if (!p.f32) return launch_cta_kernel(h, [](auto t) { return k_delta_cta<decltype(t)::value>; }, 1, cta_smem_bytes(h->n), a);
+  return with<64, 128, 256, 512>(p.cta_threads, [&](auto T) {
+    return launch(h, k_delta_cta<T, 1>, 1, T, ((cta_smem_bytes(h->n) + 15) & ~(size_t)15) + f32_smem_bytes(h->n), a);
+  });
 }
 
 int launch_reinit(pmc_handle* h, const ReinitArgs& a) {
@@ -240,71 +220,6 @@ ChainParams params_of(const pmc_case& c0, double kT_scale = 1.0) {
   P.clustering = c.clustering; P.alpha_carry = c.alpha_carry; P.cutoff_full = c.cutoff_full;
   P.planar = c.planar;
   return P;
-}
-
-// Block size for the ensemble at hand.  `base` is the shape that wins on a full machine (many chains per SM).
-// A small ensemble leaves SMs idle — 148 chains of n=100 are one warp per SM — so each chain gets 2× or 4× the
-// threads until the warps resident per SM reach what the base shape has when the machine is full
-// (profiles/r01f_tune_small_ensembles.txt: +50–80 % at one chain per SM, nothing lost on large ensembles).
-static int scaled_threads(int base, int minb, size_t smem, int tmax, int64_t chains, int sms, int max_scale = 4) {
-  const int fit = (int)std::max<size_t>(1, (size_t)233472 / (smem + 1024));  // CTAs per SM that fit in shared memory
-  const int resident_max = std::min(minb, fit);
-  const double sat = (double)resident_max * (base / 32);                     // warps per SM, full machine
-  const double res = std::min((double)chains / sms, (double)resident_max) * (base / 32);
-  int scale = 1;
-  while (scale < max_scale && base * scale * 2 <= tmax && res * scale * 2 <= sat) scale *= 2;
-  return base * scale;
-}
-
-// (Re)choose cta_threads from n and the ensemble size.
-static void choose_shape(pmc_handle* h) {
-  const int64_t chains = h->shape_chains > 0 ? h->shape_chains : h->nchains;
-  const bool cta_pairs = h->energy_type == PMC_ENERGY_INTERACTING || h->energy_type == PMC_ENERGY_CUTOFF;
-  if (h->cluster_mode && cta_pairs) {
-    const int base = pick_cluster_threads(h->n);
-    const int minb = base == 32 ? (h->n <= 40 ? 16 : h->n <= 110 ? 10 : 8) : base == 64 ? 5 : base == 128 ? cluster_fit128(h->n) : 1;
-    int t;
-    if (base == 32 && env_int("PMC_CLUSTER_SPEC", 1) != 0) {
-      // one-warp teams (n ≤ 160): the extra warps of a small ensemble run DIFFERENT trials of the same chain
-      // (k_run_cta_cluster_spec).  The largest number of teams whose CTAs are all resident at once — a second wave costs
-      // more than the teams gain (profiles/r02d_tune_spec.txt: 500 chains on 444 slots of four teams lose to two teams)
-      t = 32;
-      const int teams[3] = {8, 4, 2}, per_sm[3] = {1, 3, 5};   // launch bounds of run_cluster_cta.cu
-      for (int k = 0; k < 3; ++k) {
-        const size_t smem = cluster_spec_smem_bytes(h->n, teams[k]) + 1024;
-        const int fit = (int)std::min<size_t>((size_t)per_sm[k], (size_t)233472 / smem);
-        if (fit >= 1 && chains <= (int64_t)h->sm_count * fit && cluster_delta_smem_bytes(h->n, 32 * teams[k]) <= (size_t)kSmemMax) {
-          t = 32 * teams[k];
-          break;
-        }
-      }
-    } else {
-      t = scaled_threads(base, minb, cluster_smem_bytes(h->n, base), 256, chains, h->sm_count);
-      while (t > base && cluster_delta_smem_bytes(h->n, t) > (size_t)kSmemMax) t /= 2;
-    }
-    h->cta_threads = t;
-    return;
-  }
-  const int base = pick_cta_threads(h->n);
-  const int minb = base == 64 ? 8 : base == 128 ? 4 : base == 256 ? 2 : 1;
-  h->cta_threads = scaled_threads(base, minb, cta_smem_bytes_win(h->n), 512, chains, h->sm_count);
-  // Small ensembles of short interacting chains: one-warp teams on DIFFERENT trials of the window (k_run_cta_win_spec)
-  // instead of more warps on one trial.  Unlike the composite trial, the single-monomer trial has almost no serial head and
-  // shares well among warps, so this pays only where a warp is enough for a trial (profiles/r02e_tune_spec_plain.txt):
-  // n ≤ 64 with the largest number of teams whose CTAs are all resident at once (8 × 1, 4 × 3, 2 × 6 per SM: +10–70 %), and
-  // n ≤ 110 when every chain can have a whole SM (eight teams, +17–29 %); above that the one-trial kernels win.
-  h->spec_teams = 0;
-  if (h->energy_type == PMC_ENERGY_INTERACTING && !h->cluster_mode && h->n <= 110 && env_int("PMC_RUN_SPEC", 1) != 0) {
-    const int teams[3] = {8, 4, 2}, per_sm[3] = {1, 3, 6};
-    for (int k = 0; k < (h->n <= 64 ? 3 : 1); ++k) {
-      const size_t smem = cta_smem_bytes_spec(h->n, teams[k]) + 1024;
-      const int fit = (int)std::min<size_t>((size_t)per_sm[k], (size_t)233472 / smem);
-      if (fit >= 1 && chains <= (int64_t)h->sm_count * fit) {
-        h->spec_teams = teams[k];
-        break;
-      }
-    }
-  }
 }
 
 int fetch_dyn(pmc_handle* h) {
@@ -393,13 +308,10 @@ int32_t pmc_create(const pmc_case* cases, int64_t ncases, int32_t replicas_per_c
   for (int64_t i = 0; i < ncases; ++i)
     if (needs_cluster_path(cases[i])) h->cluster_mode = 1;
   const bool cta_pairs = h->energy_type == PMC_ENERGY_INTERACTING || h->energy_type == PMC_ENERGY_CUTOFF;
-  choose_shape(h);
-  if (h->cluster_mode && cta_pairs) {
-    if (cluster_delta_smem_bytes(n, h->cta_threads) > (size_t)kSmemMax) {
-      delete h;
-      return fail(PMC_ERR_UNSUPPORTED, "chain too long for the clustering / bending / cut-off kernels: 18 n doubles "
-                                       "must fit one CTA's 227 KB shared memory (num-monomers <= ~1570)");
-    }
+  if (h->cluster_mode && cta_pairs && cluster_delta_smem_bytes(n, plan_run(h).cta_threads) > (size_t)kSmemMax) {
+    delete h;
+    return fail(PMC_ERR_UNSUPPORTED, "chain too long for the clustering / bending / cut-off kernels: 18 n doubles "
+                                     "must fit one CTA's 227 KB shared memory (num-monomers <= ~1570)");
   }
 
   lap("validate + handle");
@@ -492,7 +404,6 @@ int32_t pmc_set_ensemble_hint(pmc_handle* h, int64_t ensemble_chains) {
   if (rc) return rc;
   if (ensemble_chains < 0) return fail(PMC_ERR_INVALID, "ensemble_chains must be >= 0");
   h->shape_chains = ensemble_chains;
-  choose_shape(h);
   return PMC_OK;
 }
 
@@ -504,9 +415,9 @@ int32_t pmc_set_pair_precision(pmc_handle* h, int32_t mode) {
   return PMC_OK;
 }
 
-int32_t pmc_pair_precision(const pmc_handle* h) { return h && use_f32_rect(h) ? PMC_PAIR_FP32 : PMC_PAIR_FP64; }
+int32_t pmc_pair_precision(const pmc_handle* h) { return h && plan_run(h).f32 ? PMC_PAIR_FP32 : PMC_PAIR_FP64; }
 
-int32_t pmc_block_threads(const pmc_handle* h) { return h ? h->cta_threads : 0; }
+int32_t pmc_block_threads(const pmc_handle* h) { return h ? plan_run(h).cta_threads : 0; }
 
 int32_t pmc_set_stream(pmc_handle* h, void* cuda_stream) {
   int rc = check_handle(h);
@@ -601,12 +512,6 @@ static int energy_range(pmc_handle* h, int64_t first, int64_t count, double* out
   return PMC_OK;
 }
 
-// Composite-trial kernels: CTA per chain for the pair-sum energies, chain per lane / warp otherwise.
-static int launch_run_cluster(pmc_handle* h, const RunArgs& a) {
-  const bool cta_pairs = h->energy_type == PMC_ENERGY_INTERACTING || h->energy_type == PMC_ENERGY_CUTOFF;
-  return cta_pairs ? launch_run_cluster_cta(h, a) : launch_run_cluster_lane(h, a);
-}
-
 static int launch_delta_segment(pmc_handle* h, const SegDeltaArgs& a) {
   const bool cta_pairs = h->energy_type == PMC_ENERGY_INTERACTING || h->energy_type == PMC_ENERGY_CUTOFF;
   if (cta_pairs) return launch_delta_segment_cta(h, a);
@@ -692,11 +597,24 @@ int64_t pmc_rows_for(const pmc_handle* h, int64_t nsteps, int64_t stepout) {
   return (step0 + nsteps) / stepout - step0 / stepout;
 }
 
-// The MCMC kernel of this handle: driver (plain / clustering), energy type, n and ensemble size select it.
+// The MCMC kernel of this handle as planned now (plan_run), followed, for the FP32 rectangle, by the energy refresh: the
+// running energy is the sum of FP32-rounded ΔU of the accepted moves; put it back on the exact energy of the chain after
+// every launch (one FP64 energy evaluation per chain ≈ three trials' worth of pairs).
 static int dispatch_run(pmc_handle* h, const RunArgs& a) {
-  if (h->cluster_mode) return launch_run_cluster(h, a);
-  if (h->energy_type == PMC_ENERGY_INTERACTING) return launch_run_cta(h, a);
-  return launch_run_lane(h, a);
+  const RunPlan p = plan_run(h);
+  int rc;
+  switch (p.family) {
+    case RunFamily::cta_win:
+    case RunFamily::cta_win_spec: rc = launch_run_cta(h, p, a); break;
+    case RunFamily::cta_pair: rc = launch_run_pair(h, p, a); break;
+    case RunFamily::lane:
+    case RunFamily::warp: rc = launch_run_lane(h, p, a); break;
+    case RunFamily::cta_cluster:
+    case RunFamily::cta_cluster_spec: rc = launch_run_cluster_cta(h, p, a); break;
+    default: rc = launch_run_cluster_lane(h, p, a); break;
+  }
+  if (rc) return rc;
+  return p.f32 ? refresh(h, /*rebind_gauge=*/false) : PMC_OK;
 }
 
 static int run_impl(pmc_handle* h, int64_t nsteps, int64_t stepout, double* traj, double* roll, int roll_cols,
@@ -748,6 +666,10 @@ static int run_args(pmc_handle* h, int64_t nsteps, int64_t stepout, int64_t rows
   a.n = h->n; a.nchains = (int)h->nchains; a.energy_type = h->energy_type;
   a.dynx = h->dynx; a.state = nstate ? h->state : nullptr; a.roll_cols = roll_cols;
   a.compensated = h->compensated;
+  // k_run_warp_cluster: trials per window.  An accepted trial invalidates the later trials of the window that read its
+  // segment and every invalidation costs a serial re-evaluation pass, but the per-window work (draws, prefix sums,
+  // averagers) is amortised over the window: 32 wins from n = 25 to 400 (profiles/r01f_tune_warp_cluster.txt).
+  a.window = 32;
   return PMC_OK;
 }
 
@@ -769,9 +691,6 @@ static int run_impl(pmc_handle* h, int64_t nsteps, int64_t stepout, double* traj
   if ((rc = run_args(h, nsteps, stepout, rows, roll_cols, state != nullptr, a))) return rc;
   PMC_CU(cudaEventRecord(h->ev0, h->stream));
   if ((rc = dispatch_run(h, a))) return rc;
-  // FP32 rectangle: the running energy is the sum of FP32-rounded ΔU of the accepted moves; put it back on the exact
-  // energy of the chain after every launch (one FP64 energy evaluation per chain ≈ three trials' worth of pairs)
-  if (use_f32_rect(h) && (rc = refresh(h, /*rebind_gauge=*/false))) return rc;
   PMC_CU(cudaEventRecord(h->ev1, h->stream));
   if (traj && rows > 0)
     PMC_CU(cudaMemcpyAsync(traj, h->traj, ntraj * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -797,13 +716,9 @@ int32_t pmc_kernel_name(pmc_handle* h, char* buf, int32_t buflen) {
   int rc = check_handle(h);
   if (rc) return rc;
   if (!buf || buflen < 1) return fail(PMC_ERR_INVALID, "null or empty name buffer");
-  RunArgs a{};
-  a.n = h->n; a.nchains = (int)h->nchains; a.energy_type = h->energy_type; a.compensated = h->compensated;
-  h->dry_run = 1;  // the launch helpers record their decision and stop
-  rc = dispatch_run(h, a);
-  h->dry_run = 0;
-  if (rc) return rc;
-  std::snprintf(buf, (size_t)buflen, "%s", h->kernel_name);
+  const RunPlan p = plan_run(h);
+  if (p.smem > (size_t)kSmemMax) return fail(PMC_ERR_UNSUPPORTED, "chain too long for this kernel's shared memory");
+  std::snprintf(buf, (size_t)buflen, "%s", kernel_name(p).c_str());
   return PMC_OK;
 }
 
@@ -1064,7 +979,6 @@ int tempering_impl(pmc_handle* h, int64_t nsteps, int64_t every, int64_t stepout
   for (int64_t k = 0; k < nsteps / every; ++k) {   // exactly pmc_run(every) followed by pmc_exchange, k times
     if ((rc = refresh(h, false))) return rc;
     if ((rc = dispatch_run(h, a))) return rc;
-    if (use_f32_rect(h) && (rc = refresh(h, /*rebind_gauge=*/false))) return rc;
     for (int j = 0; j < 3; ++j)
       if (host_out[j] && rows > 0 &&
           (rc = launch_place_rows(h, h->tt_out[j], chunk_out[j], rows, rows_total, k * rows, (int)per_row[j])))
