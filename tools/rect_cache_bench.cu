@@ -54,7 +54,7 @@ __global__ void __launch_bounds__(T, MINB) k_rect(double* out, double* __restric
   double* g = cache + (size_t)blockIdx.x * n * n;
   constexpr int W = T / 32;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  using TEAM = Team<W, 0>;
+  using TEAM = Team<W>;
   double acc = 0.0;
   for (int r = 0; r < reps; ++r) {
     const int idx = trial_idx(r, n);
