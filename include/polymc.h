@@ -292,6 +292,36 @@ int32_t pmc_run_tempering_ex(pmc_handle* h, int64_t nsteps, int64_t exchange_eve
                              double* traj, double* roll19, double* state);
 int32_t pmc_exchange_stats(pmc_handle* h, double* pair_stats, int64_t* walker, int64_t* round_trips);
 
+/* ---- conformation sampling: the shape of every chain, sampled on the device (DESIGN.md §13) ---- */
+/* A new capability: the reference measures only whole-chain scalars, and a handle without sampling runs as before.
+ * Per chain the device keeps plain FP64 running sums over samples, cols = 8 + 3n + B doubles (x_i = monomer centres,
+ * n̂_i the record's direction; averages = sums / col 0; replicas of one case pool by adding rows):
+ *   0: 1 (the sample count) · 1–6: S_xx S_yy S_zz S_xy S_xz S_yz of the gyration tensor S = (1/n) Σ_i (x_i − x̄)(x_i − x̄)ᵀ
+ *   7: (tr S)² · 8 + s, s = 0 … n−1: C_s = Σ_{i=0}^{n−1−s} n̂_i·n̂_{i+s} · 8 + n + i: n̂z_i · 8 + 2n + i: n̂z_i²
+ *   8 + 3n + k, k < B: histogram of ζ = r_z / (n b) on [−1, 1], bin k = min(B−1, max(0, ⌊(ζ+1)·B/2⌋)), r_z as
+ *   pmc_observables computes it.
+ * pmc_set_conformation: enable != 0 enables sampling with B = hist_bins (0: no histogram, at most 65536) and zeroes the
+ * sums; enable = 0 disables it and frees the sums.  PMC_ERR_INVALID for any umbrella case in the handle (its samples
+ * would need the umbrella weights) and for hist_bins out of range.
+ * pmc_conformation_cols: 8 + 3n + B, or 0 when disabled.
+ * pmc_sample_conformation: one sample of every chain's current configuration.
+ * pmc_run_sampled / _ex: pmc_run / pmc_run_ex (sample_every) followed by pmc_sample_conformation, nsteps / sample_every
+ * times, bit-identical to that loop, rows included, without host synchronisation between the chunks; preconditions and
+ * rows as pmc_run_tempering*.  With sampling enabled, pmc_run_tempering* also samples after every exchange round
+ * (pmc_run; pmc_exchange; pmc_sample_conformation, repeated).  pmc_run / pmc_run_ex never sample.
+ * pmc_conformation_sums: sums [chains][cols].
+ * pmc_begin_stage zeroes the sums; pmc_reinit keeps them; pmc_exchange leaves them with the slot (a case's averages are
+ * those of its rung).  With sampling enabled pmc_checkpoint_save appends B and the sums after the ladder block, and
+ * pmc_checkpoint_load requires the same setting; without it checkpoints are unchanged.  pmc_multi_* has no sampling
+ * of its own: enable it on each shard (pmc_multi_shard). */
+int32_t pmc_set_conformation(pmc_handle* h, int32_t enable, int32_t hist_bins);
+int64_t pmc_conformation_cols(const pmc_handle* h);
+int32_t pmc_sample_conformation(pmc_handle* h);
+int32_t pmc_run_sampled(pmc_handle* h, int64_t nsteps, int64_t sample_every, int64_t stepout, double* traj, double* roll);
+int32_t pmc_run_sampled_ex(pmc_handle* h, int64_t nsteps, int64_t sample_every, int64_t stepout,
+                           double* traj, double* roll19, double* state);
+int32_t pmc_conformation_sums(pmc_handle* h, double* sums);
+
 /* ---- one ensemble over several GPUs of one box (ABI v3) ------------------------------------ */
 /* Replaces the fan-out of the reference's launchers — `julia -p N run/interacting_dielectric_study.jl workdir`,
  * run/interacting_dielectric_study.jl:37-47 (pmap over cases, one single-threaded process per case).  The

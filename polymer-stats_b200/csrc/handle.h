@@ -105,6 +105,9 @@ struct pmc_handle {
   int64_t ex_round = 0;                 // exchange rounds since pmc_set_ladders
   double* tt_out[3] = {nullptr, nullptr, nullptr};   // traj, roll, state rows of a whole pmc_run_tempering*
   size_t tt_cap[3] = {0, 0, 0};
+  // conformation sampling (conformation.cuh), set by pmc_set_conformation; conf == nullptr: disabled
+  double* conf = nullptr;               // [chains][8 + 3n + conf_bins] running sums
+  int conf_bins = 0;
 };
 
 // Device memory of the handles comes from a per-device cache of freed blocks: a study creates and destroys one handle
@@ -167,3 +170,4 @@ int launch_run_cluster_lane(pmc_handle* h, const RunPlan& p, const pmc::RunArgs&
 int launch_exchange(pmc_handle* h, const pmc::ExchangeArgs& a, int64_t npairs);   // exchange.cu
 int launch_place_rows(pmc_handle* h, double* dst, const double* src, int64_t rows, int64_t rows_total, int64_t row0,
                       int cols);                                             // exchange.cu
+int launch_conformation(pmc_handle* h);                                      // conformation.cu

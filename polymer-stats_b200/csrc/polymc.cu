@@ -4,6 +4,7 @@
 // PMC_ERR_NO_DEVICE / PMC_ERR_CUDA otherwise.
 #include "handle.h"
 #include "exchange.cuh"
+#include "conformation.cuh"
 
 namespace {
 
@@ -389,7 +390,7 @@ void pmc_destroy(pmc_handle* h) {
   if (h->pair_order) pmc_pool_free(h->pair_order);
   if (h->pair_next) pmc_pool_free(h->pair_next);
   for (void* p : {(void*)h->ex_pairs, (void*)h->ex_stats, (void*)h->ex_walker, (void*)h->ex_wstate, (void*)h->ex_trips,
-                  (void*)h->tt_out[0], (void*)h->tt_out[1], (void*)h->tt_out[2]})
+                  (void*)h->tt_out[0], (void*)h->tt_out[1], (void*)h->tt_out[2], (void*)h->conf})
     if (p) pmc_pool_free(p);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
@@ -842,6 +843,9 @@ int32_t pmc_begin_stage(pmc_handle* h, double kT_scale) {
   ++h->launches;
   PMC_CU(cudaGetLastError());
   if ((rc = refresh(h, /*rebind_gauge=*/true))) return rc;  // chain.U = U(chain); wf = AntiDipoleWeightFunction(chain)
+  if (h->conf)   // fresh averagers, conformation sums included
+    PMC_CU(cudaMemsetAsync(h->conf, 0, (size_t)h->nchains * (8 + 3 * (size_t)h->n + (size_t)h->conf_bins) * sizeof(double),
+                           h->stream));
   PMC_CU(cudaStreamSynchronize(h->stream));
   if (!h->host_dyn.empty()) h->host_dyn[0].step = 0;
   return PMC_OK;
@@ -954,16 +958,21 @@ int exchange_round(pmc_handle* h) {
   return PMC_OK;
 }
 
-int tempering_impl(pmc_handle* h, int64_t nsteps, int64_t every, int64_t stepout, double* traj, double* roll,
-                   int roll_cols, double* state) {
+// The chunk loop of pmc_run_tempering* (exchange = true) and pmc_run_sampled* (exchange = false): nsteps / every times
+// exactly pmc_run(every), then pmc_exchange when exchanging, then pmc_sample_conformation when sampling is enabled,
+// with the rows placed on the device and no host synchronisation between the chunks.
+int chunk_impl(pmc_handle* h, int64_t nsteps, int64_t every, int64_t stepout, double* traj, double* roll,
+               int roll_cols, double* state, bool exchange) {
   int rc = check_handle(h);
   if (rc) return rc;
-  if (h->ladder.empty()) return fail(PMC_ERR_INVALID, "no ladders set (pmc_set_ladders)");
+  if (exchange && h->ladder.empty()) return fail(PMC_ERR_INVALID, "no ladders set (pmc_set_ladders)");
+  if (!exchange && !h->conf) return fail(PMC_ERR_INVALID, "conformation sampling is not enabled (pmc_set_conformation)");
   if (nsteps < 0) return fail(PMC_ERR_INVALID, "nsteps must be >= 0");
   if (nsteps == 0) return PMC_OK;
   if (nsteps >= (1LL << 40)) return fail(PMC_ERR_INVALID, "nsteps must stay below 2^40");
-  if (every < 1 || nsteps % every != 0) return fail(PMC_ERR_INVALID, "exchange_every must divide nsteps");
-  if (stepout > 0 && every % stepout != 0) return fail(PMC_ERR_INVALID, "stepout must divide exchange_every, or be 0");
+  const std::string what = exchange ? "exchange_every" : "sample_every";
+  if (every < 1 || nsteps % every != 0) return fail(PMC_ERR_INVALID, what + " must divide nsteps");
+  if (stepout > 0 && every % stepout != 0) return fail(PMC_ERR_INVALID, "stepout must divide " + what + ", or be 0");
   if ((rc = fetch_step0(h))) return rc;   // the only copy to the host before the results
   const int64_t rows_total = pmc_rows_for(h, nsteps, stepout), rows = stepout > 0 ? every / stepout : 0;
   const size_t per_row[3] = {8, (size_t)roll_cols, 2 * (size_t)h->n};
@@ -976,14 +985,15 @@ int tempering_impl(pmc_handle* h, int64_t nsteps, int64_t every, int64_t stepout
   if ((rc = run_args(h, every, stepout, rows, roll_cols, state != nullptr, a))) return rc;
   const double* chunk_out[3] = {h->traj, h->roll, h->state};
   PMC_CU(cudaEventRecord(h->ev0, h->stream));
-  for (int64_t k = 0; k < nsteps / every; ++k) {   // exactly pmc_run(every) followed by pmc_exchange, k times
+  for (int64_t k = 0; k < nsteps / every; ++k) {
     if ((rc = refresh(h, false))) return rc;
     if ((rc = dispatch_run(h, a))) return rc;
     for (int j = 0; j < 3; ++j)
       if (host_out[j] && rows > 0 &&
           (rc = launch_place_rows(h, h->tt_out[j], chunk_out[j], rows, rows_total, k * rows, (int)per_row[j])))
         return rc;
-    if ((rc = exchange_round(h))) return rc;
+    if (exchange && (rc = exchange_round(h))) return rc;
+    if (h->conf && (rc = launch_conformation(h))) return rc;
   }
   PMC_CU(cudaEventRecord(h->ev1, h->stream));
   for (int k = 0; k < 3; ++k)
@@ -1081,14 +1091,14 @@ int32_t pmc_exchange(pmc_handle* h, int32_t* accepted) {
 
 int32_t pmc_run_tempering(pmc_handle* h, int64_t nsteps, int64_t exchange_every, int64_t stepout, double* traj,
                           double* roll) {
-  return tempering_impl(h, nsteps, exchange_every, stepout, traj, roll, 17, nullptr);
+  return chunk_impl(h, nsteps, exchange_every, stepout, traj, roll, 17, nullptr, true);
 }
 
 int32_t pmc_run_tempering_ex(pmc_handle* h, int64_t nsteps, int64_t exchange_every, int64_t stepout, double* traj,
                              double* roll19, double* state) {
   if (h && !h->cluster_mode)
     return fail(PMC_ERR_INVALID, "pmc_run_tempering_ex needs a clustering-driver handle (clustering, bend-mod or cutoff case)");
-  return tempering_impl(h, nsteps, exchange_every, stepout, traj, roll19, 19, state);
+  return chunk_impl(h, nsteps, exchange_every, stepout, traj, roll19, 19, state, true);
 }
 
 int32_t pmc_exchange_stats(pmc_handle* h, double* pair_stats, int64_t* walker, int64_t* round_trips) {
@@ -1104,6 +1114,77 @@ int32_t pmc_exchange_stats(pmc_handle* h, double* pair_stats, int64_t* walker, i
   PMC_CU(cudaStreamSynchronize(h->stream));
   if (pair_stats)
     for (size_t i = 0; i < st.size(); ++i) pair_stats[i] = (double)st[i];
+  return PMC_OK;
+}
+
+// ---- conformation sampling ----------------------------------------------------------------------------------
+namespace {
+size_t conf_cols(const pmc_handle* h) { return h->conf ? 8 + 3 * (size_t)h->n + (size_t)h->conf_bins : 0; }
+
+void conf_clear(pmc_handle* h) {
+  if (h->conf) pmc_pool_free(h->conf);
+  h->conf = nullptr;
+  h->conf_bins = 0;
+}
+}  // namespace
+
+int32_t pmc_set_conformation(pmc_handle* h, int32_t enable, int32_t hist_bins) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (!enable) {
+    PMC_CU(cudaStreamSynchronize(h->stream));   // no launch in flight may still write the block
+    conf_clear(h);
+    return PMC_OK;
+  }
+  if (hist_bins < 0 || hist_bins > pmc::kConfMaxBins)
+    return fail(PMC_ERR_INVALID, "hist_bins must be in 0 … " + std::to_string(pmc::kConfMaxBins));
+  for (const pmc_case& c : h->cases)
+    if (c.umbrella) return fail(PMC_ERR_INVALID, "conformation sampling cannot serve umbrella cases: its samples would "
+                                                 "need the umbrella weights");
+  PMC_CU(cudaStreamSynchronize(h->stream));
+  conf_clear(h);
+  const size_t bytes = (size_t)h->nchains * (8 + 3 * (size_t)h->n + (size_t)hist_bins) * sizeof(double);
+  if ((rc = PMC_CU_RC(pool_alloc(&h->conf, bytes)))) return rc;
+  h->conf_bins = hist_bins;
+  if ((rc = PMC_CU_RC(cudaMemsetAsync(h->conf, 0, bytes, h->stream))) ||
+      (rc = PMC_CU_RC(cudaStreamSynchronize(h->stream)))) {
+    conf_clear(h);
+    return rc;
+  }
+  return PMC_OK;
+}
+
+int64_t pmc_conformation_cols(const pmc_handle* h) { return h ? (int64_t)conf_cols(h) : 0; }
+
+int32_t pmc_sample_conformation(pmc_handle* h) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (!h->conf) return fail(PMC_ERR_INVALID, "conformation sampling is not enabled (pmc_set_conformation)");
+  if ((rc = launch_conformation(h))) return rc;
+  PMC_CU(cudaStreamSynchronize(h->stream));
+  return PMC_OK;
+}
+
+int32_t pmc_run_sampled(pmc_handle* h, int64_t nsteps, int64_t sample_every, int64_t stepout, double* traj,
+                        double* roll) {
+  return chunk_impl(h, nsteps, sample_every, stepout, traj, roll, 17, nullptr, false);
+}
+
+int32_t pmc_run_sampled_ex(pmc_handle* h, int64_t nsteps, int64_t sample_every, int64_t stepout, double* traj,
+                           double* roll19, double* state) {
+  if (h && !h->cluster_mode)
+    return fail(PMC_ERR_INVALID, "pmc_run_sampled_ex needs a clustering-driver handle (clustering, bend-mod or cutoff case)");
+  return chunk_impl(h, nsteps, sample_every, stepout, traj, roll19, 19, state, false);
+}
+
+int32_t pmc_conformation_sums(pmc_handle* h, double* sums) {
+  int rc = check_handle(h);
+  if (rc) return rc;
+  if (!h->conf) return fail(PMC_ERR_INVALID, "conformation sampling is not enabled (pmc_set_conformation)");
+  if (!sums) return fail(PMC_ERR_INVALID, "null sums");
+  PMC_CU(cudaMemcpyAsync(sums, h->conf, (size_t)h->nchains * conf_cols(h) * sizeof(double), cudaMemcpyDeviceToHost,
+                         h->stream));
+  PMC_CU(cudaStreamSynchronize(h->stream));
   return PMC_OK;
 }
 
@@ -1132,6 +1213,18 @@ size_t ckpt_base_bytes(const pmc_handle* h) {
   return sizeof(CkptHeader) + c * (size_t)h->n * sizeof(MonoRec) + c * sizeof(ChainDyn) + c * sizeof(ChainDynX);
 }
 
+// Trailing block of a handle with conformation sampling, after the ladder block: this header and the sums
+// ([chains][cols] doubles).
+struct ConfHeader {
+  uint64_t magic;        // "PMCCONF1"
+  int64_t bins, cols, nchains;
+};
+constexpr uint64_t kConfMagic = 0x31464e4f43434d50ull;
+
+size_t conf_block_bytes(const pmc_handle* h) {
+  return h->conf ? sizeof(ConfHeader) + (size_t)h->nchains * conf_cols(h) * sizeof(double) : 0;
+}
+
 size_t ladder_block_bytes(const pmc_handle* h) {
   if (h->ladder.empty()) return 0;
   const size_t c = (size_t)h->nchains;
@@ -1142,7 +1235,7 @@ size_t ladder_block_bytes(const pmc_handle* h) {
 
 int64_t pmc_checkpoint_bytes(const pmc_handle* h) {
   if (!h) return 0;
-  return (int64_t)(ckpt_base_bytes(h) + ladder_block_bytes(h));
+  return (int64_t)(ckpt_base_bytes(h) + ladder_block_bytes(h) + conf_block_bytes(h));
 }
 
 int32_t pmc_checkpoint_save(pmc_handle* h, void* buf, int64_t bytes) {
@@ -1177,6 +1270,12 @@ int32_t pmc_checkpoint_save(pmc_handle* h, void* buf, int64_t bytes) {
     q += c * sizeof(int);
     PMC_CU(cudaMemcpyAsync(q, h->ex_trips, c * sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
   }
+  if (h->conf) {
+    unsigned char* q = static_cast<unsigned char*>(buf) + ckpt_base_bytes(h) + ladder_block_bytes(h);
+    const ConfHeader ch{kConfMagic, h->conf_bins, (int64_t)conf_cols(h), h->nchains};
+    std::memcpy(q, &ch, sizeof(ch));
+    PMC_CU(cudaMemcpyAsync(q + sizeof(ch), h->conf, c * conf_cols(h) * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+  }
   PMC_CU(cudaStreamSynchronize(h->stream));
   return PMC_OK;
 }
@@ -1202,10 +1301,22 @@ int32_t pmc_checkpoint_load(pmc_handle* h, const void* buf, int64_t bytes) {
     return fail(PMC_ERR_INVALID, "checkpoint holds replica-exchange ladders; set the same ladders before loading it");
   if (!h->ladder.empty()) {
     if (lh.magic != kLadderMagic) return fail(PMC_ERR_INVALID, "checkpoint has no replica-exchange ladders; this handle has");
-    if (bytes < pmc_checkpoint_bytes(h)) return fail(PMC_ERR_INVALID, "truncated checkpoint");
+    if (bytes < (int64_t)(ckpt_base_bytes(h) + ladder_block_bytes(h))) return fail(PMC_ERR_INVALID, "truncated checkpoint");
     if (lh.len != (int64_t)h->ladder.size() || lh.ncases != (int64_t)h->cases.size() || lh.nchains != h->nchains ||
         std::memcmp(q + sizeof(lh), h->ladder.data(), h->ladder.size() * sizeof(int32_t)) != 0)
       return fail(PMC_ERR_INVALID, "checkpoint ladders differ from this handle's (pmc_set_ladders)");
+  }
+  // the conformation block, after the ladder block
+  const unsigned char* r = static_cast<const unsigned char*>(buf) + ckpt_base_bytes(h) + ladder_block_bytes(h);
+  ConfHeader ch{};
+  if (bytes >= (int64_t)(r - static_cast<const unsigned char*>(buf) + sizeof(ch))) std::memcpy(&ch, r, sizeof(ch));
+  if (!h->conf && ch.magic == kConfMagic)
+    return fail(PMC_ERR_INVALID, "checkpoint holds conformation sums; enable the same conformation sampling before loading it");
+  if (h->conf) {
+    if (ch.magic != kConfMagic) return fail(PMC_ERR_INVALID, "checkpoint has no conformation sums; this handle samples");
+    if (ch.bins != h->conf_bins || ch.cols != (int64_t)conf_cols(h) || ch.nchains != h->nchains)
+      return fail(PMC_ERR_INVALID, "checkpoint conformation setting differs from this handle's (pmc_set_conformation)");
+    if (bytes < pmc_checkpoint_bytes(h)) return fail(PMC_ERR_INVALID, "truncated checkpoint");
   }
   if (hd.kT_scale != h->kT_scale) {  // the stage temperature lives in the per-chain constants
     std::vector<ChainParams> par(c);
@@ -1229,6 +1340,8 @@ int32_t pmc_checkpoint_load(pmc_handle* h, const void* buf, int64_t bytes) {
     PMC_CU(cudaMemcpyAsync(h->ex_trips, q, c * sizeof(long long), cudaMemcpyHostToDevice, h->stream));
     h->ex_round = lh.round;
   }
+  if (h->conf)
+    PMC_CU(cudaMemcpyAsync(h->conf, r + sizeof(ch), c * conf_cols(h) * sizeof(double), cudaMemcpyHostToDevice, h->stream));
   PMC_CU(cudaStreamSynchronize(h->stream));
   h->init = hd.init;
   h->dyn_fresh = h->dynx_fresh = false;

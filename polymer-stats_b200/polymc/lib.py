@@ -43,6 +43,9 @@ EXPORTS = [
     "pmc_release_cached_memory",
     # replica exchange across kT / force ladders of one handle
     "pmc_set_ladders", "pmc_exchange", "pmc_run_tempering", "pmc_run_tempering_ex", "pmc_exchange_stats",
+    # conformation sampling: gyration tensor, bond-orientation correlation, orientation profile, extension histogram
+    "pmc_set_conformation", "pmc_conformation_cols", "pmc_sample_conformation", "pmc_run_sampled", "pmc_run_sampled_ex",
+    "pmc_conformation_sums",
 ]
 RESULT_COLS = 24
 RESULT_NAMES = AVG_NAMES + ["acc_rate", "normalizer", "phi_step", "theta_step", "trials", "U_running", "Ealign", "psi"]
@@ -238,6 +241,13 @@ def load():
     L.pmc_run_tempering.argtypes = [hp, C.c_int64, C.c_int64, C.c_int64, dp, dp]
     L.pmc_run_tempering_ex.argtypes = [hp, C.c_int64, C.c_int64, C.c_int64, dp, dp, dp]
     L.pmc_exchange_stats.argtypes = [hp, dp, i64p, i64p]
+    L.pmc_set_conformation.argtypes = [hp, C.c_int32, C.c_int32]
+    L.pmc_conformation_cols.argtypes = [hp]
+    L.pmc_conformation_cols.restype = C.c_int64
+    L.pmc_sample_conformation.argtypes = [hp]
+    L.pmc_run_sampled.argtypes = [hp, C.c_int64, C.c_int64, C.c_int64, dp, dp]
+    L.pmc_run_sampled_ex.argtypes = [hp, C.c_int64, C.c_int64, C.c_int64, dp, dp, dp]
+    L.pmc_conformation_sums.argtypes = [hp, dp]
     for name in EXPORTS:
         f = getattr(L, name)
         if f.restype is C.c_int:  # default restype: every status-returning entry point
@@ -276,6 +286,20 @@ def fp64_peak_probe(device=0, iters=1 << 17):
     ms = C.c_float()
     _check(load().pmc_fp64_peak_probe(device, iters, C.byref(t), C.byref(ms)))
     return t.value, ms.value
+
+
+def conformation_averages(sums, n: int, bins: int) -> dict:
+    """Averages of conformation sums [chains][8 + 3n + B] (pmc_conformation_sums, or rows of one case added up):
+    S [chains][6] (S_xx S_yy S_zz S_xy S_xz S_yz), Rg2 = ⟨tr S⟩, Rg4 = ⟨(tr S)²⟩, bondcorr [chains][n] = ⟨C_s⟩/(n−s),
+    nz, nz2 [chains][n] = ⟨n̂z_i⟩, ⟨n̂z_i²⟩, hist [chains][B] = the fraction of samples in each ζ bin, samples [chains]."""
+    sums = np.asarray(sums, dtype=np.float64)
+    if sums.shape[-1] != 8 + 3 * n + bins:
+        raise PolymcError(-1, f"conformation rows have 8 + 3n + B = {8 + 3 * n + bins} columns, not {sums.shape[-1]}")
+    k = sums[..., 0:1]
+    S = sums[..., 1:7] / k
+    return {"samples": sums[..., 0].copy(), "S": S, "Rg2": S[..., 0] + S[..., 1] + S[..., 2], "Rg4": sums[..., 7] / k[..., 0],
+            "bondcorr": sums[..., 8:8 + n] / k / np.arange(n, 0, -1), "nz": sums[..., 8 + n:8 + 2 * n] / k,
+            "nz2": sums[..., 8 + 2 * n:8 + 3 * n] / k, "hist": sums[..., 8 + 3 * n:] / k}
 
 
 class Ensemble:
@@ -551,6 +575,51 @@ class Ensemble:
         _check(load().pmc_exchange_stats(self._h, _dp(ps), walker.ctypes.data_as(i64p), trips.ctypes.data_as(i64p)))
         return {"attempts": ps[:, 0].astype(np.int64), "accepts": ps[:, 1].astype(np.int64), "walker": walker,
                 "round_trips": trips}
+
+    # ---- conformation sampling (include/polymc.h, DESIGN.md §13) ----
+    def set_conformation(self, hist_bins=0, enable=True):
+        """Enable sampling of the chains' shape with an extension histogram of `hist_bins` bins (0: none) and zero the
+        sums; enable=False disables it."""
+        _check(load().pmc_set_conformation(self._h, int(bool(enable)), int(hist_bins)))
+
+    def conformation_cols(self) -> int:
+        return int(load().pmc_conformation_cols(self._h))
+
+    def sample_conformation(self):
+        """One sample of every chain's current configuration."""
+        _check(load().pmc_sample_conformation(self._h))
+
+    def _sampled_rows(self, nsteps, sample_every, stepout, fetch_rows, cols, want_state):
+        if sample_every < 1 or nsteps % sample_every:
+            raise PolymcError(-1, "sample_every must divide nsteps")
+        return self._tempering_rows(nsteps, sample_every, stepout, fetch_rows, cols, want_state)
+
+    def run_sampled(self, nsteps, sample_every, stepout=0, fetch_rows=True):
+        """run(sample_every) followed by sample_conformation(), nsteps / sample_every times, on the device without host
+        synchronisation between the chunks.  Returns (traj, roll) as run()."""
+        traj, roll, _ = self._sampled_rows(nsteps, sample_every, stepout, fetch_rows, 17, False)
+        _check(load().pmc_run_sampled(self._h, nsteps, sample_every, stepout, _dp(traj), _dp(roll)))
+        return traj, roll
+
+    def run_sampled_ex(self, nsteps, sample_every, stepout=0, fetch_rows=True, want_state=False):
+        """The clustering driver's run_ex(sample_every) followed by sample_conformation(), repeated; rows as run_ex()."""
+        traj, roll, state = self._sampled_rows(nsteps, sample_every, stepout, fetch_rows, 19, want_state)
+        _check(load().pmc_run_sampled_ex(self._h, nsteps, sample_every, stepout, _dp(traj), _dp(roll), _dp(state)))
+        return traj, roll, state
+
+    def conformation_sums(self):
+        """[chains][8 + 3n + B] running sums (include/polymc.h)."""
+        cols = self.conformation_cols()
+        if cols == 0:
+            raise PolymcError(-1, "conformation sampling is not enabled (set_conformation)")
+        s = np.empty((self.nchains, cols))
+        _check(load().pmc_conformation_sums(self._h, _dp(s)))
+        return s
+
+    def conformation(self):
+        """Per-chain averages of the samples (conformation_averages)."""
+        s = self.conformation_sums()
+        return conformation_averages(s, self.n, s.shape[1] - 8 - 3 * self.n)
 
 
 class _Shard(Ensemble):

@@ -163,9 +163,10 @@ def _collect_exchange(exchange, st, ladders, case0: int, ncases: int, nrep: int)
 
 def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0, device: int = 0,
               rank: int = 0, world: int = 1, protocol=None, bit_identical: bool = False, pair_precision: str = "fp64",
-              temper=None, exchange_every: int = 100, exchange=None):
+              temper=None, exchange_every: int = 100, exchange=None, conformation_every: int = 0,
+              conformation_bins: int = 0):
     """Run this rank's contiguous block of every (n, energy) bucket.  Returns a list of
-    (global chain ids of the bucket, lo, block [hi-lo][NCOL]).  No communication.
+    (global chain ids of the bucket, lo, block [hi-lo][NCOL + conformation columns]).  No communication.
 
     protocol None: `nsteps` trials of mcmc_eap_chain.jl's loop.  protocol = dict(burn_in=…, schedule=[…]):
     the clustering driver's ladder (mcmc_clustering_eap_chain.jl:365-386) — a burn-in stage per kT
@@ -174,9 +175,24 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
     temper "kT" / "Fz" / "Fx": replica exchange every `exchange_every` trials along the ladders of
     tempering_ladders() in every run of the protocol (each init, each burn-in stage).  A ladder lives in one
     handle, so this needs a single rank.  `exchange`, a dict, receives the ladders, the per-case attempts and
-    accepts with the next rung and the round trips of every ladder."""
+    accepts with the next rung and the round trips of every ladder.
+
+    conformation_every K > 0: the production run samples every chain's shape every K trials (Ensemble.run_sampled; with
+    temper, at the exchange rounds, so K must equal exchange_every) with an extension histogram of conformation_bins
+    bins; the chain's conformation sums (8 + 3n + B, include/polymc.h) follow the NCOL columns of its row."""
     if not isinstance(cases, lib.CaseTable):
         cases = list(cases)
+    conformation_every = int(conformation_every)
+    if conformation_every:
+        rec = cases.rec if isinstance(cases, lib.CaseTable) else lib.CaseTable(cases).rec
+        if np.any(rec["umbrella"] != 0):
+            raise lib.PolymcError(-1, "conformation sampling cannot serve umbrella cases: its samples would need the "
+                                      "umbrella weights")
+        if conformation_every < 1 or nsteps % conformation_every:
+            raise lib.PolymcError(-1, f"--conformation-every ({conformation_every}) must divide --num-steps")
+        if temper is not None and conformation_every != int(exchange_every):
+            raise lib.PolymcError(-1, "with --temper the chains are sampled at the exchange rounds: --conformation-every "
+                                      "must equal --exchange-every")
     ladders = None
     if temper is not None:
         if world > 1:
@@ -195,7 +211,8 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
         gids = (np.asarray(idxs, dtype=np.int64)[:, None] * replicas + np.arange(replicas, dtype=np.int64)).ravel()
         lo, hi = shard_range(len(gids), rank, world)
         mine = gids[lo:hi]
-        block = np.zeros((hi - lo, NCOL))
+        n_bucket = int(cases[int(idxs[0])].n)
+        block = np.zeros((hi - lo, NCOL + (8 + 3 * n_bucket + int(conformation_bins) if conformation_every else 0)))
         for pos, end, case0, ncases, nrep in _segments(mine, replicas):
             # The Markov chains (Philox streams keyed by global chain id) never depend on the sharding.  The launch shape —
             # block size, packing, one or two SMs per chain — is chosen for THIS shard's size (fastest: a 512-chain
@@ -217,11 +234,20 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
 
                     def run_ex(k, so, fetch_rows):
                         return ens.run_tempering_ex(k, exchange_every, so, fetch_rows=fetch_rows)
+                prod, prod_ex = run, run_ex        # the production run: sampled when conformation_every is set
+                if conformation_every:
+                    ens.set_conformation(conformation_bins)
+                    if not local:
+                        def prod(k, so, fetch_rows):
+                            return ens.run_sampled(k, conformation_every, so, fetch_rows=fetch_rows)
+
+                        def prod_ex(k, so, fetch_rows):
+                            return ens.run_sampled_ex(k, conformation_every, so, fetch_rows=fetch_rows)
                 if protocol is None or protocol.get("plain"):
                     # mcmc_eap_chain.jl:276-361: num-inits passes of nsteps trials with the re-initialisation rule between
                     inits = int(protocol.get("num_inits", 1)) if protocol else 1
                     for init in range(inits):
-                        run(nsteps, stepout, fetch_rows=False)
+                        prod(nsteps, stepout, fetch_rows=False)
                         if init + 1 < inits:
                             ens.reinit()
                 else:
@@ -230,8 +256,8 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
                     for mult in protocol.get("schedule", []):
                         ens.begin_stage(float(mult))
                         run_ex(int(protocol.get("burn_in", 0)), 0, fetch_rows=False)
-                    ens.begin_stage(1.0)
-                    run_ex(nsteps, 0, fetch_rows=False)
+                    ens.begin_stage(1.0)             # also zeroes the conformation sums of the burn-in
+                    prod_ex(nsteps, 0, fetch_rows=False)
                     block[pos:end, 35:37] = ens.extra_accumulators()
                 if local and exchange is not None:
                     _collect_exchange(exchange, ens.exchange_stats(), ladders, case0, ncases, nrep)
@@ -240,6 +266,8 @@ def run_shard(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0
                 block[pos:end, 16] = ar
                 block[pos:end, 17] = nrm
                 block[pos:end, 18:35] = ens.accumulators()
+                if conformation_every:
+                    block[pos:end, NCOL:] = ens.conformation_sums()
         out.append((gids, lo, block))
     return out
 
@@ -266,36 +294,50 @@ def assemble(total: int, parts):
 
 def run_sweep(cases, replicas: int, nsteps: int, stepout: int = 0, seed: int = 0, device: int = 0,
               torch_device=None, protocol=None, bit_identical: bool = False, pair_precision: str = "fp64",
-              temper=None, exchange_every: int = 100):
+              temper=None, exchange_every: int = 100, conformation_every: int = 0, conformation_bins: int = 0):
     """Run every (case, replica) chain of a sweep for nsteps trials, sharded over the ranks of the
     current torch.distributed group (or a single process), then gather the final per-chain results on
     every rank.  Chain order = case-major: avg [ncases*replicas][16], acc_rate, normalizer, sums [..][17].
-    With temper (run_shard), "exchange" holds the ladders and their exchange statistics."""
+    With temper (run_shard), "exchange" holds the ladders and their exchange statistics.  With conformation_every,
+    "conformation" is a list, one entry per bucket, of dict(n, bins, cases [k] (case indices), sums [k][8 + 3n + B]):
+    the conformation sums of every case, added over its replicas (in replica order, whatever the rank count)."""
     dist = _dist()
     rank = dist.get_rank() if dist else 0
     world = dist.get_world_size() if dist else 1
     if not isinstance(cases, lib.CaseTable):
         cases = list(cases)
     parts, exchange = [], {}
+    conformation = []
     for gids, lo, block in run_shard(cases, replicas, nsteps, stepout, seed, device, rank, world, protocol, bit_identical,
-                                     pair_precision, temper, exchange_every, exchange):
-        parts.append((gids, gather_rows(block, len(gids), lo, device=torch_device)))
+                                     pair_precision, temper, exchange_every, exchange, conformation_every,
+                                     conformation_bins):
+        full = gather_rows(block, len(gids), lo, device=torch_device)
+        parts.append((gids, full))
+        if conformation_every:   # a bucket holds whole cases, replicas consecutive
+            sums = full[:, NCOL:].reshape(len(gids) // replicas, replicas, -1).sum(axis=1)
+            conformation.append(dict(n=(sums.shape[1] - 8 - int(conformation_bins)) // 3, bins=int(conformation_bins),
+                                     cases=gids[::replicas] // replicas, sums=sums))
     res = assemble(len(cases) * replicas, parts)
     if temper is not None:
         res["exchange"] = exchange
+    if conformation_every:
+        res["conformation"] = conformation
     return res
 
 
 def sweep_table(pargs_list, driver: str = "plain", runs: int = 1, seed: int = 0, device: int = 0, torch_device=None,
                 kappaflag: bool = False, pooled: bool = False, with_entries: bool = False, bit_identical: bool = False,
-                temper=None, exchange_every: int = 100, exchange=None):
+                temper=None, exchange_every: int = 100, exchange=None, conformation_every: int = 0,
+                conformation_bins: int = 0, conformation=None):
     """A whole launcher + aggregate_mcmc.jl (+ reduce_tabular_data.jl) pipeline in one call (SURVEY §8f
     rank 3): every pargs dict of `pargs_list` is one case (one launcher command line), run `runs` times as
     independent replica chains (the launchers' `run-NNN` cases); the result is the aggregated table the
     reference's scripts would build from the `.out` files.  Returns (header, rows, entries) with entries =
     [(prefix, stdout text)] for optional `.out` emission.  temper / exchange_every: replica exchange along the
     ladders of the sweep (run_shard); the table keeps its format, a row per case being a row per rung.  `exchange`,
-    a dict, receives the ladders and their statistics (see exchange_rows)."""
+    a dict, receives the ladders and their statistics (see exchange_rows).  conformation_every / conformation_bins:
+    sample the production run's conformations (run_shard); `conformation`, a dict, receives run_sweep's "conformation"
+    list under "buckets" (see conformation_tables).  The table keeps its format."""
     from . import aggregate as agg
     from . import mcmc as plain_host
     from . import mcmc_clustering as cl_host
@@ -341,9 +383,11 @@ def sweep_table(pargs_list, driver: str = "plain", runs: int = 1, seed: int = 0,
                                       "part of the file-name tokens (aggregate_mcmc.jl:40-57; use --kappaflag for bend-mod)")
         seen[pre] = i
     res = run_sweep(cases, runs, p0["num-steps"], 0, seed, device, torch_device, protocol, bit_identical,
-                    p0.get("pair-precision", "fp64"), temper, exchange_every)
+                    p0.get("pair-precision", "fp64"), temper, exchange_every, conformation_every, conformation_bins)
     if exchange is not None and temper is not None:
         exchange.update(res["exchange"])
+    if conformation is not None and conformation_every:
+        conformation["buckets"] = res["conformation"]
     runflag = runs > 1
     entries, texts = [], []
     for i, p in enumerate(pargs_list):
@@ -381,8 +425,41 @@ def exchange_rows(pargs_list, temper: str, exchange: dict, fixed=()):
     return header, rows
 
 
+def conformation_tables(pargs_list, conformation: dict, fixed=()):
+    """The four conformation tables of a sampled sweep, each row led by the case's `fixed` options (e.g. the grid axes),
+    from the pooled sums of every case (run_sweep's "conformation"):
+      summary:   samples, S_xx S_yy S_zz S_xy S_xz S_yz, Rg2, Rg4
+      bondcorr:  s, C = ⟨C_s⟩/(n−s), s = 0 … n−1
+      profile:   i (1-based, as the reference numbers monomers), nz = ⟨n̂z_i⟩, nz2 = ⟨n̂z_i²⟩
+      extension: zeta_lo, zeta_hi, count, density = count / (samples·Δζ), one row per bin of ζ = r_z/(n b) on [−1, 1]
+    -> dict name -> (header, rows)."""
+    fixed = list(fixed)
+    out = {"summary": (fixed + ["samples", "S_xx", "S_yy", "S_zz", "S_xy", "S_xz", "S_yz", "Rg2", "Rg4"], []),
+           "bondcorr": (fixed + ["s", "C"], []), "profile": (fixed + ["i", "nz", "nz2"], []),
+           "extension": (fixed + ["zeta_lo", "zeta_hi", "count", "density"], [])}
+    per_case = {}
+    for bucket in conformation["buckets"]:
+        avg = lib.conformation_averages(bucket["sums"], bucket["n"], bucket["bins"])
+        for k, c in enumerate(bucket["cases"].tolist()):
+            per_case[c] = (bucket, k, avg)
+    for c in range(len(pargs_list)):
+        bucket, k, avg = per_case[c]
+        n, B = bucket["n"], bucket["bins"]
+        lead = [pargs_list[c][f] for f in fixed]
+        samples = int(avg["samples"][k])
+        out["summary"][1].append(lead + [samples, *avg["S"][k].tolist(), float(avg["Rg2"][k]), float(avg["Rg4"][k])])
+        out["bondcorr"][1].extend(lead + [s, float(avg["bondcorr"][k, s])] for s in range(n))
+        out["profile"][1].extend(lead + [i + 1, float(avg["nz"][k, i]), float(avg["nz2"][k, i])] for i in range(n))
+        counts = bucket["sums"][k, 8 + 3 * n:]
+        dz = 2.0 / B if B else 0.0
+        out["extension"][1].extend(lead + [-1 + j * dz, -1 + (j + 1) * dz, int(counts[j]), counts[j] / (samples * dz)]
+                                   for j in range(B))
+    return out
+
+
 def write_exchange_csv(path: str, header, rows):
-    """exchange_rows() as CSV: counts as integers, other numbers as Julia prints Float64, anything else as text."""
+    """exchange_rows() or a conformation table as CSV: counts as integers, other numbers as Julia prints Float64,
+    anything else as text."""
     from .output import julia_float
 
     def cell(x):

@@ -50,9 +50,24 @@ def main(argv=None) -> int:
     ap.add_argument("--exchange-every", type=int, default=100, help="trials between two exchange rounds")
     ap.add_argument("--exchange-out", default=None,
                     help="CSV of the exchange statistics: one row per adjacent rung pair (needs --temper)")
+    ap.add_argument("--conformation-every", type=int, default=0,
+                    help="sample every chain's shape every K trials of the production run (0: off; with --temper it "
+                         "must equal --exchange-every)")
+    ap.add_argument("--conformation-bins", type=int, default=0,
+                    help="bins of the extension histogram, zeta = r_z / (n b) on [-1, 1] (0: none)")
+    ap.add_argument("--conformation-out", default=None, metavar="PREFIX",
+                    help="write PREFIX_summary.csv, PREFIX_bondcorr.csv, PREFIX_profile.csv and PREFIX_extension.csv "
+                         "(needs --conformation-every)")
     a = ap.parse_args(argv)
     if a.exchange_out and not a.temper:
         ap.error("--exchange-out needs --temper")
+    if a.conformation_out and a.conformation_every <= 0:
+        ap.error("--conformation-out needs --conformation-every")
+    if a.conformation_every < 0 or a.conformation_bins < 0:
+        ap.error("--conformation-every and --conformation-bins must be >= 0")
+    if a.conformation_every and a.temper and a.conformation_every != a.exchange_every:
+        ap.error("with --temper the chains are sampled at the exchange rounds: --conformation-every must equal "
+                 "--exchange-every")
     host = {"plain": mcmc, "clustering": mcmc_clustering, "clustering2d": mcmc_clustering_2d}[a.driver]
     axes = []
     for g in a.grid:
@@ -79,11 +94,13 @@ def main(argv=None) -> int:
         rank = dist.get_rank()
     if a.by and not a.by_outdir:
         ap.error("--by needs --by-outdir")
-    exchange = {}
+    exchange, conformation = {}, {}
     header, rows, texts, entries = sweep.sweep_table(pargs_list, driver=a.driver, runs=a.runs, seed=a.seed,
                                                      device=a.device, torch_device=torch_device,
                                                      kappaflag=a.kappaflag, with_entries=True, bit_identical=a.bit_identical,
-                                                     temper=a.temper, exchange_every=a.exchange_every, exchange=exchange)
+                                                     temper=a.temper, exchange_every=a.exchange_every, exchange=exchange,
+                                                     conformation_every=a.conformation_every,
+                                                     conformation_bins=a.conformation_bins, conformation=conformation)
     if world > 1:
         import torch.distributed as dist
         dist.destroy_process_group()
@@ -99,6 +116,10 @@ def main(argv=None) -> int:
     if a.exchange_out:
         fixed = [name for name, _ in axes if name != a.temper]
         sweep.write_exchange_csv(a.exchange_out, *sweep.exchange_rows(pargs_list, a.temper, exchange, fixed))
+    if a.conformation_out:
+        fixed = [name for name, _ in axes]
+        for name, (h, r) in sweep.conformation_tables(pargs_list, conformation, fixed).items():
+            sweep.write_exchange_csv(f"{a.conformation_out}_{name}.csv", h, r)
     if a.by:
         os.makedirs(a.by_outdir, exist_ok=True)
         ct = pargs_list[0]["chain-type"]
